@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W    # the reference algorithm on the host cores (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 Headline workload (north_star target, BASELINE.json configs[4]/[2]): synthetic 12 MP Bayer frames (4032x3024, 10-bit:
 wp 1023, bl 64, Poisson-Gaussian noise), 8 frames per GPU per step, image-parallel across the GPUs; GuidedResUnet
@@ -144,6 +145,38 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm), "scope": scope}
 
 
+DUMP_SAMPLE = 1 << 22   # values kept of an output larger than this: a fixed seeded set of positions, the same for every output
+DUMP_LIMIT = 64 << 20   # bytes written by --dump-outputs in all
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: array or tensor} as out_dir/<name>.npy in float32 / float64, so that the outputs of two builds can be compared
+    file by file.  An output of more than DUMP_SAMPLE values is written as a 1-D array of its values at DUMP_SAMPLE seeded flat
+    positions (sorted, duplicates dropped); the positions depend on the output's size only."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        a = a if torch.is_tensor(a) else torch.from_numpy(np.asarray(a))
+        if a.numel() > DUMP_SAMPLE:
+            pos = np.unique(np.random.default_rng(0).integers(0, a.numel(), DUMP_SAMPLE))
+            a = a.reshape(-1)[torch.from_numpy(pos).to(a.device)]
+        a = a.cpu().numpy()
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        total += a.nbytes
+        if total > DUMP_LIMIT:
+            raise ValueError(f"--dump-outputs would write more than {DUMP_LIMIT >> 20} MB")
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def last_step_outputs(res):
+    """The arrays IterDenoise hands its caller: the denoised frames of the first and the final round, (beta1, beta2) of every
+    round, and how many rounds each frame completed."""
+    out = {"raw_dns_round1": res["raw_dns"][0], "raw_dns_final": res["raw_dns"][-1], "rounds": res["rounds"]}
+    out.update({f"regs_round{i + 1}": np.asarray(r, np.float64) for i, r in enumerate(res["regs"])})
+    return out
+
+
 def measured_peaks():
     try:
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
@@ -190,8 +223,11 @@ def run_reference(args):
         cpu_reference_step(frames[w % 2], sd, lut)
     t0 = time.perf_counter()
     for s in range(args.steps):
-        rounds.append(len(cpu_reference_step(frames[s % 2], sd, lut)["raw_dns"]))
+        res = cpu_reference_step(frames[s % 2], sd, lut)
+        rounds.append(len(res["raw_dns"]))
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step_outputs(dict(res, rounds=np.array([rounds[-1]]))))
     mp = args.steps * CPU_SAMPLE[0] * CPU_SAMPLE[1] / 1e6
     val = mp / dt
     try:
@@ -298,6 +334,8 @@ def run_b200(args):
     def step_frames():  # one host thread, one stream: every stage once for all 8 frames; one small read-back at the end
         res = drv.iter_denoise_batch(dev_in, dict(P0))
         last["rounds"] = res["rounds"]
+        if args.dump_outputs:  # only then are a step's outputs kept alive into the next step
+            last["res"] = res
         if world > 1:
             gather_frames(res["raw_dns"][-1])
 
@@ -332,6 +370,10 @@ def run_b200(args):
     hbm_prof = Y._lib.prof_read(reset=True)
     net.set_profile(False)
     Y._lib.prof_enable(False)
+    last_res = last.pop("res", None)
+    if last_res is not None and rank == 0:
+        dump_outputs(args.dump_outputs, last_step_outputs(last_res))
+    del last_res
     for _ in range(args.warmup):  # the end-to-end leg warms up like the device-resident one (pinned buffers, staging ring, streams)
         step_frames_e2e()
     collect(0)
@@ -387,8 +429,7 @@ def run_b200(args):
         step = lambda: parallel.denoise_frame_sharded(drv, fr, dict(p))  # noqa: E731
         for _ in range(2):
             step()
-        k = max(3, min(args.steps, 10))
-        ms_f = timed(step, k) / k
+        ms_f = timed(step, args.steps) / args.steps
         res = step()
         _, rnds, _ = drv.read_summary(res)
         frame_sharded[name] = {"ms_per_frame": ms_f, "MP_per_s": H * W / 1e6 / (ms_f / 1e3), "ranks": world, "rounds": int(rnds[0]),
@@ -535,7 +576,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of the headline workload (rank 0) "
+                    "as DIR/<name>.npy; the inputs are the same in every run")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -41,8 +41,10 @@ def test_library_exports_every_declared_symbol(Y):
 
 def test_library_is_sm100a_tcgen05():
     """The conv kernel object must contain tcgen05 / TMA machine code (UTCHMMA, UTMALDG, LDTM), not legacy HMMA."""
+    from yond_public_b200 import build
     obj = os.path.join(ROOT, "yond_public_b200", "build", "conv_tc.o")
-    sass = subprocess.run(["cuobjdump", "-sass", obj], capture_output=True, text=True).stdout
+    cuda_bin = os.path.dirname(build._nvcc())  # the toolkit the library was built with, also when it is not on PATH
+    sass = subprocess.run([os.path.join(cuda_bin, "cuobjdump") if cuda_bin else "cuobjdump", "-sass", obj], capture_output=True, text=True).stdout
     if not sass:
         pytest.skip("cuobjdump not available")
     assert "UTCHMMA" in sass and "UTMALDG" in sass and "LDTM" in sass

@@ -260,16 +260,25 @@ def test_render_golden(golden):
     np.testing.assert_allclose(ss, g["ssim_u8_blocks"].mean(), rtol=0, atol=1e-12)
 
 
-def test_demosaic_restatement_matches_cv2():
-    """The edge-aware demosaic restatement against OpenCV itself (the third-party routine behind demosaic_CV2), bit for bit, on
-    seeded mosaics: full 14-bit range, tiny ranges (gradient ties everywhere), constant images, the smallest legal size."""
-    cv2 = pytest.importorskip("cv2")
-    rng = np.random.default_rng(5)
-    for (h, w, hi) in [(4, 4, 16384), (6, 10, 16384), (64, 96, 16384), (66, 130, 8), (32, 34, 2), (30, 62, 3), (128, 258, 16384)]:
-        b = rng.integers(0, hi, size=(h, w), dtype=np.uint16)
-        assert np.array_equal(O.demosaic_ea_u16(b), cv2.cvtColor(b, cv2.COLOR_BayerBG2RGB_EA)), (h, w, hi)
-    b = np.full((8, 12), 16383, np.uint16)
-    assert np.array_equal(O.demosaic_ea_u16(b), cv2.cvtColor(b, cv2.COLOR_BayerBG2RGB_EA))
+def test_demosaic_restatement_matches_cv2(golden):
+    """The edge-aware demosaic restatement against OpenCV (the third-party routine behind demosaic_CV2), bit for bit, on seeded
+    mosaics: full 14-bit range, tiny ranges (gradient ties everywhere), constant images, the smallest legal size.  Checked against
+    the CRC-32 of cv2's outputs (make_golden_demosaic.py), and against cv2 itself where it is installed."""
+    g = golden("demosaic_cv2")
+    rng = np.random.default_rng(int(g["seed"]))
+    mosaics = [rng.integers(0, hi, size=(h, w), dtype=np.uint16) for (h, w, hi) in g["cases"].tolist()]
+    h, w, v = g["flat"].tolist()
+    mosaics.append(np.full((h, w), v, np.uint16))
+    assert len(mosaics) == len(g["crc"])
+    try:
+        import cv2
+    except ImportError:
+        cv2 = None
+    for b, want in zip(mosaics, g["crc"]):
+        got = O.demosaic_ea_u16(b)
+        assert crc(got) == want, b.shape
+        if cv2 is not None:
+            assert np.array_equal(got, cv2.cvtColor(b, cv2.COLOR_BayerBG2RGB_EA)), b.shape
 
 
 def test_rgb_metrics_oracle():
