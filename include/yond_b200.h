@@ -199,7 +199,12 @@ int yond_masked_sums(const float* lap, const float* mean, const float* var, size
  *   of the first input — the bound of the fallback bias table (:393, isp_algos.py:101).  `work`: yond_nlf_work_bytes(B,h,w,4).
  *   mode 0: self maps (y unused); 1: collab maps; 2: collab maps where `var` holds, on entry, the var map of the SELF estimate of
  *   the same frames in the same geometry — SelfNLF's var is stdfilt(lr, k)**2 and CollabNLF starts from the very same float32
- *   expression (:66-68, :94-97), so the pass over x is skipped and `var` is updated in place (x is not read).
+ *   expression (:66-68, :94-97), so the pass over x is skipped and `var` is updated in place (x is not read); 3: var =
+ *   stdfilt(x, k)**2 alone (y, mean, lap untouched): the noisy-frame statistics every collab round of IterDenoise shares.
+ * yond_nlf_maps_collab_cached: the collab maps of a round from a cached `lr_var` = stdfilt(lr, k)**2 in the same geometry (the
+ *   var map of mode 0 or mode 3; read only, may be `var` itself = mode 2): var = lr_var - stdfilt(y, k)**2, mean = blur_k(y),
+ *   lap = stdfilt(y, k), one box pass over the float32 frame y (layout / geometry arguments as above).  The noisy frame is not
+ *   an argument, so the call is the same for float32 and uint16 sensor inputs.
  * yond_nlf_fit: percentiles -> score3 threshold -> masked sums (with the empty-mask fallbacks of :77-84) -> line fit,
  *   per segment, all on the device: regs_dev (nseg,2) float64 = (beta1, beta2).  `quants_host`: the nq <= 24 ascending
  *   percentiles of get_threshold (np.linspace(step,100,100//step)).  detail_dev (optional, (nseg, 52) float64):
@@ -212,6 +217,8 @@ int yond_nlf_maps_bayer(const float* x, int x_mosaic, const float* y, int y_mosa
 int yond_nlf_maps_raw16(const uint16_t* x, const yond_raw_norm* nrm, int x_mosaic, const float* y, int y_mosaic, float* var, float* mean,
                         float* lap, int nimg, int nblk, int H, int W, int split_blocks, int k, int mode, float* seg_max, void* work,
                         void* stream);
+int yond_nlf_maps_collab_cached(const float* y, int y_mosaic, const float* lr_var, float* var, float* mean, float* lap, int nimg,
+                                int nblk, int H, int W, int split_blocks, int k, void* stream);
 size_t yond_nlf_fit_work_bytes(int nseg);
 int yond_nlf_fit(const float* var, const float* mean, const float* lap, size_t seg_len, int nseg, const double* quants_host,
                  int nq, double* regs_dev, double* detail_dev, void* work, void* stream);
@@ -221,8 +228,9 @@ int yond_nlf_fit(const float* var, const float* mean, const float* lap, size_t s
  * :49-140 (get_bias: the numeric Poisson (*) Gaussian fallback table — SURVEY 8(f)-2, generated on the device).
  * yond_vst_params_fill: regs_dev (nseg,2) -> per-frame yond_vst_params (nseg*frames_per_seg), t_dev (same count), and per
  *   image one bias row + its node positions in rows / xnodes (nseg, row_stride).  round 1: sigma = sqrt(max(beta2,0));
- *   round 2: beta2 < 0 -> beta1^2 and ok_dev[s] = (beta1 >= 0) (images with ok = 0 get `prev_params`, their output is
- *   discarded by yond_vst_inv_place).  bias_mode: 0 = None, 1 = 'pre' (bias applied, t*1.03), 2 = 'post' (no bias is
+ *   round >= 2: beta2 < 0 -> beta1^2 and ok_dev[s] = (beta1 >= 0) && prev_ok[s] (images with ok = 0 get `prev_params`, their
+ *   output is discarded by yond_vst_inv_place).  prev_ok (optional, the previous round's ok_dev; NULL = every image live):
+ *   chains the live mask over the rounds of IterDenoise, an image that stopped never comes back whatever its later beta1.  bias_mode: 0 = None, 1 = 'pre' (bias applied, t*1.03), 2 = 'post' (no bias is
  *   applied, like the reference).  lut2d (nx,nsg) f32 + sg_lut_dev (nsg) f64 + x_lut_dev (nx) f32: the BiasLUT, or NULL:
  *   then — and for sigma/K beyond the table — the numeric table up to bound = seg_max[s]*bound_scale (float32 product).
  *   regs_out (optional, (nseg,4) f64): beta1, beta2 (after the guard), gain, sigma.  `work`: yond_chain_work_bytes(nseg).
@@ -234,7 +242,8 @@ int yond_vst_params_fill(const double* regs_dev, const float* seg_max_dev, int n
                          double scale, double bound_scale, int round, int bias_mode, int exact_inverse, const float* lut2d,
                          const double* sg_lut_dev, const float* x_lut_dev, int nx, int nsg,
                          const yond_vst_params* prev_params, yond_vst_params* params_dev, float* t_dev, float* rows,
-                         float* xnodes, int row_stride, double* regs_out, int32_t* ok_dev, void* work, void* stream);
+                         float* xnodes, int row_stride, double* regs_out, int32_t* ok_dev, void* work, void* stream,
+                         const int32_t* prev_ok);
 int yond_bias_table(double gain, double sigma, float bound, float* nodes_dev, float* vals_dev, int cap,
                     int32_t* n_nodes_dev, void* work, void* stream);
 /* get_bias_points(lams, K, sigGs, pho_min, close_form=True) (isp_algos.py:142-160): the bias at explicit float64 points

@@ -63,11 +63,12 @@ SIGNATURES = {
     "yond_masked_sums": (_I, [_P, _P, _P, _SZ, _I, _P, _P, _P]),
     "yond_nlf_maps_bayer": (_I, [_P, _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
     "yond_nlf_maps_raw16": (_I, [_P, C.POINTER(RawNorm), _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "yond_nlf_maps_collab_cached": (_I, [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "yond_nlf_fit_work_bytes": (_SZ, [_I]),
     "yond_nlf_fit": (_I, [_P, _P, _P, _SZ, _I, C.POINTER(_D), _I, _P, _P, _P, _P]),
     "yond_chain_work_bytes": (_SZ, [_I]),
     "yond_bias_table_nodes": (_I, [C.c_float]),
-    "yond_vst_params_fill": (_I, [_P, _P, _I, _I, _D, _D, _D, _I, _I, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P]),
+    "yond_vst_params_fill": (_I, [_P, _P, _I, _I, _D, _D, _D, _I, _I, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P]),
     "yond_bias_table": (_I, [_D, _D, C.c_float, _P, _P, _I, _P, _P, _P]),
     "yond_bias_points": (_I, [_P, _I, _D, _D, _I, _P, _P, _P]),
     "yond_vst_inv_place": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _I, _I, _I, _P, _I, _P, _P]),

@@ -1,6 +1,6 @@
 // Device-resident VST parameter chain: from the estimator's (beta1, beta2) to everything the fused VST kernels need,
 // without a host read-back.
-//   reference: YOND_SIDD.py:356 / :438-447 (gain, sigma and the round-2 guards), :252-269,284-285 (bias source, VST(0),
+//   reference: YOND_SIDD.py:356 / :419-472 (gain, sigma and the guards of the collab rounds), :252-269,284-285 (bias source, VST(0),
 //              VST(scale), nsr, t), utils/isp_algos.py:179-231 (BiasLUT.pos_interp / data_merge over sigma),
 //              :49-82,84-96,98-140 (getGsP / close_form_bias / get_bias: the fallback bias table).
 // All scalar arithmetic is float64 with explicit round-to-nearest operations in NumPy's evaluation order.
@@ -18,7 +18,7 @@ struct SegChain {     // per image; written by params_fill_kernel, consumed by t
   int use_lut;        // 1: sigma-interpolated BiasLUT row
   int need_table;     // 1: numeric get_bias table
   int n_nodes;        // nodes of that table
-  int ok;             // round 2: beta1 >= 0
+  int ok;             // rounds >= 2: still live (beta1 >= 0 in this round and every earlier one)
 };
 
 __device__ __forceinline__ double vst_d(double v, double K, double sig) {
@@ -208,8 +208,8 @@ struct FillArgs {
 // One thread per image.
 __global__ void params_fill_kernel(FillArgs a, const double* __restrict__ regs, const float* __restrict__ seg_max,
                                    const double* __restrict__ sg_lut, const yond_vst_params* __restrict__ prev,
-                                   yond_vst_params* __restrict__ params, float* __restrict__ t_out, SegChain* __restrict__ chain,
-                                   double* __restrict__ regs_out, int32_t* __restrict__ ok_out) {
+                                   const int32_t* __restrict__ prev_ok, yond_vst_params* __restrict__ params, float* __restrict__ t_out,
+                                   SegChain* __restrict__ chain, double* __restrict__ regs_out, int32_t* __restrict__ ok_out) {
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= a.nseg) return;
   double b1 = regs[2 * s], b2 = regs[2 * s + 1];
@@ -218,7 +218,8 @@ __global__ void params_fill_kernel(FillArgs a, const double* __restrict__ regs, 
   if (a.round >= 2) {  // YOND_SIDD.py:438-447
     if (b2 < 0.0) b2 = __dmul_rn(b1, b1);
     sig = __dmul_rn(sqrt(b2), a.scale_est);
-    ok = !(b1 < 0.0);
+    // the reference leaves its loop at the first beta1 < 0: an image that stopped in an earlier round stays stopped
+    ok = !(b1 < 0.0) && (!prev_ok || prev_ok[s]);
   } else {             // :356  sqrt(max(beta2, 0))
     sig = __dmul_rn(sqrt(0.0 > b2 ? 0.0 : b2), a.scale_est);
   }
@@ -237,8 +238,8 @@ __global__ void params_fill_kernel(FillArgs a, const double* __restrict__ regs, 
   yond_vst_params q{};
   float t = 0.f;
   if (!ok && prev) {
-    // beta1 < 0: the reference keeps the round-1 result; this image's round-2 output is discarded by the back half, the
-    // parameters of round 1 keep the wasted pass well-defined
+    // stopped: the reference keeps the previous round's result; this image's output of this round is discarded by the back half,
+    // the parameters of its last live round (carried from round to round in `prev`) keep the wasted pass well-defined
     q = prev[(size_t)s * a.frames_per_seg];
     q.lut_row = -1;
     q.table_n = 0;
@@ -328,7 +329,7 @@ int yond_vst_params_fill(const double* regs_dev, const float* seg_max_dev, int n
                          double scale, double bound_scale, int round, int bias_mode, int exact_inverse, const float* lut2d,
                          const double* sg_lut_dev, const float* x_lut_dev, int nx, int nsg, const yond_vst_params* prev_params,
                          yond_vst_params* params_dev, float* t_dev, float* rows, float* xnodes, int row_stride, double* regs_out,
-                         int32_t* ok_dev, void* work, void* stream) {
+                         int32_t* ok_dev, void* work, void* stream, const int32_t* prev_ok) {
   YOND_REQUIRE(regs_dev && params_dev && t_dev && work, "yond_vst_params_fill: null argument");
   YOND_REQUIRE(nseg > 0 && nseg <= 65535 && frames_per_seg > 0, "yond_vst_params_fill: bad batch geometry");
   YOND_REQUIRE(bias_mode >= 0 && bias_mode <= 2, "yond_vst_params_fill: bias_mode 0 (None), 1 ('pre'), 2 ('post')");
@@ -348,8 +349,8 @@ int yond_vst_params_fill(const double* regs_dev, const float* seg_max_dev, int n
   a.nsg = nsg;
   a.has_lut = lut2d != nullptr;
   a.max_nodes = row_stride;
-  params_fill_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(a, regs_dev, seg_max_dev, sg_lut_dev, prev_params, params_dev, t_dev, chain,
-                                                      regs_out, ok_dev);
+  params_fill_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(a, regs_dev, seg_max_dev, sg_lut_dev, prev_params, prev_ok, params_dev, t_dev,
+                                                      chain, regs_out, ok_dev);
   YOND_LAUNCH_CHECK();
   if (bias_mode == 1) {
     if (lut2d) {

@@ -26,10 +26,10 @@ __device__ __forceinline__ float4 sq4(const float4& v) {
 // fewer instructions than scanning the column sums where they live).  All sums are float64 sums of float32 values,
 // so the result equals cv2.blur's float64 accumulation rounded to float32 up to the (far below float32) float64
 // rounding of the summation order.  S is double-buffered by row parity: two __syncthreads per row.
-// OP_MEAN_VAR: out0 = mean, out1 = std^2 (SelfNLF's var).  OP_COLLAB: out0 = mean, out1 = std (lap), out2 = aux^2 - std^2
-// with aux = the std map of the other frame (CollabNLF's var).  Squares / difference in float32 with explicit rounding,
-// like the reference's elementwise float32 expressions.
-enum { OP_MEAN = 0, OP_MEAN_STD = 1, OP_STD = 2, OP_MEAN_VAR = 3, OP_COLLAB = 4, OP_COLLAB_SQ = 5 };  // _SQ: out2 holds aux^2 on entry
+// OP_MEAN_VAR: out0 = mean, out1 = std^2 (SelfNLF's var).  OP_VAR: out0 = std^2.  OP_COLLAB: out0 = mean, out1 = std (lap),
+// out2 = aux - std^2 with aux = std_k(other frame)^2 (CollabNLF's var), a read-only map that may be out2 itself (in place).
+// Squares / difference in float32 with explicit rounding, like the reference's elementwise float32 expressions.
+enum { OP_MEAN = 0, OP_MEAN_STD = 1, OP_STD = 2, OP_MEAN_VAR = 3, OP_VAR = 4, OP_COLLAB = 5 };
 constexpr int kBoxThreads = 256;
 // Where the k x k window reads its pixels from.  kBayer = false: packed frames (B,h,w,4) float32.  kBayer = true: the Bayer
 // mosaic itself (two 64-bit loads per packed pixel, rows 2i and 2i+1) — the estimator then needs no pack pass at all — with
@@ -62,7 +62,7 @@ __device__ __forceinline__ int reflect_once(int i, int n) {
 template <bool kSq, int kCols, bool kBayer, bool kNarrow, int kRows>  // kCols = 256, or 160 when a whole row plus both halos fits
 __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, float4* __restrict__ out0,
                                                                 float4* __restrict__ out1, int B, int h, int w, int k, int op,
-                                                                int rows_per_strip, const float4* __restrict__ aux,
+                                                                int rows_per_strip, const float4* aux,  // may alias out2
                                                                 float4* __restrict__ out2) {
   constexpr int NQ = kSq ? 8 : 4;
   constexpr int CH = kCols / 32;           // columns per scan chunk (8 or 5)
@@ -282,15 +282,12 @@ __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, floa
           } else if (op == OP_MEAN_VAR) {
             out0[o] = m;
             out1[o] = sq4(st);
+          } else if (op == OP_VAR) {
+            out0[o] = sq4(st);
           } else if (op == OP_COLLAB) {
             out0[o] = m;
             out1[o] = st;
-            const float4 ax = __ldg(aux + o), a2 = sq4(ax), s2 = sq4(st);
-            out2[o] = make_float4(__fsub_rn(a2.x, s2.x), __fsub_rn(a2.y, s2.y), __fsub_rn(a2.z, s2.z), __fsub_rn(a2.w, s2.w));
-          } else if (op == OP_COLLAB_SQ) {  // out2 already holds std_k(other frame)^2 (the self estimate's var map): in place
-            out0[o] = m;
-            out1[o] = st;
-            const float4 a2 = out2[o], s2 = sq4(st);
+            const float4 a2 = aux[o], s2 = sq4(st);
             out2[o] = make_float4(__fsub_rn(a2.x, s2.x), __fsub_rn(a2.y, s2.y), __fsub_rn(a2.z, s2.z), __fsub_rn(a2.w, s2.w));
           } else {
             out0[o] = st;
@@ -950,6 +947,13 @@ int box_pass(const BoxSrc& src, bool bayer, float* out0, float* out1, int B, int
   return YOND_OK;
 }
 
+// CollabNLF's maps from a cached std_k(lr)^2 map `lr_var` in the same geometry (read only; may be `var` itself): the one box pass over
+// the denoised frame y.  var = lr_var - std_k(y)^2, mean = blur_k(y), lap = std_k(y).
+int collab_from_lr_var(const BoxSrc& y, bool bayer, const float* lr_var, float* var, float* mean, float* lap, int B, int h, int w, int k,
+                       cudaStream_t s) {
+  return box_pass(y, bayer, mean, lap, B, h, w, k, true, OP_COLLAB, s, lr_var, var);
+}
+
 // Maps of SelfNLF / CollabNLF from either source kind
 int nlf_maps_impl(const BoxSrc& x, const BoxSrc* y, bool bayer, float* var, float* mean, float* lap, int B, int h, int w, int k, int mode,
                   void* work, cudaStream_t s) {
@@ -957,10 +961,11 @@ int nlf_maps_impl(const BoxSrc& x, const BoxSrc* y, bool bayer, float* var, floa
   float* tmpA = reinterpret_cast<float*>(work);
   float* tmpB = tmpA + n;
   int rc;
-  // algorithmic bytes per Bayer pixel (SURVEY 8d): self 4 R + 12 W (lap, mean, var), collab 8 R + 12 W
-  YondProfScope prof(mode == 0 ? "nlf_maps_self (3 box_fused passes)"
-                               : (mode == 1 ? "nlf_maps_collab (2 box_fused passes)" : "nlf_maps_collab (1 box_fused pass, lr statistics reused)"),
-                     s, (mode == 0 ? 16.0 : 20.0) * (double)n);
+  // algorithmic bytes per Bayer pixel (SURVEY 8d): self 4 R + 12 W (lap, mean, var), collab 8 R + 12 W, lr var 4 R + 4 W
+  static const char* names[4] = {"nlf_maps_self (3 box_fused passes)", "nlf_maps_collab (2 box_fused passes)",
+                                 "nlf_maps_collab (1 box_fused pass, lr statistics reused)", "nlf_maps_lr_var (1 box_fused pass)"};
+  static const double bytes[4] = {16.0, 20.0, 20.0, 8.0};
+  YondProfScope prof(names[mode], s, bytes[mode] * (double)n);
   BoxSrc x_nomax = x;
   x_nomax.seg_max = nullptr;
   if (mode == 0) {
@@ -972,14 +977,40 @@ int nlf_maps_impl(const BoxSrc& x, const BoxSrc* y, bool bayer, float* var, floa
     if ((rc = box_pass(packed_src(tmpB, h, w), false, lap, nullptr, B, h, w, k, true, OP_STD, s))) return rc;
   } else if (mode == 2) {
     // `var` holds std_k(lr)^2 from the self estimate of the same frames (SelfNLF's var map IS stdfilt(lr, k)**2, YOND_SIDD.py:66-68 /
-    // :94-97: the same float32 expression): only the statistics of the denoised frame are new
-    if ((rc = box_pass(*y, bayer, mean, lap, B, h, w, k, true, OP_COLLAB_SQ, s, nullptr, var))) return rc;
+    // :94-97: the same float32 expression): only the statistics of the denoised frame are new, `var` is updated in place
+    if ((rc = collab_from_lr_var(*y, bayer, var, var, mean, lap, B, h, w, k, s))) return rc;
+  } else if (mode == 3) {
+    // var = std_k(x)^2 alone: the cached lr statistics of the collab rounds (mean / lap untouched)
+    if ((rc = box_pass(x, bayer, var, nullptr, B, h, w, k, true, OP_VAR, s))) return rc;
   } else {
-    // std_k(lr) -> tmpA ; mean = blur_k(hr), lap = std_k(hr) ; var = std_lr^2 - std_hr^2
-    if ((rc = box_pass(x, bayer, tmpA, nullptr, B, h, w, k, true, OP_STD, s))) return rc;
-    if ((rc = box_pass(*y, bayer, mean, lap, B, h, w, k, true, OP_COLLAB, s, tmpA, var))) return rc;
+    // std_k(lr)^2 -> tmpA ; mean = blur_k(hr), lap = std_k(hr) ; var = std_lr^2 - std_hr^2
+    if ((rc = box_pass(x, bayer, tmpA, nullptr, B, h, w, k, true, OP_VAR, s))) return rc;
+    if ((rc = collab_from_lr_var(*y, bayer, tmpA, var, mean, lap, B, h, w, k, s))) return rc;
   }
   return YOND_OK;
+}
+
+// Bayer inputs of the box filters: `nimg` images of `nblk` blocks of (H,W), blocks layout (nimg,nblk,H,W) or mosaic layout
+// (nimg,H,nblk*W).  split_blocks = 1: every block is its own image for the box filters (SIDD_256, YOND_SIDD.py:65,91-93);
+// split_blocks = 0: the nblk blocks of an image form one mosaic (:315), h x (nblk*w) packed pixels.  With split_blocks the
+// box-filter image index runs over blocks, and a block's origin in a mosaic is not a multiple of the image stride: it is folded
+// into per-image / per-block strides.
+BoxSrc bayer_src(const float* base, int mosaic, int nblk, int H, int W, int split_blocks) {
+  BoxSrc d{};
+  d.base = base;
+  d.blk_w = W / 2;
+  d.imgs_per_seg = split_blocks ? nblk : 1;
+  if (!mosaic) {
+    d.row_len = W;
+    d.blk_stride = (long long)H * W;
+    d.img_stride = split_blocks ? (long long)H * W : (long long)nblk * H * W;
+  } else {
+    d.row_len = nblk * W;
+    d.blk_stride = W;
+    d.img_stride = split_blocks ? 0 : (long long)nblk * H * W;  // split_blocks: see box kernel (image b = mosaic b / nblk, block b % nblk)
+    d.mosaic_blocks = split_blocks ? nblk : 0;
+  }
+  return d;
 }
 
 }  // namespace
@@ -1015,45 +1046,23 @@ int yond_nlf_maps(const float* x, const float* y, float* var, float* mean, float
 static int nlf_maps_bayer_impl(const float* x, const uint16_t* x16, const yond_raw_norm* nrm, int x_mosaic, const float* y, int y_mosaic,
                                float* var, float* mean, float* lap, int nimg, int nblk, int H, int W, int split_blocks, int k, int mode,
                                float* seg_max, void* work, void* stream) {
-  YOND_REQUIRE((x || x16) && var && mean && lap && work, "yond_nlf_maps_bayer: null argument");
+  YOND_REQUIRE((x || x16) && var && (mode == 3 || (mean && lap)) && work, "yond_nlf_maps_bayer: null argument");
   YOND_REQUIRE(!x16 || (nrm && nrm->white > nrm->black && (uintptr_t)x16 % 4 == 0), "yond_nlf_maps_raw16: normalisation / 4-byte aligned mosaic required");
   YOND_REQUIRE(nimg > 0 && nblk > 0 && H > 0 && W > 0 && H % 2 == 0 && W % 2 == 0, "yond_nlf_maps_bayer: H,W must be even");
   YOND_REQUIRE(k % 2 == 1 && k >= 3 && k <= kMaxK, "yond_nlf_maps_bayer: odd k <= %d required (got %d)", kMaxK, k);
-  YOND_REQUIRE(mode == 0 || ((mode == 1 || mode == 2) && y != nullptr), "yond_nlf_maps_bayer: collab mode needs the second input");
+  YOND_REQUIRE(mode == 0 || mode == 3 || ((mode == 1 || mode == 2) && y != nullptr), "yond_nlf_maps_bayer: mode 0..3, collab modes need the second input");
   YOND_REQUIRE((!x || (uintptr_t)x % 8 == 0) && (!y || (uintptr_t)y % 8 == 0), "yond_nlf_maps_bayer: 8-byte aligned frames required");
   cudaStream_t s = (cudaStream_t)stream;
-  // split_blocks = 1: every block is its own image for the box filters (SIDD_256, YOND_SIDD.py:65,91-93);
-  // split_blocks = 0: the nblk blocks of an image form one mosaic (:315), h x (nblk*w) packed pixels.
   const int h = H / 2, wb = W / 2;
   const int B = split_blocks ? nimg * nblk : nimg;
   const int w = split_blocks ? wb : nblk * wb;
   YOND_REQUIRE(h > k / 2 && w > k / 2, "yond_nlf_maps_bayer: frame smaller than the filter radius");
   YOND_REQUIRE(B <= 65535, "yond_nlf_maps_bayer: at most 65535 images per call");
-  // layouts of the Bayer inputs: blocks (nimg, nblk, H, W) — the SIDD dataset layout — or mosaic (nimg, H, nblk*W) — what
-  // the back half writes (yond_vst_inv_place).  With split_blocks the box-filter image index runs over blocks, and a
-  // block's origin in a mosaic is not a multiple of the image stride: it is folded into per-image / per-block strides.
-  auto describe = [&](const float* base, int mosaic) {
-    BoxSrc d{};
-    d.base = base;
-    d.blk_w = wb;
-    d.imgs_per_seg = split_blocks ? nblk : 1;
-    if (!mosaic) {
-      d.row_len = W;
-      d.blk_stride = (long long)H * W;
-      d.img_stride = split_blocks ? (long long)H * W : (long long)nblk * H * W;
-    } else {
-      d.row_len = nblk * W;
-      d.blk_stride = W;
-      d.img_stride = split_blocks ? 0 : (long long)nblk * H * W;  // split_blocks: see box kernel (image b = mosaic b / nblk, block b % nblk)
-      d.mosaic_blocks = split_blocks ? nblk : 0;
-    }
-    return d;
-  };
-  BoxSrc xs = describe(x, x_mosaic);
+  BoxSrc xs = bayer_src(x, x_mosaic, nblk, H, W, split_blocks);
   xs.raw = make_raw_norm(x16, nrm);
   xs.seg_max = seg_max;
   if (seg_max) YOND_CUDA_CHECK(cudaMemsetAsync(seg_max, 0, sizeof(float) * nimg, s));
-  BoxSrc ys = describe(y, y_mosaic);
+  BoxSrc ys = bayer_src(y, y_mosaic, nblk, H, W, split_blocks);
   return nlf_maps_impl(xs, &ys, true, var, mean, lap, B, h, w, k, mode, work, s);
 }
 int yond_nlf_maps_bayer(const float* x, int x_mosaic, const float* y, int y_mosaic, float* var, float* mean, float* lap, int nimg,
@@ -1068,6 +1077,23 @@ int yond_nlf_maps_raw16(const uint16_t* x, const yond_raw_norm* nrm, int x_mosai
   YOND_REQUIRE(x != nullptr && nrm != nullptr, "yond_nlf_maps_raw16: null argument");
   return nlf_maps_bayer_impl(nullptr, x, nrm, x_mosaic, y, y_mosaic, var, mean, lap, nimg, nblk, H, W, split_blocks, k, mode, seg_max, work,
                              stream);
+}
+
+int yond_nlf_maps_collab_cached(const float* y, int y_mosaic, const float* lr_var, float* var, float* mean, float* lap, int nimg, int nblk,
+                                int H, int W, int split_blocks, int k, void* stream) {
+  YOND_REQUIRE(y && lr_var && var && mean && lap, "yond_nlf_maps_collab_cached: null argument");
+  YOND_REQUIRE(nimg > 0 && nblk > 0 && H > 0 && W > 0 && H % 2 == 0 && W % 2 == 0, "yond_nlf_maps_collab_cached: H,W must be even");
+  YOND_REQUIRE(k % 2 == 1 && k >= 3 && k <= kMaxK, "yond_nlf_maps_collab_cached: odd k <= %d required (got %d)", kMaxK, k);
+  YOND_REQUIRE((uintptr_t)y % 8 == 0 && (uintptr_t)lr_var % 16 == 0, "yond_nlf_maps_collab_cached: aligned buffers required");
+  const int h = H / 2, wb = W / 2;
+  const int B = split_blocks ? nimg * nblk : nimg;
+  const int w = split_blocks ? wb : nblk * wb;
+  YOND_REQUIRE(h > k / 2 && w > k / 2, "yond_nlf_maps_collab_cached: frame smaller than the filter radius");
+  YOND_REQUIRE(B <= 65535, "yond_nlf_maps_collab_cached: at most 65535 images per call");
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t n = (size_t)B * h * w * 4;
+  YondProfScope prof("nlf_maps_collab (1 box_fused pass, lr statistics reused)", s, 20.0 * (double)n);
+  return collab_from_lr_var(bayer_src(y, y_mosaic, nblk, H, W, split_blocks), true, lr_var, var, mean, lap, B, h, w, k, s);
 }
 
 size_t yond_select_work_bytes(int nseg) { return (size_t)(nseg < 1 ? 1 : nseg) * sizeof(SelectWork) + 256; }

@@ -130,7 +130,7 @@ class NlfEstimator:
     DETAIL = 4 + 2 * 24
 
     def estimate_dev(self, x, y=None, k=29, split_blocks=False, x_mosaic=False, y_mosaic=False, nblk=None, seg_max=None,
-                     details=False, step=5, raw=None, reuse_self_var=False):
+                     details=False, step=5, raw=None, reuse_self_var=False, var_map=None):
         """SelfNLF (y None) / CollabNLF straight from Bayer frames, everything on the device.
 
         x: blocks layout (nimg, nblk, H, W) or, with x_mosaic, mosaic layout (nimg, H, nblk*W) (`nblk` then required; plain
@@ -139,7 +139,9 @@ class NlfEstimator:
         device [, detail (nimg, DETAIL)]; nothing is read back.  x may be the uint16 sensor mosaic (a 16-bit integer tensor) with
         raw = _lib.RawNorm(black, white, ratio, clip): it is normalised on load (SURVEY 8(f)-1).
         reuse_self_var (collab only): the previous call on this estimator was the SELF estimate of the same x in the same geometry,
-        so its var map (= stdfilt(x, k)**2, exactly what CollabNLF computes first) is still in place and the pass over x is skipped."""
+        so its var map (= stdfilt(x, k)**2, exactly what CollabNLF computes first) is still in place and the pass over x is skipped.
+        var_map (self only; float32 CUDA, at least B*h*w*4 values): the var map goes there instead of the estimator's scratch, where
+        no later call overwrites it — the cached noisy-frame statistics of the collab rounds (estimate_collab_cached)."""
         lib = self.lib
         if x_mosaic:
             nimg, H, Wm = x.shape
@@ -155,6 +157,9 @@ class NlfEstimator:
         n_el = B * h * w * 4
         maps = self._buf("maps3", 3 * n_el * 4, dev).view(torch.float32)
         var, mean, lap = maps[:n_el], maps[n_el:2 * n_el], maps[2 * n_el:3 * n_el]
+        if var_map is not None:
+            assert y is None and var_map.dtype == torch.float32 and var_map.is_cuda and var_map.numel() >= n_el
+            var = var_map.reshape(-1)[:n_el]
         work = self._buf("maps", lib.yond_nlf_work_bytes(B, h, w, 4), dev)
         mode = 0 if y is None else (2 if reuse_self_var and getattr(self, "_self_key", None) == (x.data_ptr(), B, h, w, int(k)) else 1)
         self._self_key = (x.data_ptr(), B, h, w, int(k)) if y is None else None
@@ -166,6 +171,11 @@ class NlfEstimator:
         else:
             check(lib.yond_nlf_maps_bayer(ptr(x), int(bool(x_mosaic)), ptr(y), int(bool(y_mosaic)), ptr(var), ptr(mean), ptr(lap), nimg, nb,
                                           H, W, int(bool(split_blocks)), int(k), mode, ptr(seg_max), ptr(work), stream_ptr()))
+        return self._fit(var, mean, lap, nimg, details, step)
+
+    def _fit(self, var, mean, lap, nimg, details=False, step=5):
+        lib, dev = self.lib, var.device
+        n_el = var.numel()
         quants = np.ascontiguousarray(np.linspace(step, 100, 100 // step, endpoint=True), np.float64)
         regs = torch.empty((nimg, 2), device=dev, dtype=torch.float64)
         detail = torch.empty((nimg, self.DETAIL), device=dev, dtype=torch.float64) if details else None
@@ -174,6 +184,58 @@ class NlfEstimator:
         check(lib.yond_nlf_fit(ptr(var), ptr(mean), ptr(lap), n_el // nimg, nimg, quants.ctypes.data_as(C.POINTER(C.c_double)),
                                len(quants), ptr(regs), ptr(detail), ptr(fwork[off:]), stream_ptr()))
         return (regs, detail) if details else regs
+
+    # -- the collab rounds of IterDenoise from cached noisy-frame statistics ---------------------------
+    # Every collab round r >= 2 estimates on (lr, out_{r-1}) in the same geometry.  Its var map is stdfilt(lr, k)**2 -
+    # stdfilt(out_{r-1}, k)**2, and the first term is the same in every round: it is computed once per batch (the self estimate's
+    # var map when the geometries agree, else one lr_var_dev pass) and each round makes one box pass over out_{r-1}.
+    @staticmethod
+    def collab_geometry(nimg, nblk, H, W, split_blocks):
+        """Number of float32 values of a map in the box-filter geometry of `nimg` images of `nblk` (H,W) blocks."""
+        return (nimg * nblk if split_blocks else nimg) * (H // 2) * ((W // 2) if split_blocks else nblk * (W // 2)) * 4
+
+    def lr_var_dev(self, x, out, k=29, split_blocks=False, x_mosaic=False, nblk=None, raw=None):
+        """out <- stdfilt(x, k)**2 in the box-filter geometry (one box pass; x layouts / raw as in estimate_dev)."""
+        lib = self.lib
+        if x_mosaic:
+            nimg, H, Wm = x.shape
+            nb = int(nblk or 1)
+            W = Wm // nb
+        else:
+            nimg, nb, H, W = x.shape
+        assert x.is_cuda and x.is_contiguous() and out.is_contiguous() and out.dtype == torch.float32
+        assert out.numel() >= self.collab_geometry(nimg, nb, H, W, split_blocks)
+        work = self._buf("maps", lib.yond_nlf_work_bytes(1, 1, 1, 4), x.device)  # mode 3 uses no scratch
+        if x.dtype in (torch.int16, torch.uint16):
+            check(lib.yond_nlf_maps_raw16(ptr(x), C.byref(raw), int(bool(x_mosaic)), None, 0, ptr(out), None, None, nimg, nb, H, W,
+                                          int(bool(split_blocks)), int(k), 3, None, ptr(work), stream_ptr()))
+        else:
+            assert x.dtype == torch.float32
+            check(lib.yond_nlf_maps_bayer(ptr(x), int(bool(x_mosaic)), None, 0, ptr(out), None, None, nimg, nb, H, W,
+                                          int(bool(split_blocks)), int(k), 3, None, ptr(work), stream_ptr()))
+        return out
+
+    def collab_maps_cached(self, y, lr_var, nblk, k=29, split_blocks=False, y_mosaic=True):
+        """CollabNLF maps (var, mean, lap) of the float32 frames y — mosaic layout (nimg, H, nblk*W) or, y_mosaic False, blocks
+        layout (nimg, nblk, H, W) — against the cached lr_var = stdfilt(lr, k)**2 (read only) in the same geometry."""
+        if y_mosaic:
+            nimg, H, Wm = y.shape
+            W = Wm // nblk
+        else:
+            nimg, _, H, W = y.shape
+        assert y.is_cuda and y.dtype == torch.float32 and y.is_contiguous() and lr_var.dtype == torch.float32
+        n_el = self.collab_geometry(nimg, nblk, H, W, split_blocks)
+        assert lr_var.numel() >= n_el
+        maps = self._buf("maps3", 3 * n_el * 4, y.device).view(torch.float32)
+        var, mean, lap = maps[:n_el], maps[n_el:2 * n_el], maps[2 * n_el:3 * n_el]
+        check(self.lib.yond_nlf_maps_collab_cached(ptr(y), int(bool(y_mosaic)), ptr(lr_var.reshape(-1)), ptr(var), ptr(mean), ptr(lap),
+                                                   nimg, nblk, H, W, int(bool(split_blocks)), int(k), stream_ptr()))
+        return var, mean, lap
+
+    def estimate_collab_cached(self, y, lr_var, nblk, k=29, split_blocks=False, y_mosaic=True, details=False, step=5):
+        """CollabNLF (beta1, beta2) of a collab round from the cached lr statistics: regs (nimg, 2) float64 on the device."""
+        var, mean, lap = self.collab_maps_cached(y, lr_var, nblk, k, split_blocks, y_mosaic)
+        return self._fit(var, mean, lap, y.shape[0], details, step)
 
     # -- SelfNLF / CollabNLF ----------------------------------------------------------------------
     def estimate(self, lr_rggb, hr_rggb=None, k=29, details=False, nseg=1, timings=None):

@@ -148,7 +148,8 @@ class YondEngine:
 
     def chain_params(self, regs, seg_max, nseg, fps, scale_est, scale, bound_scale, rnd, bias_corr, vst_type, prev=None):
         """regs: (nseg,2) float64 CUDA.  Returns a dict of device buffers: params (bytes), t, rows, xnodes, stride,
-        regs4 (nseg,4: beta1, beta2 after the guards, gain, sigma), ok (nseg int32)."""
+        regs4 (nseg,4: beta1, beta2 after the guards, gain, sigma), ok (nseg int32: still live after this round).
+        prev: the chain of the previous round (rnd >= 2) — its params are kept by images that are not live, and its ok is chained."""
         if bias_corr not in self.BIAS_MODES:
             raise NotImplementedError(f"bias_corr={bias_corr!r}")
         lib, dev = self.lib, regs.device
@@ -170,7 +171,8 @@ class YondEngine:
         check(lib.yond_vst_params_fill(ptr(regs), ptr(seg_max), nseg, fps, float(scale_est), float(scale), float(bound_scale), int(rnd), mode,
                                        exact, ptr(lut[0]) if lut else None, ptr(lut[2]) if lut else None, ptr(lut[1]) if lut else None,
                                        1921, 1101, ptr(prev["params"]) if prev is not None else None, ptr(out["params"]), ptr(out["t"]),
-                                       ptr(rows), ptr(xnodes), stride, ptr(out["regs4"]), ptr(out["ok"]), ptr(work), stream_ptr()))
+                                       ptr(rows), ptr(xnodes), stride, ptr(out["regs4"]), ptr(out["ok"]), ptr(work), stream_ptr(),
+                                       ptr(prev["ok"]) if prev is not None else None))
         return out
 
     def vst_denoise_dev(self, frames, chain, out, frames_per_row=1, fps=1, select=False, fallback=None, clip01=True, raw=None):
@@ -444,23 +446,30 @@ class YOND_SIDD:
         results["hr_raw"] = (np.concatenate(list(hr), axis=-1) if isinstance(hr, np.ndarray) and hr.ndim == 3 else hr)
         return results
 
-    # -- the blind two-round pipeline, device-resident and free of host synchronisation -----------------------------
+    # -- the blind N-round pipeline, device-resident and free of host synchronisation ----------------------------
     reuse_self_var = True  # collab estimate of plain frames starts from the self estimate's var map (one box pass less)
 
     def iter_denoise_dev(self, x, p, lr_full=None, timings=None, raw=None, after_round1=None):
         """IterDenoise (YOND_SIDD.py:301-483, `simple` estimator) for a batch of images: x (nimg, nblk, H, W) CUDA f32 —
         SIDD images of nblk blocks, or full frames with nblk = 1.  Every stage runs once for the whole batch; the noise
-        estimate, the reference's guards, the VST constants, the bias rows and the round-2 selection all stay on the device,
+        estimate, the reference's guards, the VST constants, the bias rows and the per-round selection all stay on the device,
         so nothing is read back until the caller asks for the numbers.
 
-        Returns device tensors: dn1 / final (nimg, H, nblk*W) (the reference's mosaic layout), regs1 / regs2 (nimg, 4) float64
-        = (beta1, beta2 after the guards, gain, sigma) per round (regs2 None without round 2), ok (nimg,) int32 = the round-2
-        result was kept (beta1 >= 0, :445-447).
+        Rounds: round 1 (self estimate) and, with pipe['iter'] == 'iter', pipe['max_iter'] collab rounds (:419-472).  A batch
+        always runs every round on the device: an image whose beta1 < 0 stopped the reference's loop is carried through the
+        later rounds by selection (its output is a copy of its last live round's, its parameters are those of that round), so
+        no round needs a read-back.
+
+        Returns device tensors: dns / regs4 / live = per-round lists of the outputs (nimg, H, nblk*W) (the reference's mosaic
+        layout), (nimg, 4) float64 = (beta1, beta2 after the guards, gain, sigma), and (nimg,) int32 = the image is still live
+        after this round (all ones in round 1).  dn1 / regs1 = round 1, final = the last round, regs2 / ok = round 2 (None without
+        collab rounds).
 
         raw = (black, white, ratio[, clip]): x is the uint16 SENSOR mosaic (16-bit integer tensor) and the dataset normalisation
         (raw - black) * ratio / (white - black) of the 14-bit drivers (data_process/yond_datasets.py:955-961, :1053-1056) is applied
         on load by the estimator and the VST front end — the float32 frame never exists (SURVEY 8(f)-1)."""
         pipe = self.pipe
+        n_collab = collab_rounds(pipe)
         if raw is not None:
             assert x.dtype in (torch.int16, torch.uint16) and lr_full is None
             raw = _lib.RawNorm(float(raw[0]), float(raw[1]), float(raw[2]), int(bool(raw[3])) if len(raw) > 3 else 0)
@@ -487,11 +496,28 @@ class YOND_SIDD:
             mos_blocks, W, nblk = nblk, nblk * W, 1
         else:
             mos_blocks = nblk
+        # Geometry of the collab estimates.  The shipped driver hard-codes SIDD_256 = True (:431): the mosaic is cut into 32 strips
+        # along W that the box filters treat as separate images.  That is the SIDD layout; for plain frames (the drivers of the
+        # other datasets are not in the repository) the default here is one image, `sidd_256: True` in the pipeline dict restores
+        # the hard-coded behaviour (needs W % 64 == 0).
+        sidd = bool(pipe.get("sidd_256", mos_blocks == 32))
+        if n_collab and sidd and nblk == 1:  # a frame (or a full_dn mosaic): the 32 strips are split out of the mosaic layout
+            assert W % 64 == 0, "SIDD_256 splits the packed frame into 32 strips along W (YOND_SIDD.py:91-93)"
+            cx, cnb, c_mosaic = x.reshape(nimg, H, W), 32, True
+        else:
+            cx, cnb, c_mosaic = x, nblk, False
+        # stdfilt(lr, k)**2 in the collab geometry, shared by every collab round: the self estimate's var map when it ran in the same
+        # geometry (not SIDD_256, not on lr_full), else one box pass over lr in round 2
+        reuse = n_collab > 0 and not sidd and lr_full is None and self.reuse_self_var
+        lr_var = None
+        if n_collab:
+            n_el = est.collab_geometry(nimg, cnb, H, W // cnb if c_mosaic else W, sidd)
+            lr_var = eng._buf("lr_var", (n_el,), torch.float32, dev)
         need_max = bias_corr == "pre"
         seg_max = torch.empty(nimg, device=dev, dtype=torch.float32) if need_max else None
         # ---- round 1: self-calibration on the mosaic (:315, :338-341) or on the full-resolution frame when given
         if lr_full is None:
-            regs = est.estimate_dev(x, None, k, split_blocks=False, seg_max=seg_max, raw=raw)
+            regs = est.estimate_dev(x, None, k, split_blocks=False, seg_max=seg_max, raw=raw, var_map=lr_var if reuse else None)
         else:
             assert nimg == 1
             regs = est.estimate_dev(lr_full.reshape(1, 1, *lr_full.shape[-2:]), None, k)
@@ -500,78 +526,80 @@ class YOND_SIDD:
         mark("estimate_self")
         # the bound of a fallback bias table: full_dn round 1 = the frame's max in DN of p['scale'] (:256); everything else
         # lr_raw.max()*(wp-bl) (:393, :449)
-        ch1 = eng.chain_params(regs, seg_max, nimg, nblk, scale_est, scale, scale if full_dn else scale_est, 1, bias_corr, vst_type)
+        ch = eng.chain_params(regs, seg_max, nimg, nblk, scale_est, scale, scale if full_dn else scale_est, 1, bias_corr, vst_type)
         frames = x.reshape(nimg * nblk, H, W)
-        dn1 = torch.empty((nimg, H, nblk * W), device=dev, dtype=torch.float32)
-        eng.vst_denoise_dev(frames, ch1, dn1, frames_per_row=nblk, fps=nblk, raw=raw)
+        out = torch.empty((nimg, H, nblk * W), device=dev, dtype=torch.float32)
+        eng.vst_denoise_dev(frames, ch, out, frames_per_row=nblk, fps=nblk, raw=raw)
         mark("denoise_round1")
-        if after_round1 is not None:  # round 1 is enqueued: a caller may start downloading it under round 2
-            after_round1(dn1)
-        res = {"dn1": dn1, "final": dn1, "regs1": ch1["regs4"], "regs2": None, "ok": None, "lr": x, "nblk": nblk}
-        if pipe.get("iter") == "iter" and pipe["max_iter"] >= 1:
-            assert pipe["max_iter"] == 1, "the shipped configurations use max_iter = 1"
-            # The shipped driver hard-codes SIDD_256 = True (:431): the mosaic is cut into 32 strips along W that the box
-            # filters treat as separate images.  That is the SIDD layout; for plain frames (the drivers of the other
-            # datasets are not in the repository) the default here is one image, `sidd_256: True` in the pipeline dict
-            # restores the hard-coded behaviour (needs W % 64 == 0).
-            sidd = bool(pipe.get("sidd_256", mos_blocks == 32))
-            if sidd and nblk == 1:  # a frame (or a full_dn mosaic): the 32 strips are split out of the mosaic layout
-                assert W % 64 == 0, "SIDD_256 splits the packed frame into 32 strips along W (YOND_SIDD.py:91-93)"
-                regs2 = est.estimate_dev(x.reshape(nimg, H, W), dn1, k, split_blocks=True, x_mosaic=True, y_mosaic=True, nblk=32, raw=raw)
-            else:
-                # (not SIDD_256: the same box-filter geometry as the self estimate above, whose var map is reused)
-                regs2 = est.estimate_dev(x, dn1, k, split_blocks=sidd, y_mosaic=True, raw=raw,  # :431 (mode 'collab')
-                                         reuse_self_var=(not sidd and lr_full is None and self.reuse_self_var))
+        if after_round1 is not None:  # round 1 is enqueued: a caller may start downloading it under the collab rounds
+            after_round1(out)
+        dns, regs4, live = [out], [ch["regs4"]], [ch["ok"]]
+        # ---- rounds 2 .. max_iter + 1: collab estimate on (lr, previous output) (:431), guards, VST denoise, selection (:445-447)
+        for r in range(2, n_collab + 2):
+            if r == 2 and not reuse:
+                est.lr_var_dev(cx, lr_var, k, split_blocks=sidd, x_mosaic=c_mosaic, nblk=cnb, raw=raw)
+            regs = est.estimate_collab_cached(out, lr_var, cnb, k, split_blocks=sidd, y_mosaic=True)
             mark("estimate_collab")
-            ch2 = eng.chain_params(regs2, seg_max, nimg, nblk, scale_est, scale, scale_est, 2, bias_corr, vst_type, prev=ch1)
-            final = torch.empty_like(dn1)
-            eng.vst_denoise_dev(frames, ch2, final, frames_per_row=nblk, fps=nblk, select=True, fallback=dn1, raw=raw)
-            mark("denoise_round2")
-            res.update(final=final, regs2=ch2["regs4"], ok=ch2["ok"])
-        return res
+            ch = eng.chain_params(regs, seg_max, nimg, nblk, scale_est, scale, scale_est, r, bias_corr, vst_type, prev=ch)
+            prev_out, out = out, torch.empty_like(out)
+            eng.vst_denoise_dev(frames, ch, out, frames_per_row=nblk, fps=nblk, select=True, fallback=prev_out, raw=raw)
+            mark(f"denoise_round{r}")
+            dns.append(out)
+            regs4.append(ch["regs4"])
+            live.append(ch["ok"])
+        two = len(dns) > 1
+        return {"dns": dns, "regs4": regs4, "live": live, "dn1": dns[0], "final": dns[-1], "regs1": regs4[0],
+                "regs2": regs4[1] if two else None, "ok": live[1] if two else None, "lr": x, "nblk": nblk}
 
     @staticmethod
     def summary_async(res):
         """Enqueues (on the current stream) the download of a batch's numbers into pinned host memory; read_summary then
         needs no device synchronisation of its own beyond the event the caller waits for."""
         host = {}
-        for k in ("regs1", "regs2", "ok"):
-            t = res.get(k)
-            if t is not None:
-                host[k] = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
-                host[k].copy_(t, non_blocking=True)
+        for key in ("regs4", "live"):
+            host[key] = []
+            for t in res[key]:
+                h = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
+                h.copy_(t, non_blocking=True)
+                host[key].append(h)
         res["host"] = host
 
     @staticmethod
-    def read_summary(res):
-        """One read-back of the numbers of a finished batch: regs per round as (nimg,2) float64 arrays (rows of images whose
-        round 2 was abandoned are NaN in round 2 — the reference does not append them, :445-447), rounds per image."""
+    def host_numbers(res):
+        """The per-round (nimg,4) regs4 and (nimg,) live arrays of a batch as NumPy: from the pinned copies of summary_async, else
+        read back (one small copy per round and list)."""
         host = res.get("host")
-        get = (lambda k: host[k].numpy()) if host is not None else (lambda k: res[k].cpu().numpy())
-        r1 = get("regs1")
-        nimg = r1.shape[0]
-        regs = [r1[:, :2].copy()]
+        src = host if host is not None else res
+        return [t.cpu().numpy() for t in src["regs4"]], [t.cpu().numpy().astype(bool) for t in src["live"]]
+
+    @staticmethod
+    def read_summary(res):
+        """One read-back of the numbers of a finished batch: regs per round as (nimg,2) float64 arrays (rows of images that did
+        not complete a round are NaN in it — the reference does not append them, :445-447), rounds per image (1 + the live
+        collab rounds), and (gain, sigma) per round as (nimg,2) arrays (not masked: the values the estimate gave)."""
+        r4, live = YOND_SIDD.host_numbers(res)
+        nimg = r4[0].shape[0]
+        regs = [r4[0][:, :2].copy()]
+        gains = [r4[0][:, 2:].copy()]
         rounds = np.ones(nimg, np.int64)
-        gains = [r1[:, 2:].copy()]
-        if res["regs2"] is not None:
-            r2 = get("regs2")
-            ok = get("ok").astype(bool)
-            reg2 = r2[:, :2].copy()
-            reg2[~ok] = np.nan
-            regs.append(reg2)
-            gains.append(r2[:, 2:].copy())
-            rounds[ok] = 2
+        for r in range(1, len(r4)):
+            reg = r4[r][:, :2].copy()
+            reg[~live[r]] = np.nan
+            regs.append(reg)
+            gains.append(r4[r][:, 2:].copy())
+            rounds += live[r]
         return regs, rounds, gains
 
     def iter_denoise_batch(self, blocks, p, log=None, timings=None, raw=None):
         """IterDenoise for a BATCH of SIDD-shaped images (or full frames, nblk = 1) at once: blocks (nimg, nblk, H, W) CUDA
         f32.  Same per-image algorithm and guards as the reference (YOND_SIDD.py:301-483); every device stage runs once for
         all images and the host reads back ONE small array at the end.
-        Returns {'raw_dns': [round-1 (nimg,H,nblk*W), final (nimg,H,nblk*W)], 'regs': [(nimg,2) per round; NaN rows in round
-        2 where the beta1 < 0 guard kept the round-1 result], 'rounds': (nimg,) number of denoise rounds each image completed}."""
+        Returns {'raw_dns': [(nimg,H,nblk*W) per round, max_iter + 1 of them], 'regs': [(nimg,2) per round; NaN rows in the
+        rounds an image did not complete (a beta1 < 0 guard kept its previous result)], 'rounds': (nimg,) number of denoise rounds
+        each image completed}.  An image's entries of raw_dns beyond its rounds repeat its last completed round."""
         res = self.iter_denoise_dev(blocks, p, timings=timings, raw=raw)
         regs, rounds, _ = self.read_summary(res)
-        return {"raw_dns": [res["dn1"], res["final"]], "regs": regs, "rounds": rounds, "lr_raw": None, "dev": res}
+        return {"raw_dns": list(res["dns"]), "regs": regs, "rounds": rounds, "lr_raw": None, "dev": res}
 
     def iter_denoise_host(self, host_in, host_out, p, group=8, lanes=1, wait=True, raw=None):
         """End-to-end batched IterDenoise on HOST buffers: host_in (nimg,nblk,H,W) f32 pinned -> host_out (nimg,H,nblk*W) f32
@@ -630,10 +658,11 @@ class YOND_SIDD:
             with torch.cuda.stream(s_out):
                 host_out[a:b].copy_(res["final"], non_blocking=True)
                 self.summary_async(res)
-            for k in ("final", "regs1", "regs2", "ok"):
-                if res.get(k) is not None:
-                    res[k].record_stream(s_out)
+            res["final"].record_stream(s_out)
+            for t in res["regs4"] + res["live"]:
+                t.record_stream(s_out)
             res.pop("lr", None)  # a view of the staging buffer, which is reused
+            res.pop("dns", None)  # only the final round is downloaded: the intermediate rounds' frames are released
             results.append(res)
         out_done = torch.cuda.Event()
         out_done.record(s_out)
@@ -657,20 +686,32 @@ class YOND_SIDD:
         if "simple" not in pipe["est_type"]:
             raise NotImplementedError(f"est_type '{pipe['est_type']}' needs external estimate files / networks (YOND_SIDD.py:316-353)")
         res = self.iter_denoise_dev(blk[None].contiguous(), p, lr_full=lr_full, after_round1=after_round1)
-        if before_summary is not None:  # everything is enqueued; host work placed here overlaps round 2
+        if before_summary is not None:  # everything is enqueued; host work placed here overlaps the collab rounds
             before_summary()
-        regs, rounds, gs = self.read_summary(res)
-        reg = regs[0][0]
-        self._log(f"Self Est: K={gs[0][0, 0]:.4f}, b={gs[0][0, 1]:.4f} (beta1={reg[0]:.3e}, beta2={reg[1]:.3e})")
-        p["gain"], p["sigma"] = gs[0][0, 0], gs[0][0, 1]  # :356
-        raw_dns, out_regs = [res["dn1"][0]], [reg]
-        if res["regs2"] is not None:
-            r2 = res["regs2"].cpu().numpy()[0]
-            p["gain"], p["sigma"] = r2[2], r2[3]  # :442 — set before the guard, like the reference
-            self._log(f"Iter 1 Est: K={r2[2]:.4f}, sigma={r2[3]:.4f} (beta1={r2[0]:.3e}, beta2={r2[1]:.3e})")
-            if rounds[0] == 2:
-                raw_dns.append(res["final"][0])
-                out_regs.append(regs[1][0])
-            else:
+        r4, live = self.host_numbers(res)
+        b1, b2, g, s_ = r4[0][0]
+        self._log(f"Self Est: K={g:.4f}, b={s_:.4f} (beta1={b1:.3e}, beta2={b2:.3e})")
+        p["gain"], p["sigma"] = g, s_  # :356
+        raw_dns, out_regs = [res["dns"][0][0]], [r4[0][0, :2].copy()]
+        # the rounds the reference evaluates: every live collab round and the first one that fails the beta1 guard
+        for r in range(1, len(r4)):
+            b1, b2, g, s_ = r4[r][0]
+            p["gain"], p["sigma"] = g, s_  # :442 — set before the guard, like the reference
+            self._log(f"Iter {r} Est: K={g:.4f}, sigma={s_:.4f} (beta1={b1:.3e}, beta2={b2:.3e})")
+            if not live[r][0]:
                 self._log("Warning!!! Wrong noise level! Backup to iter_0 result.")  # :445-447
+                break
+            raw_dns.append(res["dns"][r][0])
+            out_regs.append(r4[r][0, :2].copy())
         return {"raw_dns": raw_dns, "regs": out_regs, "lr_raw": mosaic}  # lr_raw: a thunk (the mosaic copy is only made on request)
+
+
+def collab_rounds(pipe):
+    """Number of collab rounds IterDenoise runs after round 1 (YOND_SIDD.py:419-472): pipe['max_iter'] with pipe['iter'] == 'iter',
+    else 0.  max_iter must be an integer >= 0 (ValueError otherwise)."""
+    if pipe.get("iter") != "iter":
+        return 0
+    n = pipe.get("max_iter")
+    if isinstance(n, (bool, np.bool_)) or not isinstance(n, (int, np.integer)) or n < 0:
+        raise ValueError(f"pipeline max_iter must be an integer >= 0, got {n!r}")
+    return int(n)
