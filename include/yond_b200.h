@@ -171,25 +171,8 @@ size_t yond_nlf_work_bytes(int B, int h, int w, int C);
 int yond_nlf_maps(const float* x, const float* y, float* var, float* mean, float* lap, int B, int h, int w, int C,
                   int k, int mode, void* work, void* stream);
 
-/* ---- A9: get_threshold(mode='score3') — YOND_SIDD.py:22-49.  All three entry points are batched over `nseg`
- * independent segments (one per image) of `seg_len` contiguous floats each.
- * yond_order_stats: exact k-th smallest values (0-based ranks, shared by all segments, nranks <= 64) by radix select;
- *   out (nseg, nranks).  The host applies np.percentile's linear interpolation in float64.
- *   `work`: yond_select_work_bytes(nseg).
- * yond_score3_bins: npeaks[s][i] = number of occupied bins of int(clip(mean,0,1)*1000) over {lap <= ths[s][i]} (:37-43),
- *   ths ascending per segment (float64, (nseg, nth), nth <= 32).  `work`: >= nseg*1001*4 bytes. */
-size_t yond_select_work_bytes(int nseg);
-int yond_order_stats(const float* data, size_t seg_len, int nseg, const uint64_t* ranks_dev, int nranks, float* out_dev,
-                     void* work, void* stream);
-int yond_score3_bins(const float* lap, const float* mean, size_t seg_len, int nseg, const double* ths_dev, int nth,
-                     int32_t* npeaks_dev, void* work, void* stream);
-/* ---- A10: masked line fit — YOND_SIDD.py:77-78 (strict lap<th), utils/isp_algos.py:345-365.  Per segment s:
- * sums_dev[s][0..5]  = {N, Sx, Sy, Sxx, Sxy, Syy} over {lap < ths_dev[s]};
- * sums_dev[s][6..11] = same over {lap < th, 1e-4 < mean < 0.8} (polyfit's non-saturated subset), float64. */
-int yond_masked_sums(const float* lap, const float* mean, const float* var, size_t seg_len, int nseg,
-                     const double* ths_dev, double* sums_dev, void* stream);
-
-/* ---- the estimator without host round trips (same reference lines as above, arithmetic in float64 on the device) ----
+/* ---- the estimator on the device — A9 get_threshold('score3') YOND_SIDD.py:22-49, A10 masked line fit :77-86 and
+ * utils/isp_algos.py:345-365, in float64 ----
  * yond_nlf_maps_bayer: the maps straight from the Bayer frames (no pack pass).  Inputs are `nimg` images of `nblk`
  *   blocks of (H,W) each, in the blocks layout (nimg,nblk,H,W) (`*_mosaic` = 0, the SIDD dataset layout) or the mosaic
  *   layout (nimg,H,nblk*W) (`*_mosaic` = 1, np.concatenate(blocks, -1) of YOND_SIDD.py:315/:408).  split_blocks = 0: an
@@ -197,16 +180,15 @@ int yond_masked_sums(const float* lap, const float* mean, const float* var, size
  *   split_blocks = 1: every block is its own image (SIDD_256, :65,:91-93).  Maps come out packed, (B,h,w,4) with
  *   B = nimg*nblk / w = W/2 (split) or B = nimg / w = nblk*W/2.  `seg_max` (optional, nimg floats): max(x, 0) per image
  *   of the first input — the bound of the fallback bias table (:393, isp_algos.py:101).  `work`: yond_nlf_work_bytes(B,h,w,4).
- *   mode 0: self maps (y unused); 1: collab maps; 2: collab maps where `var` holds, on entry, the var map of the SELF estimate of
- *   the same frames in the same geometry — SelfNLF's var is stdfilt(lr, k)**2 and CollabNLF starts from the very same float32
- *   expression (:66-68, :94-97), so the pass over x is skipped and `var` is updated in place (x is not read); 3: var =
- *   stdfilt(x, k)**2 alone (y, mean, lap untouched): the noisy-frame statistics every collab round of IterDenoise shares.
+ *   mode 0: self maps (y unused); 1: collab maps; 3: var = stdfilt(x, k)**2 alone (y, mean, lap untouched): the noisy-frame
+ *   statistics every collab round of IterDenoise shares.  Any other mode is rejected with YOND_ERR_INVALID.
  * yond_nlf_maps_collab_cached: the collab maps of a round from a cached `lr_var` = stdfilt(lr, k)**2 in the same geometry (the
- *   var map of mode 0 or mode 3; read only, may be `var` itself = mode 2): var = lr_var - stdfilt(y, k)**2, mean = blur_k(y),
+ *   var map of mode 0 or mode 3; read only, may be `var` itself): var = lr_var - stdfilt(y, k)**2, mean = blur_k(y),
  *   lap = stdfilt(y, k), one box pass over the float32 frame y (layout / geometry arguments as above).  The noisy frame is not
  *   an argument, so the call is the same for float32 and uint16 sensor inputs.
  * yond_nlf_fit: percentiles -> score3 threshold -> masked sums (with the empty-mask fallbacks of :77-84) -> line fit,
- *   per segment, all on the device: regs_dev (nseg,2) float64 = (beta1, beta2).  `quants_host`: the nq <= 24 ascending
+ *   per segment, all on the device: regs_dev (nseg,2) float64 = (beta1, beta2).
+ *   The order statistics behind the percentiles are exact, computed by radix select.  `quants_host`: the nq <= 24 ascending
  *   percentiles of get_threshold (np.linspace(step,100,100//step)).  detail_dev (optional, (nseg, 52) float64):
  *   th, index, percent, redo flag, ths[24], npeaks[24].  `work`: yond_nlf_fit_work_bytes(nseg), 256-byte aligned. */
 int yond_nlf_maps_bayer(const float* x, int x_mosaic, const float* y, int y_mosaic, float* var, float* mean, float* lap,

@@ -1,5 +1,5 @@
 """CPU tests (no GPU): the C-ABI library loads and exports every symbol include/yond_b200.h declares, the host-side
-logic (state-dict layout, FLOP accounting, percentile interpolation, padding math, sharding) is right, and the product
+logic (state-dict layout, FLOP accounting, padding math, sharding) is right, and the product
 path refuses to run without CUDA (no CPU fallback)."""
 import ctypes as C
 import os
@@ -140,18 +140,16 @@ def test_unknown_arch_and_key_rejected(Y):
     lib.yond_net_destroy(h)
 
 
-def test_percentile_lerp_matches_numpy(Y):
-    from yond_public_b200.nlf import _percentiles_from_order_stats
-    rng = np.random.default_rng(0)
-    for n in (10, 1000, 65537):
-        d = rng.random(n).astype(np.float32) ** 3
-        q = np.linspace(5, 100, 20)
-        qq = np.true_divide(q, 100)
-        vi = (n - 1) * qq
-        lo = np.floor(vi).astype(np.int64)
-        hi = np.minimum(lo + 1, n - 1)
-        sd = np.sort(d)
-        assert np.array_equal(_percentiles_from_order_stats(sd[lo], sd[hi], vi - lo), np.percentile(d, q, method="linear"))
+def test_nlf_maps_modes_checked(Y):
+    """yond_nlf_maps_bayer / _raw16 take modes 0, 1 and 3 only; any other mode is refused before device work (YOND_ERR_INVALID)."""
+    lib = Y._lib.load()
+    buf = C.c_void_p(256)  # never dereferenced: the arguments are checked first
+    nrm = Y._lib.RawNorm(64.0, 1023.0, 1.0, 0)
+    for mode in (2, 4, -1):
+        assert lib.yond_nlf_maps_bayer(buf, 1, buf, 1, buf, buf, buf, 1, 1, 64, 64, 0, 29, mode, None, buf, None) == 1
+        assert b"mode" in lib.yond_last_error()
+        assert lib.yond_nlf_maps_raw16(buf, C.byref(nrm), 1, buf, 1, buf, buf, buf, 1, 1, 64, 64, 0, 29, mode, None, buf, None) == 1
+        assert b"mode" in lib.yond_last_error()
 
 
 def test_host_math_matches_oracle(Y, golden):

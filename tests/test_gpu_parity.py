@@ -114,19 +114,21 @@ def test_blur_stdfilt_golden(Y, golden):
 
 
 @pytest.mark.parametrize("n", [1000, 65536, 3_000_004])
-def test_order_stats_and_percentiles_exact(Y, n):
+def test_fit_percentiles_exact(Y, n):
     from yond_public_b200.nlf import NlfEstimator
     rng = np.random.default_rng(n)
     d = (rng.random(n).astype(np.float32) ** 3) * 0.2
     d[::7] = d[3]  # ties
     est = NlfEstimator()
     q = np.linspace(5, 100, 20)
-    got = est.percentiles(torch.from_numpy(d).cuda(), q)
+    lap = torch.from_numpy(d).cuda()
+    _, detail = est._fit(torch.zeros_like(lap), torch.rand_like(lap), lap, 1, details=True)
+    got = detail[0, 4:24].cpu().numpy()  # the percentiles of get_threshold, from the exact order statistics
     assert np.array_equal(got, np.percentile(d, q, method="linear"))
-    assert est.percentiles(torch.from_numpy(d).cuda(), [25.0])[0] == np.percentile(d, 25, method="linear")
+    assert got[list(q).index(25.0)] == np.percentile(d, 25, method="linear")
 
 
-def test_estimator_self_and_collab_golden(Y, golden):
+def test_nlf_fit_self_and_collab_golden(Y, golden):
     g = golden("nlf")
     r2 = np.random.default_rng(int(g["seed"]))
     clean = O.synth_clean(r2, 256, 384)
@@ -138,11 +140,12 @@ def test_estimator_self_and_collab_golden(Y, golden):
     np.testing.assert_allclose(mean[0].cpu().numpy()[::16, ::16], g["mean_sub"], rtol=0, atol=6e-8)
     np.testing.assert_allclose(var[0].cpu().numpy()[::16, ::16], g["var_sub"], rtol=0, atol=1e-7)
     np.testing.assert_allclose(lap[0].cpu().numpy()[::16, ::16], g["lap_sub"], rtol=0, atol=5e-7)
-    th, pct, info = est.threshold_score3(lap, mean)
+    _, detail = est._fit(var, mean, lap, 1, details=True)
+    d = detail.cpu().numpy()
     _, _, oinfo = O.get_threshold_score3(*[a for a in O.self_maps(O.bayer2rggb(noisy), 29)[2:0:-1]])
-    assert pct == float(g["pct"])
-    np.testing.assert_allclose(th, float(g["th"]), rtol=1e-6)
-    np.testing.assert_array_equal(info["npeaks"], oinfo["npeaks"])
+    assert d[0, 2] == float(g["pct"])
+    np.testing.assert_allclose(d[0, 4 + int(d[0, 1])], float(g["th"]), rtol=1e-6)  # the score3 threshold
+    np.testing.assert_array_equal(d[0, 28:48], oinfo["npeaks"])
     reg = Y.SimpleNLF(noisy, k=29, setting={"mode": "self"})
     np.testing.assert_allclose(reg, g["reg_self"], rtol=TOL_EST)
     blocks_c = np.stack([O.synth_clean(r2, 64, 64) for _ in range(32)])
@@ -151,6 +154,18 @@ def test_estimator_self_and_collab_golden(Y, golden):
     mos_n, mos_d = np.concatenate(list(blocks_n), -1), np.concatenate(list(blocks_d), -1)
     np.testing.assert_allclose(Y.SimpleNLF(mos_n, mos_d, 29, {"mode": "collab", "SIDD_256": True}), g["reg_collab"], rtol=TOL_EST)
     np.testing.assert_allclose(Y.SimpleNLF(mos_n, mos_d, 29, {"mode": "collab"}), g["reg_collab_plain"], rtol=TOL_EST)
+    # the public packed-input estimators on the same mosaic: against the oracle, and against SimpleNLF (same maps, same tail)
+    lr, hr = O.bayer2rggb(mos_n), O.bayer2rggb(mos_d)
+    for kw in ({}, {"SIDD_256": True}):
+        sidd = bool(kw)
+        got = Y.SelfNLF(lr, 29, kw)
+        assert got.shape == (2,) and got.dtype == np.float64
+        np.testing.assert_allclose(got, O.SelfNLF(lr, 29, sidd), rtol=TOL_EST)
+        np.testing.assert_allclose(got, Y.SimpleNLF(mos_n, None, 29, {"mode": "self", **kw}), rtol=1e-12)
+        got = Y.CollabNLF(lr, hr, 29, kw)
+        assert got.shape == (2,) and got.dtype == np.float64
+        np.testing.assert_allclose(got, O.CollabNLF(lr, hr, 29, sidd), rtol=TOL_EST)
+        np.testing.assert_allclose(got, Y.SimpleNLF(mos_n, mos_d, 29, {"mode": "collab", **kw}), rtol=1e-12)
 
 
 def test_estimator_12mp_frame_vs_oracle(Y):
@@ -370,7 +385,7 @@ def test_iterdenoise_golden_two_rounds(Y, golden, key):
     np.testing.assert_allclose(np.asarray(res["regs"][0]), g["regs"][0], rtol=TOL_EST)
     # The round-2 (collab) estimate is a function of OUR round-1 output, which differs from the reference's by the
     # bf16 conv stack (<= 2e-3 allowed, ~1e-5 here); the 1e-4 bar applies to identical inputs and is checked on
-    # identical inputs in test_estimator_self_and_collab_golden.  Here only input-perturbation-sized drift is allowed.
+    # identical inputs in test_nlf_fit_self_and_collab_golden.  Here only input-perturbation-sized drift is allowed.
     np.testing.assert_allclose(np.asarray(res["regs"][1]), g["regs"][1], rtol=2e-3)
     assert float(np.abs(res["raw_dns"][0][::8, ::8] - g["dn0_sub"]).max()) < TOL_ABS
     assert float(np.abs(res["raw_dns"][1][::8, ::8] - g["dn1_sub"]).max()) < TOL_ABS
@@ -472,19 +487,11 @@ def test_full_frame_identity_roundtrip(Y):
 
 
 # ------------------------------------------------------------------ device-resident estimator tail and parameter chain
-def _host_tail(est, var, mean, lap, nseg):
-    th, pct, info = est.threshold_score3(lap, mean, step=5, nseg=nseg)
-    reg, th2 = est.masked_fit(var, mean, lap, th, nseg=nseg)
-    return np.atleast_2d(reg), np.atleast_1d(th2), np.atleast_1d(pct), {k: np.atleast_2d(v) for k, v in info.items()}
-
-
 @pytest.mark.parametrize("case", ["noise", "ties", "flat"])
-def test_device_estimator_tail_equals_host_path(Y, case):
-    """yond_nlf_fit (percentile lerp, score3 argmin, empty-mask fallbacks, line fit — all on the device) against the
-    host-scalar path of the same maps: thresholds and bin counts identical, (beta1, beta2) to 1e-10."""
+def test_device_estimator_tail_equals_oracle(Y, case):
+    """yond_nlf_fit (percentile lerp, score3 argmin, empty-mask fallbacks, line fit — all on the device) against the oracle's
+    get_threshold_score3 + _masked_fit on each segment: percentiles, bin counts and thresholds identical, (beta1, beta2) to 1e-10."""
     from yond_public_b200.nlf import NlfEstimator
-    from yond_public_b200._lib import check, ptr, stream_ptr
-    import ctypes as C
     rng = np.random.default_rng(17)
     nseg, n = 3, 64 * 96 * 4
     lap = (rng.random((nseg, n)).astype(np.float32) ** 2) * 0.05
@@ -496,25 +503,21 @@ def test_device_estimator_tail_equals_host_path(Y, case):
         lap[1] = 0.25          # constant: th = min, the strict mask is empty and the 25th percentile equals th -> unmasked fit
         lap[2, : n // 2] = 0.0  # th25 == th == 0 as well
     est = NlfEstimator()
-    tv, tm, tl = (torch.from_numpy(a).cuda() for a in (var, mean, lap))
-    reg_h, th_h, pct_h, info = _host_tail(est, tv, tm, tl, nseg)
-    lib = Y._lib.load()
-    quants = np.ascontiguousarray(np.linspace(5, 100, 20), np.float64)
-    regs = torch.empty((nseg, 2), device="cuda", dtype=torch.float64)
-    detail = torch.empty((nseg, est.DETAIL), device="cuda", dtype=torch.float64)
-    work = torch.empty(lib.yond_nlf_fit_work_bytes(nseg) + 256, device="cuda", dtype=torch.uint8)
-    off = (-work.data_ptr()) % 256
-    check(lib.yond_nlf_fit(ptr(tv), ptr(tm), ptr(tl), n, nseg, quants.ctypes.data_as(C.POINTER(C.c_double)), 20, ptr(regs), ptr(detail),
-                           ptr(work[off:]), stream_ptr()))
-    d = detail.cpu().numpy()
-    assert np.array_equal(d[:, 4:24], info["ths"])
-    assert np.array_equal(d[:, 28:48], info["npeaks"])
-    assert np.array_equal(d[:, 2], pct_h)
-    assert np.array_equal(d[:, 0], th_h)
-    np.testing.assert_allclose(regs.cpu().numpy(), reg_h, rtol=1e-10)
-    for s in range(nseg):  # and the host path itself against NumPy / the oracle's fit
-        ths = np.percentile(lap[s], quants, method="linear")
-        assert np.array_equal(d[s, 4:24], ths)
+    regs, detail = est._fit(*(torch.from_numpy(a).cuda() for a in (var, mean, lap)), nseg, details=True)
+    regs, d = regs.cpu().numpy(), detail.cpu().numpy()
+    for s in range(nseg):
+        th, pct, info = O.get_threshold_score3(lap[s], mean[s], step=5)
+        reg, th_fit = O._masked_fit(var[s], mean[s], lap[s], th)
+        assert np.array_equal(d[s, 4:24], info["ths"])
+        assert np.array_equal(d[s, 28:48], info["npeaks"])
+        assert d[s, 2] == pct
+        if not (lap[s] < th).any() and th_fit == th:
+            assert d[s, 0] == np.inf  # the reference keeps the unmasked maps: the device fits with threshold +inf
+        else:
+            assert d[s, 0] == th_fit
+        np.testing.assert_allclose(regs[s], reg, rtol=1e-10)
+    if case == "flat":
+        assert d[1, 0] == np.inf
 
 
 @pytest.mark.parametrize("img_max,sig,K", [(700.0, 6.0, 4.0), (40.0, 0.9, 0.4), (961.0, 31.0, 2.9), (30.2, 0.8, 0.31), (333.0, 0.0, 1.0),
@@ -858,7 +861,7 @@ def test_c4_frame_golden(Y, golden, lut_table, ratio, wname):
     np.testing.assert_allclose(np.asarray(res["regs"][0]), regs[0], rtol=TOL_EST)
     if nrounds == 2:
         # round 2 estimates var = std(lr)^2 - std(dn)^2 from OUR round-1 output (bf16 conv stack, <= 2e-3 allowed): the 1e-4
-        # bar applies to identical inputs (checked above and in test_estimator_self_and_collab_golden); here the drift of a
+        # bar applies to identical inputs (checked above and in test_nlf_fit_self_and_collab_golden); here the drift of a
         # cancelling difference under input perturbation is bounded
         np.testing.assert_allclose(np.asarray(res["regs"][1]), regs[1], rtol=1e-2)
     hard = (ratio, wname) == (100, "mix")

@@ -57,10 +57,6 @@ SIGNATURES = {
     "yond_box_blur": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _P, _P]),
     "yond_nlf_work_bytes": (_SZ, [_I, _I, _I, _I]),
     "yond_nlf_maps": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _P]),
-    "yond_select_work_bytes": (_SZ, [_I]),
-    "yond_order_stats": (_I, [_P, _SZ, _I, _P, _I, _P, _P, _P]),
-    "yond_score3_bins": (_I, [_P, _P, _SZ, _I, _P, _I, _P, _P, _P]),
-    "yond_masked_sums": (_I, [_P, _P, _P, _SZ, _I, _P, _P, _P]),
     "yond_nlf_maps_bayer": (_I, [_P, _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
     "yond_nlf_maps_raw16": (_I, [_P, C.POINTER(RawNorm), _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
     "yond_nlf_maps_collab_cached": (_I, [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),

@@ -773,7 +773,7 @@ __global__ void __launch_bounds__(256) masked_sums_kernel(const float* __restric
 // Everything the reference does on a few dozen scalars per image after the maps (YOND_SIDD.py:22-49 np.percentile lerp,
 // score, argmin; :77-84 empty-mask fallback; utils/isp_algos.py:345-365 polyfit) as tiny float64 kernels, so that the
 // estimate never leaves the GPU.  Arithmetic follows NumPy operation by operation (explicit round-to-nearest mul / add /
-// div: no FMA contraction), so thresholds are the same doubles the host path (nlf.py) computes.
+// div: no FMA contraction), so thresholds are the same doubles np.percentile computes (oracle/yond_oracle.py).
 constexpr int kMaxQ = 24;
 struct QuantList {
   int nq;
@@ -962,9 +962,10 @@ int nlf_maps_impl(const BoxSrc& x, const BoxSrc* y, bool bayer, float* var, floa
   float* tmpB = tmpA + n;
   int rc;
   // algorithmic bytes per Bayer pixel (SURVEY 8d): self 4 R + 12 W (lap, mean, var), collab 8 R + 12 W, lr var 4 R + 4 W
-  static const char* names[4] = {"nlf_maps_self (3 box_fused passes)", "nlf_maps_collab (2 box_fused passes)",
-                                 "nlf_maps_collab (1 box_fused pass, lr statistics reused)", "nlf_maps_lr_var (1 box_fused pass)"};
-  static const double bytes[4] = {16.0, 20.0, 20.0, 8.0};
+  // Indexed by mode; there is no mode 2, so modes 1 and 3 keep the numbers of the C entry points.
+  static const char* names[4] = {"nlf_maps_self (3 box_fused passes)", "nlf_maps_collab (2 box_fused passes)", nullptr,
+                                 "nlf_maps_lr_var (1 box_fused pass)"};
+  static const double bytes[4] = {16.0, 20.0, 0.0, 8.0};
   YondProfScope prof(names[mode], s, bytes[mode] * (double)n);
   BoxSrc x_nomax = x;
   x_nomax.seg_max = nullptr;
@@ -975,10 +976,6 @@ int nlf_maps_impl(const BoxSrc& x, const BoxSrc* y, bool bayer, float* var, floa
     const int k2 = k / 3 * 2 + 1;
     if ((rc = box_pass(x_nomax, bayer, tmpB, nullptr, B, h, w, k2, false, OP_MEAN, s))) return rc;
     if ((rc = box_pass(packed_src(tmpB, h, w), false, lap, nullptr, B, h, w, k, true, OP_STD, s))) return rc;
-  } else if (mode == 2) {
-    // `var` holds std_k(lr)^2 from the self estimate of the same frames (SelfNLF's var map IS stdfilt(lr, k)**2, YOND_SIDD.py:66-68 /
-    // :94-97: the same float32 expression): only the statistics of the denoised frame are new, `var` is updated in place
-    if ((rc = collab_from_lr_var(*y, bayer, var, var, mean, lap, B, h, w, k, s))) return rc;
   } else if (mode == 3) {
     // var = std_k(x)^2 alone: the cached lr statistics of the collab rounds (mean / lap untouched)
     if ((rc = box_pass(x, bayer, var, nullptr, B, h, w, k, true, OP_VAR, s))) return rc;
@@ -1050,7 +1047,7 @@ static int nlf_maps_bayer_impl(const float* x, const uint16_t* x16, const yond_r
   YOND_REQUIRE(!x16 || (nrm && nrm->white > nrm->black && (uintptr_t)x16 % 4 == 0), "yond_nlf_maps_raw16: normalisation / 4-byte aligned mosaic required");
   YOND_REQUIRE(nimg > 0 && nblk > 0 && H > 0 && W > 0 && H % 2 == 0 && W % 2 == 0, "yond_nlf_maps_bayer: H,W must be even");
   YOND_REQUIRE(k % 2 == 1 && k >= 3 && k <= kMaxK, "yond_nlf_maps_bayer: odd k <= %d required (got %d)", kMaxK, k);
-  YOND_REQUIRE(mode == 0 || mode == 3 || ((mode == 1 || mode == 2) && y != nullptr), "yond_nlf_maps_bayer: mode 0..3, collab modes need the second input");
+  YOND_REQUIRE(mode == 0 || mode == 3 || (mode == 1 && y != nullptr), "yond_nlf_maps_bayer: mode 0, 1 or 3, the collab mode needs the second input");
   YOND_REQUIRE((!x || (uintptr_t)x % 8 == 0) && (!y || (uintptr_t)y % 8 == 0), "yond_nlf_maps_bayer: 8-byte aligned frames required");
   cudaStream_t s = (cudaStream_t)stream;
   const int h = H / 2, wb = W / 2;
@@ -1096,11 +1093,10 @@ int yond_nlf_maps_collab_cached(const float* y, int y_mosaic, const float* lr_va
   return collab_from_lr_var(bayer_src(y, y_mosaic, nblk, H, W, split_blocks), true, lr_var, var, mean, lap, B, h, w, k, s);
 }
 
-size_t yond_select_work_bytes(int nseg) { return (size_t)(nseg < 1 ? 1 : nseg) * sizeof(SelectWork) + 256; }
-
 }  // extern "C"
+
 namespace {
-// data = lap; with `mean` + `binmin` the first counting pass also collects the per-bin minimum of lap (score3)
+// data = lap; the first counting pass also collects the per-bin minimum of lap over the `mean` bins (score3) into `binmin`
 int order_stats_impl(const float* data, const float* mean, unsigned int* binmin, size_t seg_len, int nseg, const uint64_t* ranks_dev,
                      int nranks, float* out_dev, void* work, cudaStream_t s) {
   SelectWork* wk = reinterpret_cast<SelectWork*>(work);
@@ -1109,13 +1105,10 @@ int order_stats_impl(const float* data, const float* mean, unsigned int* binmin,
   dim3 g(stream_grid(seg_len), nseg);
   if ((size_t)g.x * nseg > (size_t)yond_num_sms() * 16) g.x = (unsigned)((yond_num_sms() * 16 + nseg - 1) / nseg);
   const double nel = (double)seg_len * nseg;
-  if (binmin) {
-    YOND_CUDA_CHECK(cudaMemsetAsync(binmin, 0xff, (size_t)nseg * 1024 * sizeof(unsigned int), s));
+  YOND_CUDA_CHECK(cudaMemsetAsync(binmin, 0xff, (size_t)nseg * 1024 * sizeof(unsigned int), s));
+  {
     YondProfScope prof("hist0+score3_binmin", s, 8.0 * nel);
     hist0_kernel<true><<<g, 256, 0, s>>>(data, mean, seg_len, wk, binmin);
-  } else {
-    YondProfScope prof("hist0", s, 4.0 * nel);
-    hist0_kernel<false><<<g, 256, 0, s>>>(data, nullptr, seg_len, wk, nullptr);
   }
   YOND_LAUNCH_CHECK();
   select0_kernel<<<nseg, 1024, 0, s>>>(wk, reinterpret_cast<const unsigned long long*>(ranks_dev), nranks);
@@ -1155,42 +1148,11 @@ int order_stats_impl(const float* data, const float* mean, unsigned int* binmin,
   YOND_LAUNCH_CHECK();
   return YOND_OK;
 }
-}  // namespace
-extern "C" {
 
-int yond_order_stats(const float* data, size_t seg_len, int nseg, const uint64_t* ranks_dev, int nranks, float* out_dev,
-                     void* work, void* stream) {
-  YOND_REQUIRE(nranks > 0 && nranks <= kMaxRanks, "yond_order_stats: 1..%d ranks (got %d)", kMaxRanks, nranks);
-  YOND_REQUIRE(seg_len > 0 && seg_len < 0xffffffffull && nseg > 0 && nseg <= 65535, "yond_order_stats: 1 .. 2^32-2 elements per segment");
-  YOND_REQUIRE(seg_len % 4 == 0 && (uintptr_t)data % 16 == 0, "yond_order_stats: segments must hold whole 4-channel pixels (16-byte aligned)");
-  return order_stats_impl(data, nullptr, nullptr, seg_len, nseg, ranks_dev, nranks, out_dev, work, (cudaStream_t)stream);
-}
-
-int yond_score3_bins(const float* lap, const float* mean, size_t seg_len, int nseg, const double* ths_dev, int nth,
-                     int32_t* npeaks_dev, void* work, void* stream) {
-  YOND_REQUIRE(nth > 0 && nth <= 32, "yond_score3_bins: 1..32 thresholds (got %d)", nth);
-  YOND_REQUIRE(nseg > 0 && nseg <= 65535, "yond_score3_bins: bad segment count");
-  YOND_REQUIRE(seg_len % 4 == 0 && (uintptr_t)lap % 16 == 0 && (uintptr_t)mean % 16 == 0, "yond_score3_bins: 4-channel pixel segments required");
-  cudaStream_t s = (cudaStream_t)stream;
-  unsigned int* binmin = reinterpret_cast<unsigned int*>(work);
-  YOND_CUDA_CHECK(cudaMemsetAsync(binmin, 0xff, (size_t)nseg * 1024 * sizeof(unsigned int), s));
-  dim3 g(stream_grid(seg_len), nseg);
-  if ((size_t)g.x * nseg > (size_t)yond_num_sms() * 16) g.x = (unsigned)((yond_num_sms() * 16 + nseg - 1) / nseg);
-  {
-    YondProfScope prof("score3_binmin", s, 8.0 * (double)seg_len * nseg);
-    hist0_kernel<true><<<g, 256, 0, s>>>(lap, mean, seg_len, nullptr, binmin);
-  }
-  YOND_LAUNCH_CHECK();
-  score3_count_kernel<<<nseg, 256, 0, s>>>(binmin, ths_dev, nth, npeaks_dev);
-  YOND_LAUNCH_CHECK();
-  return YOND_OK;
-}
-
-int yond_masked_sums(const float* lap, const float* mean, const float* var, size_t seg_len, int nseg, const double* ths_dev,
-                     double* sums_dev, void* stream) {
-  YOND_REQUIRE(nseg > 0 && nseg <= 65535, "yond_masked_sums: bad segment count");
-  YOND_REQUIRE(seg_len % 4 == 0, "yond_masked_sums: 4-channel pixel segments required");
-  cudaStream_t s = (cudaStream_t)stream;
+// sums_dev[s][0..5] = {N, Sx, Sy, Sxx, Sxy, Syy} over {lap < ths_dev[s]} (YOND_SIDD.py:77-78, strict), [6..11] the same over
+// {lap < th, 1e-4 < mean < 0.8} (polyfit's non-saturated subset, utils/isp_algos.py:348-350), float64
+int masked_sums(const float* lap, const float* mean, const float* var, size_t seg_len, int nseg, const double* ths_dev, double* sums_dev,
+                cudaStream_t s) {
   YOND_CUDA_CHECK(cudaMemsetAsync(sums_dev, 0, (size_t)nseg * 12 * sizeof(double), s));
   dim3 g(stream_grid(seg_len), nseg);
   if ((size_t)g.x * nseg > (size_t)yond_num_sms() * 16) g.x = (unsigned)((yond_num_sms() * 16 + nseg - 1) / nseg);
@@ -1202,10 +1164,7 @@ int yond_masked_sums(const float* lap, const float* mean, const float* var, size
   return YOND_OK;
 }
 
-
 // Scratch of yond_nlf_fit: the radix-select tables + a few hundred bytes of scalars per segment.
-}  // extern "C"
-namespace {
 struct FitWork {
   SelectWork* sel;
   unsigned long long* ranks;
@@ -1242,6 +1201,7 @@ FitWork carve_fit(void* base, int nseg) {
   return w;
 }
 }  // namespace
+
 extern "C" {
 
 size_t yond_nlf_fit_work_bytes(int nseg) { return carve_fit(nullptr, nseg < 1 ? 1 : nseg).bytes + 256; }
@@ -1273,7 +1233,7 @@ int yond_nlf_fit(const float* var, const float* mean, const float* lap, size_t s
   YOND_LAUNCH_CHECK();
   pick_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(ql, w.ths, w.npeaks, w.th, w.idx, nseg);
   YOND_LAUNCH_CHECK();
-  if ((rc = yond_masked_sums(lap, mean, var, seg_len, nseg, w.th, w.sums, stream))) return rc;
+  if ((rc = masked_sums(lap, mean, var, seg_len, nseg, w.th, w.sums, s))) return rc;
   backup_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(w.sums, w.th, w.th25, w.th2, w.redo, w.sums2, nseg);
   YOND_LAUNCH_CHECK();
   {  // second pass: only the segments whose mask came out empty do any work
