@@ -138,10 +138,13 @@ int yond_vst_fwd(const float* bayer, float* z, float* ub, int B, int H, int W, i
                  int pad_b, const yond_vst_params* params_dev, const float* rows, const float* xnodes,
                  int row_stride, void* stream);
 /* The same front end reading the uint16 sensor mosaic (B,H,W) and normalising it on load (SURVEY 8(f)-1: 2 B/px reads; the
- * float32 frame of data_process/yond_datasets.py:955-961 / :1053-1056 never exists in memory). */
+ * float32 frame of data_process/yond_datasets.py:955-961 / :1053-1056 never exists in memory).  `nrm` (HOST) applies to every frame.
+ * nrm_dev (optional, DEVICE, one entry per image of frames_per_img consecutive frames; may be NULL): frame b is normalised with
+ * nrm_dev[b / frames_per_img] instead (per-image white / black level / ratio of a mixed batch, same float32 arithmetic; `nrm`
+ * may then be NULL).  The call must start at an image boundary: pass the entry of its first image. */
 int yond_vst_fwd_raw16(const uint16_t* raw, const yond_raw_norm* nrm, float* z, float* ub, int B, int H, int W, int pad_l, int pad_r,
                        int pad_t, int pad_b, const yond_vst_params* params_dev, const float* rows, const float* xnodes, int row_stride,
-                       void* stream);
+                       void* stream, const yond_raw_norm* nrm_dev, int frames_per_img);
 /* ---- A18 back half (YOND_SIDD.py:286,289-298, caller's clip :389/:406): y (B,hp,wp,4) f32 -> clamp(0,1) -> crop ->
  * de-normalise -> inverse VST -> unpack -> /scale -> [clip 0..1] -> Bayer (B,H,W) f32. */
 int yond_vst_inv(const float* y, float* bayer, int B, int H, int W, int pad_l, int pad_r, int pad_t, int pad_b,
@@ -195,10 +198,16 @@ int yond_nlf_maps_bayer(const float* x, int x_mosaic, const float* y, int y_mosa
                         int nimg, int nblk, int H, int W, int split_blocks, int k, int mode, float* seg_max, void* work,
                         void* stream);
 /* The same maps with the FIRST input given as the uint16 sensor mosaic, normalised on load (the second input of the collab mode is
- * the float32 output of round 1). */
+ * the float32 output of round 1).  `nrm` (HOST) applies to every image.
+ * yond_nlf_maps_raw16_per_image: the same with `nrm_dev`, a DEVICE array of nimg entries: image i (with split_blocks, every block
+ *   of image i) is normalised with nrm_dev[i] — the per-image white / black level / ratio of a mixed batch, same float32
+ *   arithmetic.  A separate entry point, so that bindings of yond_nlf_maps_raw16 keep their argument list. */
 int yond_nlf_maps_raw16(const uint16_t* x, const yond_raw_norm* nrm, int x_mosaic, const float* y, int y_mosaic, float* var, float* mean,
                         float* lap, int nimg, int nblk, int H, int W, int split_blocks, int k, int mode, float* seg_max, void* work,
                         void* stream);
+int yond_nlf_maps_raw16_per_image(const uint16_t* x, const yond_raw_norm* nrm_dev, int x_mosaic, const float* y, int y_mosaic,
+                                  float* var, float* mean, float* lap, int nimg, int nblk, int H, int W, int split_blocks, int k,
+                                  int mode, float* seg_max, void* work, void* stream);
 int yond_nlf_maps_collab_cached(const float* y, int y_mosaic, const float* lr_var, float* var, float* mean, float* lap, int nimg,
                                 int nblk, int H, int W, int split_blocks, int k, void* stream);
 size_t yond_nlf_fit_work_bytes(int nseg);
@@ -216,6 +225,10 @@ int yond_nlf_fit(const float* var, const float* mean, const float* lap, size_t s
  *   applied, like the reference).  lut2d (nx,nsg) f32 + sg_lut_dev (nsg) f64 + x_lut_dev (nx) f32: the BiasLUT, or NULL:
  *   then — and for sigma/K beyond the table — the numeric table up to bound = seg_max[s]*bound_scale (float32 product).
  *   regs_out (optional, (nseg,4) f64): beta1, beta2 (after the guard), gain, sigma.  `work`: yond_chain_work_bytes(nseg).
+ *   seg_scales_dev (optional, DEVICE, (nseg,3) f64; may be NULL): per image (scale_est, scale, bound_scale), replacing the scalar
+ *   arguments of the same names: a batch of images with their own white / black levels and ratios.  gain = beta1*scale_est,
+ *   sigma = sqrt(beta2)*scale_est, VST(scale), q.scale = scale, the fallback table bound seg_max[s]*bound_scale.  An array of equal
+ *   entries gives the same bits as the scalar call.
  * yond_bias_table: get_bias(bound, sigma, gain) nodes / values (float32, `cap` entries available) for one parameter
  *   set; n_nodes_dev receives the node count (= yond_bias_table_nodes(bound), a host-side helper). */
 size_t yond_chain_work_bytes(int nseg);
@@ -225,7 +238,7 @@ int yond_vst_params_fill(const double* regs_dev, const float* seg_max_dev, int n
                          const double* sg_lut_dev, const float* x_lut_dev, int nx, int nsg,
                          const yond_vst_params* prev_params, yond_vst_params* params_dev, float* t_dev, float* rows,
                          float* xnodes, int row_stride, double* regs_out, int32_t* ok_dev, void* work, void* stream,
-                         const int32_t* prev_ok);
+                         const int32_t* prev_ok, const double* seg_scales_dev);
 int yond_bias_table(double gain, double sigma, float bound, float* nodes_dev, float* vals_dev, int cap,
                     int32_t* n_nodes_dev, void* work, void* stream);
 /* get_bias_points(lams, K, sigGs, pho_min, close_form=True) (isp_algos.py:142-160): the bias at explicit float64 points

@@ -50,7 +50,7 @@ SIGNATURES = {
     "yond_lut_apply": (_I, [_P, _P, _SZ, _P, _P, _I, _D, _D, _P]),
     "yond_table_apply": (_I, [_P, _P, _SZ, _P, _P, _I, _P]),
     "yond_vst_fwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P]),
-    "yond_vst_fwd_raw16": (_I, [_P, C.POINTER(RawNorm), _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P]),
+    "yond_vst_fwd_raw16": (_I, [_P, C.POINTER(RawNorm), _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P, _P, _I]),
     "yond_vst_inv": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _I, _P]),
     "yond_pack_pad": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "yond_crop_unpack": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
@@ -59,12 +59,13 @@ SIGNATURES = {
     "yond_nlf_maps": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _P]),
     "yond_nlf_maps_bayer": (_I, [_P, _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
     "yond_nlf_maps_raw16": (_I, [_P, C.POINTER(RawNorm), _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "yond_nlf_maps_raw16_per_image": (_I, [_P, _P, _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
     "yond_nlf_maps_collab_cached": (_I, [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "yond_nlf_fit_work_bytes": (_SZ, [_I]),
     "yond_nlf_fit": (_I, [_P, _P, _P, _SZ, _I, C.POINTER(_D), _I, _P, _P, _P, _P]),
     "yond_chain_work_bytes": (_SZ, [_I]),
     "yond_bias_table_nodes": (_I, [C.c_float]),
-    "yond_vst_params_fill": (_I, [_P, _P, _I, _I, _D, _D, _D, _I, _I, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P]),
+    "yond_vst_params_fill": (_I, [_P, _P, _I, _I, _D, _D, _D, _I, _I, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P]),
     "yond_bias_table": (_I, [_D, _D, C.c_float, _P, _P, _I, _P, _P, _P]),
     "yond_bias_points": (_I, [_P, _I, _D, _D, _I, _P, _P, _P]),
     "yond_vst_inv_place": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _I, _I, _I, _P, _I, _P, _P]),

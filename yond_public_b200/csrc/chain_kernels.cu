@@ -209,21 +209,28 @@ struct FillArgs {
 __global__ void params_fill_kernel(FillArgs a, const double* __restrict__ regs, const float* __restrict__ seg_max,
                                    const double* __restrict__ sg_lut, const yond_vst_params* __restrict__ prev,
                                    const int32_t* __restrict__ prev_ok, yond_vst_params* __restrict__ params, float* __restrict__ t_out,
-                                   SegChain* __restrict__ chain, double* __restrict__ regs_out, int32_t* __restrict__ ok_out) {
+                                   SegChain* __restrict__ chain, double* __restrict__ regs_out, int32_t* __restrict__ ok_out,
+                                   const double* __restrict__ seg_scales) {
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= a.nseg) return;
+  double scale_est = a.scale_est, scale = a.scale, bound_scale = a.bound_scale;
+  if (seg_scales) {  // this image's (scale_est, scale, bound_scale)
+    scale_est = seg_scales[3 * s];
+    scale = seg_scales[3 * s + 1];
+    bound_scale = seg_scales[3 * s + 2];
+  }
   double b1 = regs[2 * s], b2 = regs[2 * s + 1];
   int ok = 1;
   double sig;
   if (a.round >= 2) {  // YOND_SIDD.py:438-447
     if (b2 < 0.0) b2 = __dmul_rn(b1, b1);
-    sig = __dmul_rn(sqrt(b2), a.scale_est);
+    sig = __dmul_rn(sqrt(b2), scale_est);
     // the reference leaves its loop at the first beta1 < 0: an image that stopped in an earlier round stays stopped
     ok = !(b1 < 0.0) && (!prev_ok || prev_ok[s]);
   } else {             // :356  sqrt(max(beta2, 0))
-    sig = __dmul_rn(sqrt(0.0 > b2 ? 0.0 : b2), a.scale_est);
+    sig = __dmul_rn(sqrt(0.0 > b2 ? 0.0 : b2), scale_est);
   }
-  const double gain = __dmul_rn(b1, a.scale_est);
+  const double gain = __dmul_rn(b1, scale_est);
   if (regs_out) {
     regs_out[4 * s] = b1;
     regs_out[4 * s + 1] = b2;
@@ -247,11 +254,11 @@ __global__ void params_fill_kernel(FillArgs a, const double* __restrict__ regs, 
     const double c0 = __dadd_rn(__dmul_rn(0.375, __dmul_rn(gain, gain)), __dmul_rn(sig, sig));
     const double two_g = __ddiv_rn(2.0, gain);
     const double lower = __dmul_rn(two_g, sqrt(c0 > 0.0 ? c0 : 0.0));
-    const double up_arg = __dadd_rn(__dmul_rn(gain, a.scale), c0);
+    const double up_arg = __dadd_rn(__dmul_rn(gain, scale), c0);
     const double upper = __dmul_rn(two_g, sqrt(up_arg > 0.0 ? up_arg : 0.0));
     q.gain = (float)gain;
     q.sigma = (float)sig;
-    q.scale = (float)a.scale;
+    q.scale = (float)scale;
     q.lower = (float)lower;
     q.upper = (float)upper;
     q.exact_inverse = a.exact_inverse;
@@ -270,7 +277,7 @@ __global__ void params_fill_kernel(FillArgs a, const double* __restrict__ regs, 
         ch.use_lut = 1;
       } else {  // no LUT, or sigma/K beyond it: the numeric table up to this image's maximum (:254-257, isp_algos.py:204-212)
         const float mx = seg_max ? seg_max[s] : 1.0f;
-        ch.bound = __fmul_rn(mx > 0.f ? mx : 0.f, (float)a.bound_scale);
+        ch.bound = __fmul_rn(mx > 0.f ? mx : 0.f, (float)bound_scale);
         int n = table_nodes(ch.bound);
         if (n > a.max_nodes) n = a.max_nodes;  // the caller sized the rows for its data range
         ch.n_nodes = n;
@@ -329,7 +336,7 @@ int yond_vst_params_fill(const double* regs_dev, const float* seg_max_dev, int n
                          double scale, double bound_scale, int round, int bias_mode, int exact_inverse, const float* lut2d,
                          const double* sg_lut_dev, const float* x_lut_dev, int nx, int nsg, const yond_vst_params* prev_params,
                          yond_vst_params* params_dev, float* t_dev, float* rows, float* xnodes, int row_stride, double* regs_out,
-                         int32_t* ok_dev, void* work, void* stream, const int32_t* prev_ok) {
+                         int32_t* ok_dev, void* work, void* stream, const int32_t* prev_ok, const double* seg_scales_dev) {
   YOND_REQUIRE(regs_dev && params_dev && t_dev && work, "yond_vst_params_fill: null argument");
   YOND_REQUIRE(nseg > 0 && nseg <= 65535 && frames_per_seg > 0, "yond_vst_params_fill: bad batch geometry");
   YOND_REQUIRE(bias_mode >= 0 && bias_mode <= 2, "yond_vst_params_fill: bias_mode 0 (None), 1 ('pre'), 2 ('post')");
@@ -350,7 +357,7 @@ int yond_vst_params_fill(const double* regs_dev, const float* seg_max_dev, int n
   a.has_lut = lut2d != nullptr;
   a.max_nodes = row_stride;
   params_fill_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(a, regs_dev, seg_max_dev, sg_lut_dev, prev_params, prev_ok, params_dev, t_dev,
-                                                      chain, regs_out, ok_dev);
+                                                      chain, regs_out, ok_dev, seg_scales_dev);
   YOND_LAUNCH_CHECK();
   if (bias_mode == 1) {
     if (lut2d) {

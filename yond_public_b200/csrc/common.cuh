@@ -100,24 +100,43 @@ __device__ __forceinline__ void reds_add(uint32_t a, uint32_t by = 1u) {
 // Sensor mosaic read in place of a float32 Bayer frame (SURVEY 8(f)-1): the dataset normalisation of
 // data_process/yond_datasets.py:955-961 / :1053-1056, (float32(raw) - black) * ratio / (white - black) in float32 in that order,
 // is applied on load, so the normalised frame never exists in memory (2 B/px instead of 4 per read).  base == nullptr: float source.
+// per_img != nullptr: one yond_raw_norm per dataset image in device memory; a kernel's unit u (a box-filter image, a frame) belongs
+// to image u / units_per_img, and raw_norm_at replaces the uniform fields with that image's entry, once per thread or CTA.
 struct RawNorm {
   const uint16_t* base;
   float bl, ratio, denom;
   int clip;
+  const yond_raw_norm* per_img;
+  int units_per_img;
 };
 __device__ __forceinline__ float raw_norm(uint32_t v, const RawNorm& q) {
   float t = __fdiv_rn(__fmul_rn(__fsub_rn((float)v, q.bl), q.ratio), q.denom);
   if (q.clip) t = fminf(fmaxf(t, 0.f), 1.f);
   return t;
 }
-static inline RawNorm make_raw_norm(const uint16_t* base, const yond_raw_norm* n) {
+__device__ __forceinline__ RawNorm raw_norm_at(RawNorm q, int unit) {
+  if (q.per_img) {
+    const yond_raw_norm n = q.per_img[unit / q.units_per_img];
+    q.bl = n.black;
+    q.ratio = n.ratio;
+    q.denom = __fsub_rn(n.white, n.black);  // the host's float32 white - black of make_raw_norm
+    q.clip = n.clip;
+  }
+  return q;
+}
+static inline RawNorm make_raw_norm(const uint16_t* base, const yond_raw_norm* n, const yond_raw_norm* per_img = nullptr,
+                                    int units_per_img = 1) {
   RawNorm q{};
-  if (base && n) {
+  if (base && (n || per_img)) {
     q.base = base;
-    q.bl = n->black;
-    q.ratio = n->ratio;
-    q.denom = n->white - n->black;
-    q.clip = n->clip;
+    if (n) {
+      q.bl = n->black;
+      q.ratio = n->ratio;
+      q.denom = n->white - n->black;
+      q.clip = n->clip;
+    }
+    q.per_img = per_img;
+    q.units_per_img = units_per_img;
   }
   return q;
 }

@@ -329,10 +329,11 @@ __global__ void __launch_bounds__(kBlock, 5) vst_fwd_kernel(const float* __restr
                                                          float* __restrict__ ub, int H, int W, int pl, int pt, int hp, int wp,
                                                          const yond_vst_params* __restrict__ params,
                                                          const float* __restrict__ rows, const float* __restrict__ xnodes,
-                                                         int row_stride, RawNorm raw) {
+                                                         int row_stride, RawNorm raw_in) {
   extern __shared__ float4 tab[];
   __shared__ TabInfo ti;
   const int b = blockIdx.y;
+  const RawNorm raw = raw_norm_at(raw_in, b);  // every pixel of a CTA belongs to frame b
   const int h = H >> 1, w = W >> 1;
   VstConst c{};
   if (kVst) {
@@ -681,11 +682,12 @@ int yond_vst_fwd(const float* bayer, float* z, float* ub, int B, int H, int W, i
 }
 int yond_vst_fwd_raw16(const uint16_t* raw, const yond_raw_norm* nrm, float* z, float* ub, int B, int H, int W, int pad_l, int pad_r,
                        int pad_t, int pad_b, const yond_vst_params* params_dev, const float* rows, const float* xnodes, int row_stride,
-                       void* stream) {
-  YOND_REQUIRE(params_dev != nullptr && raw != nullptr && nrm != nullptr, "yond_vst_fwd_raw16: null argument");
-  YOND_REQUIRE(nrm->white > nrm->black && (uintptr_t)raw % 4 == 0 && W % 2 == 0, "yond_vst_fwd_raw16: bad normalisation / alignment");
+                       void* stream, const yond_raw_norm* nrm_dev, int frames_per_img) {
+  YOND_REQUIRE(params_dev != nullptr && raw != nullptr && (nrm != nullptr || nrm_dev != nullptr), "yond_vst_fwd_raw16: null argument");
+  YOND_REQUIRE((nrm_dev ? frames_per_img >= 1 : nrm->white > nrm->black) && (uintptr_t)raw % 4 == 0 && W % 2 == 0,
+               "yond_vst_fwd_raw16: bad normalisation / alignment");
   return launch_fwd(true, nullptr, z, ub, B, H, W, pad_l, pad_r, pad_t, pad_b, params_dev, rows, xnodes, row_stride, stream,
-                    make_raw_norm(raw, nrm));
+                    make_raw_norm(raw, nrm, nrm_dev, frames_per_img));
 }
 int yond_pack_pad(const float* bayer, float* z, float* ub, int B, int H, int W, int pad_l, int pad_r, int pad_t, int pad_b,
                   void* stream) {

@@ -112,6 +112,8 @@ __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, floa
   }
   const float* colbase = src.base + coloff;
   const uint16_t* colbase16 = kBayer && src.raw.base ? src.raw.base + coloff : nullptr;
+  // per thread: in the narrow layout one block holds images of different dataset images
+  const RawNorm rn = kBayer ? raw_norm_at(src.raw, b) : src.raw;
   const uint32_t row_pitch = kBayer ? 2u * (uint32_t)src.row_len : (uint32_t)src.row_len;  // an image stays below 2^32 floats
   float vmax = 0.f;
   double s[NQ];
@@ -131,7 +133,7 @@ __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, floa
     if (kBayer && colbase16) {  // uint16 mosaic: two 32-bit loads per packed pixel, normalised on load
       const uint32_t a = __ldg(reinterpret_cast<const uint32_t*>(colbase16 + roff));
       const uint32_t d = __ldg(reinterpret_cast<const uint32_t*>(colbase16 + roff + src.row_len));
-      v = make_float4(raw_norm(a & 0xffffu, src.raw), raw_norm(a >> 16, src.raw), raw_norm(d & 0xffffu, src.raw), raw_norm(d >> 16, src.raw));
+      v = make_float4(raw_norm(a & 0xffffu, rn), raw_norm(a >> 16, rn), raw_norm(d & 0xffffu, rn), raw_norm(d >> 16, rn));
     } else if (kBayer) {
       const float2 a = __ldg(reinterpret_cast<const float2*>(p)), d = __ldg(reinterpret_cast<const float2*>(p + src.row_len));
       v = make_float4(a.x, a.y, d.x, d.y);
@@ -1040,11 +1042,12 @@ int yond_nlf_maps(const float* x, const float* y, float* var, float* mean, float
   return nlf_maps_impl(xs, &ys, false, var, mean, lap, B, h, w, k, mode, work, (cudaStream_t)stream);
 }
 
-static int nlf_maps_bayer_impl(const float* x, const uint16_t* x16, const yond_raw_norm* nrm, int x_mosaic, const float* y, int y_mosaic,
-                               float* var, float* mean, float* lap, int nimg, int nblk, int H, int W, int split_blocks, int k, int mode,
-                               float* seg_max, void* work, void* stream) {
+static int nlf_maps_bayer_impl(const float* x, const uint16_t* x16, const yond_raw_norm* nrm, const yond_raw_norm* nrm_dev, int x_mosaic,
+                               const float* y, int y_mosaic, float* var, float* mean, float* lap, int nimg, int nblk, int H, int W,
+                               int split_blocks, int k, int mode, float* seg_max, void* work, void* stream) {
   YOND_REQUIRE((x || x16) && var && (mode == 3 || (mean && lap)) && work, "yond_nlf_maps_bayer: null argument");
-  YOND_REQUIRE(!x16 || (nrm && nrm->white > nrm->black && (uintptr_t)x16 % 4 == 0), "yond_nlf_maps_raw16: normalisation / 4-byte aligned mosaic required");
+  YOND_REQUIRE(!x16 || ((nrm_dev || (nrm && nrm->white > nrm->black)) && (uintptr_t)x16 % 4 == 0),
+               "yond_nlf_maps_raw16: normalisation / 4-byte aligned mosaic required");
   YOND_REQUIRE(nimg > 0 && nblk > 0 && H > 0 && W > 0 && H % 2 == 0 && W % 2 == 0, "yond_nlf_maps_bayer: H,W must be even");
   YOND_REQUIRE(k % 2 == 1 && k >= 3 && k <= kMaxK, "yond_nlf_maps_bayer: odd k <= %d required (got %d)", kMaxK, k);
   YOND_REQUIRE(mode == 0 || mode == 3 || (mode == 1 && y != nullptr), "yond_nlf_maps_bayer: mode 0, 1 or 3, the collab mode needs the second input");
@@ -1056,7 +1059,7 @@ static int nlf_maps_bayer_impl(const float* x, const uint16_t* x16, const yond_r
   YOND_REQUIRE(h > k / 2 && w > k / 2, "yond_nlf_maps_bayer: frame smaller than the filter radius");
   YOND_REQUIRE(B <= 65535, "yond_nlf_maps_bayer: at most 65535 images per call");
   BoxSrc xs = bayer_src(x, x_mosaic, nblk, H, W, split_blocks);
-  xs.raw = make_raw_norm(x16, nrm);
+  xs.raw = make_raw_norm(x16, nrm, nrm_dev, xs.imgs_per_seg);  // box-filter image b is dataset image b / imgs_per_seg
   xs.seg_max = seg_max;
   if (seg_max) YOND_CUDA_CHECK(cudaMemsetAsync(seg_max, 0, sizeof(float) * nimg, s));
   BoxSrc ys = bayer_src(y, y_mosaic, nblk, H, W, split_blocks);
@@ -1065,15 +1068,22 @@ static int nlf_maps_bayer_impl(const float* x, const uint16_t* x16, const yond_r
 int yond_nlf_maps_bayer(const float* x, int x_mosaic, const float* y, int y_mosaic, float* var, float* mean, float* lap, int nimg,
                         int nblk, int H, int W, int split_blocks, int k, int mode, float* seg_max, void* work, void* stream) {
   YOND_REQUIRE(x != nullptr, "yond_nlf_maps_bayer: null argument");
-  return nlf_maps_bayer_impl(x, nullptr, nullptr, x_mosaic, y, y_mosaic, var, mean, lap, nimg, nblk, H, W, split_blocks, k, mode, seg_max, work,
-                             stream);
+  return nlf_maps_bayer_impl(x, nullptr, nullptr, nullptr, x_mosaic, y, y_mosaic, var, mean, lap, nimg, nblk, H, W, split_blocks, k, mode,
+                             seg_max, work, stream);
 }
 int yond_nlf_maps_raw16(const uint16_t* x, const yond_raw_norm* nrm, int x_mosaic, const float* y, int y_mosaic, float* var, float* mean,
                         float* lap, int nimg, int nblk, int H, int W, int split_blocks, int k, int mode, float* seg_max, void* work,
                         void* stream) {
   YOND_REQUIRE(x != nullptr && nrm != nullptr, "yond_nlf_maps_raw16: null argument");
-  return nlf_maps_bayer_impl(nullptr, x, nrm, x_mosaic, y, y_mosaic, var, mean, lap, nimg, nblk, H, W, split_blocks, k, mode, seg_max, work,
-                             stream);
+  return nlf_maps_bayer_impl(nullptr, x, nrm, nullptr, x_mosaic, y, y_mosaic, var, mean, lap, nimg, nblk, H, W, split_blocks, k, mode,
+                             seg_max, work, stream);
+}
+int yond_nlf_maps_raw16_per_image(const uint16_t* x, const yond_raw_norm* nrm_dev, int x_mosaic, const float* y, int y_mosaic,
+                                  float* var, float* mean, float* lap, int nimg, int nblk, int H, int W, int split_blocks, int k,
+                                  int mode, float* seg_max, void* work, void* stream) {
+  YOND_REQUIRE(x != nullptr && nrm_dev != nullptr, "yond_nlf_maps_raw16_per_image: null argument");
+  return nlf_maps_bayer_impl(nullptr, x, nullptr, nrm_dev, x_mosaic, y, y_mosaic, var, mean, lap, nimg, nblk, H, W, split_blocks, k, mode,
+                             seg_max, work, stream);
 }
 
 int yond_nlf_maps_collab_cached(const float* y, int y_mosaic, const float* lr_var, float* var, float* mean, float* lap, int nimg, int nblk,

@@ -54,7 +54,8 @@ class NlfEstimator:
         frames are nblk = 1 in either layout).  split_blocks: every block is its own image for the box filters (SIDD_256).
         seg_max (optional, (nimg,) f32 CUDA): receives max(x, 0) per image.  Returns regs (nimg, 2) float64 on the
         device [, detail (nimg, DETAIL)]; nothing is read back.  x may be the uint16 sensor mosaic (a 16-bit integer tensor) with
-        raw = _lib.RawNorm(black, white, ratio, clip): it is normalised on load (SURVEY 8(f)-1).
+        raw = _lib.RawNorm(black, white, ratio, clip), or a CUDA uint8 tensor of nimg yond_raw_norm records (one per image): it is
+        normalised on load (SURVEY 8(f)-1).
         var_map (self only; float32 CUDA, at least B*h*w*4 values): the var map goes there instead of the estimator's scratch, where
         no later call overwrites it — the cached noisy-frame statistics of the collab rounds (estimate_collab_cached)."""
         lib = self.lib
@@ -80,8 +81,9 @@ class NlfEstimator:
         if y is not None:
             assert y.is_cuda and y.dtype == torch.float32 and y.is_contiguous() and y.numel() == x.numel()
         if is_raw:
-            check(lib.yond_nlf_maps_raw16(ptr(x), C.byref(raw), int(bool(x_mosaic)), ptr(y), int(bool(y_mosaic)), ptr(var), ptr(mean), ptr(lap),
-                                          nimg, nb, H, W, int(bool(split_blocks)), int(k), mode, ptr(seg_max), ptr(work), stream_ptr()))
+            fn, nrm = _raw16_maps(lib, raw)
+            check(fn(ptr(x), nrm, int(bool(x_mosaic)), ptr(y), int(bool(y_mosaic)), ptr(var), ptr(mean), ptr(lap),
+                     nimg, nb, H, W, int(bool(split_blocks)), int(k), mode, ptr(seg_max), ptr(work), stream_ptr()))
         else:
             check(lib.yond_nlf_maps_bayer(ptr(x), int(bool(x_mosaic)), ptr(y), int(bool(y_mosaic)), ptr(var), ptr(mean), ptr(lap), nimg, nb,
                                           H, W, int(bool(split_blocks)), int(k), mode, ptr(seg_max), ptr(work), stream_ptr()))
@@ -121,8 +123,9 @@ class NlfEstimator:
         assert out.numel() >= self.collab_geometry(nimg, nb, H, W, split_blocks)
         work = self._buf("maps", lib.yond_nlf_work_bytes(1, 1, 1, 4), x.device)  # mode 3 uses no scratch
         if x.dtype in (torch.int16, torch.uint16):
-            check(lib.yond_nlf_maps_raw16(ptr(x), C.byref(raw), int(bool(x_mosaic)), None, 0, ptr(out), None, None, nimg, nb, H, W,
-                                          int(bool(split_blocks)), int(k), 3, None, ptr(work), stream_ptr()))
+            fn, nrm = _raw16_maps(lib, raw)
+            check(fn(ptr(x), nrm, int(bool(x_mosaic)), None, 0, ptr(out), None, None, nimg, nb, H, W, int(bool(split_blocks)), int(k), 3,
+                     None, ptr(work), stream_ptr()))
         else:
             assert x.dtype == torch.float32
             check(lib.yond_nlf_maps_bayer(ptr(x), int(bool(x_mosaic)), None, 0, ptr(out), None, None, nimg, nb, H, W,
@@ -150,6 +153,14 @@ class NlfEstimator:
         """CollabNLF (beta1, beta2) of a collab round from the cached lr statistics: regs (nimg, 2) float64 on the device."""
         var, mean, lap = self.collab_maps_cached(y, lr_var, nblk, k, split_blocks, y_mosaic)
         return self._fit(var, mean, lap, y.shape[0], details, step)
+
+
+def _raw16_maps(lib, raw):
+    """The uint16 maps entry point and its normalisation argument: one host RawNorm for every image, or the per-image device records."""
+    if isinstance(raw, torch.Tensor):
+        assert raw.is_cuda and raw.dtype == torch.uint8 and raw.is_contiguous()
+        return lib.yond_nlf_maps_raw16_per_image, ptr(raw)
+    return lib.yond_nlf_maps_raw16, C.byref(raw)
 
 
 _EST = threading.local()

@@ -18,6 +18,66 @@ from . import _lib, archs, isp, nlf
 from ._lib import VstParams, check, ptr, stream_ptr
 
 SIGMA_CORR_PRE = 1.03  # YOND_SIDD.py:284
+RAW_REC = np.dtype([("black", "<f4"), ("white", "<f4"), ("ratio", "<f4"), ("clip", "<i4")])  # yond_raw_norm
+assert RAW_REC.itemsize == C.sizeof(_lib.RawNorm)
+
+
+def _per_image(v, nimg, name):
+    a = np.asarray(v)
+    if a.ndim > 1 or (a.ndim == 1 and a.shape[0] != nimg):
+        raise ValueError(f"{name}: a scalar or {nimg} values (one per image) expected, got shape {a.shape}")
+    try:
+        f = a.astype(np.float64)
+    except (TypeError, ValueError):
+        raise ValueError(f"{name}: numbers expected, got {v!r}") from None
+    if not np.isfinite(f).all():
+        raise ValueError(f"{name}: non-finite value in {v!r}")
+    return np.broadcast_to(a, (nimg,))
+
+
+def batch_exposure(p, nimg, raw=None):
+    """The exposure parameters of a batch of `nimg` images, one value per image.  p['wp'], p['bl'], p['scale'] (default wp - bl) and
+    each entry of raw = (black, white, ratio[, clip]) are a scalar (every image) or a length-nimg sequence / 1-D array.
+    Returns (scale_est, scale, raw_rec): float64 (nimg,) arrays scale_est = wp - bl and scale, and the (nimg,) RAW_REC records of
+    raw (None without raw).  Raises ValueError for a wrong length, wp <= bl, scale <= 0, ratio <= 0, white <= black or a
+    non-finite value."""
+    wp, bl = _per_image(p["wp"], nimg, "p['wp']"), _per_image(p["bl"], nimg, "p['bl']")
+    scale_est = (wp - bl).astype(np.float64)
+    if not (scale_est > 0).all():
+        raise ValueError(f"p['wp'] must exceed p['bl'] for every image: wp={p['wp']!r}, bl={p['bl']!r}")
+    scale = _per_image(p["scale"], nimg, "p['scale']").astype(np.float64) if "scale" in p else scale_est
+    if not (scale > 0).all():
+        raise ValueError(f"p['scale'] must be positive for every image, got {p['scale']!r}")
+    if raw is None:
+        return scale_est, scale, None
+    if not 3 <= len(raw) <= 4:
+        raise ValueError(f"raw = (black, white, ratio[, clip]) expected, got {raw!r}")
+    rec = np.zeros(nimg, RAW_REC)
+    for field, v in zip(("black", "white", "ratio", "clip"), raw):
+        a = _per_image(v, nimg, f"raw {field}")
+        rec[field] = a.astype(bool) if field == "clip" else a.astype(np.float64)
+    if not (rec["white"] > rec["black"]).all():
+        raise ValueError(f"raw: white must exceed black for every image, got {raw!r}")
+    if not (rec["ratio"] > 0).all():
+        raise ValueError(f"raw: ratio must be positive for every image, got {raw!r}")
+    return scale_est, scale, rec
+
+
+def _upload(arrays, device):
+    """One non-blocking copy of the concatenated bytes of `arrays` from pinned memory on the current stream; returns the device byte
+    buffer and the byte offset of each array.  The caching allocators keep both buffers until the copy and the kernels enqueued
+    after it on this stream have run, so nothing waits for the host."""
+    offs, parts, n = [], [], 0
+    for a in arrays:
+        n = (n + 7) // 8 * 8
+        offs.append(n)
+        parts.append((n, np.ascontiguousarray(a).view(np.uint8).reshape(-1)))
+        n += parts[-1][1].size
+    host = torch.empty(n, dtype=torch.uint8, pin_memory=True)
+    h = host.numpy()
+    for o, b in parts:
+        h[o:o + b.size] = b
+    return host.to(device, non_blocking=True), offs
 
 
 def build_net(arch: dict, device="cuda"):
@@ -65,7 +125,8 @@ class YondEngine:
         Bias source per frame, like the reference (YOND_SIDD.py:252-262, utils/isp_algos.py:196-231): only
         bias_corr == 'pre' applies a bias ('post' computes one and never uses it, :261 / :294-295); the BiasLUT row for this
         sigma/K when a LUT is loaded and sigma/K is inside its range, otherwise the fallback `get_bias` table up to this
-        frame's maximum (`frame_max`: callable returning per-frame max in DN), generated on the device."""
+        frame's maximum (`frame_max`: callable returning per-frame max in DN), generated on the device.  `scale`: one value or one
+        per frame."""
         gains = np.asarray(gains, np.float64)
         sigmas = np.asarray(sigmas, np.float64)
         B = len(gains)
@@ -146,9 +207,11 @@ class YondEngine:
     BIAS_MODES = {None: 0, "pre": 1, "post": 2}
     max_value = 1.0  # upper bound of the (normalised) input data assumed when sizing fallback bias tables; raise for noclip data
 
-    def chain_params(self, regs, seg_max, nseg, fps, scale_est, scale, bound_scale, rnd, bias_corr, vst_type, prev=None):
+    def chain_params(self, regs, seg_max, nseg, fps, scale_est, scale, bound_scale, rnd, bias_corr, vst_type, prev=None, scales_dev=None):
         """regs: (nseg,2) float64 CUDA.  Returns a dict of device buffers: params (bytes), t, rows, xnodes, stride,
         regs4 (nseg,4: beta1, beta2 after the guards, gain, sigma), ok (nseg int32: still live after this round).
+        scale_est, scale, bound_scale: one value or one per image.  scales_dev (optional): the same as a (nseg,3) float64 CUDA array
+        already on the device; else they are copied there.
         prev: the chain of the previous round (rnd >= 2) — its params are kept by images that are not live, and its ok is chained."""
         if bias_corr not in self.BIAS_MODES:
             raise NotImplementedError(f"bias_corr={bias_corr!r}")
@@ -156,10 +219,14 @@ class YondEngine:
         mode = self.BIAS_MODES[bias_corr]
         exact = 1 if (bias_corr is None and vst_type == "exact") else 0
         lut = self.biaslut.device_arrays() if (self.biaslut is not None and mode == 1) else None
+        scale_est, scale, bound_scale = (np.broadcast_to(np.asarray(v, np.float64), (nseg,)) for v in (scale_est, scale, bound_scale))
+        if scales_dev is None:
+            buf, _ = _upload([np.stack([scale_est, scale, bound_scale], 1)], dev)
+            scales_dev = buf.view(torch.float64)
         stride = 1921
         rows = xnodes = None
-        if mode == 1:
-            cap = int(lib.yond_bias_table_nodes(float(np.float32(self.max_value) * np.float32(bound_scale))))
+        if mode == 1:  # rows sized for the largest bound of the batch
+            cap = int(lib.yond_bias_table_nodes(float((np.float32(self.max_value) * bound_scale.astype(np.float32)).max())))
             stride = max(1921, cap) if lut is not None else max(cap, 8)
             rows = torch.empty((nseg, stride), device=dev, dtype=torch.float32)
             xnodes = torch.empty((nseg, stride), device=dev, dtype=torch.float32)
@@ -168,16 +235,19 @@ class YondEngine:
                    t=torch.empty(nseg * fps, device=dev, dtype=torch.float32), rows=rows, xnodes=xnodes, stride=stride,
                    regs4=torch.empty((nseg, 4), device=dev, dtype=torch.float64), ok=torch.empty(nseg, device=dev, dtype=torch.int32))
         work = self._buf("chain", (int(lib.yond_chain_work_bytes(nseg)),), torch.uint8, dev)
-        check(lib.yond_vst_params_fill(ptr(regs), ptr(seg_max), nseg, fps, float(scale_est), float(scale), float(bound_scale), int(rnd), mode,
+        # the per-image array replaces the scalar (scale_est, scale, bound_scale) arguments
+        check(lib.yond_vst_params_fill(ptr(regs), ptr(seg_max), nseg, fps, 0.0, 0.0, 0.0, int(rnd), mode,
                                        exact, ptr(lut[0]) if lut else None, ptr(lut[2]) if lut else None, ptr(lut[1]) if lut else None,
                                        1921, 1101, ptr(prev["params"]) if prev is not None else None, ptr(out["params"]), ptr(out["t"]),
                                        ptr(rows), ptr(xnodes), stride, ptr(out["regs4"]), ptr(out["ok"]), ptr(work), stream_ptr(),
-                                       ptr(prev["ok"]) if prev is not None else None))
+                                       ptr(prev["ok"]) if prev is not None else None, ptr(scales_dev)))
         return out
 
     def vst_denoise_dev(self, frames, chain, out, frames_per_row=1, fps=1, select=False, fallback=None, clip01=True, raw=None):
         """VST_Denoiser for frames (B,H,W) with device-filled parameters; writes `out` (plain (B,H,W) or the mosaic layout
-        (B/n, H, n*W) for frames_per_row = n).  select: frames of images with chain['ok'] == 0 copy `fallback` instead."""
+        (B/n, H, n*W) for frames_per_row = n).  select: frames of images with chain['ok'] == 0 copy `fallback` instead.
+        raw: frames is the uint16 sensor mosaic and raw the CUDA uint8 tensor of the yond_raw_norm records of its images (fps frames
+        each)."""
         B, H, W = frames.shape
         dev = frames.device
         h, w = H // 2, W // 2
@@ -194,9 +264,10 @@ class YondEngine:
         for b0 in range(0, B, cb):
             n = min(cb, B - b0)
             pch = params[b0 * psz:]
-            if raw is not None:  # uint16 sensor mosaic, normalised on load
-                check(self.lib.yond_vst_fwd_raw16(ptr(frames[b0:b0 + n]), C.byref(raw), ptr(z[:n]), ptr(ub[:n]), n, H, W, pl, pr, pt, pb, ptr(pch),
-                                                  ptr(chain["rows"]), ptr(chain["xnodes"]), chain["stride"], st))
+            if raw is not None:  # uint16 sensor mosaic, normalised on load with each image's record (b0 starts an image)
+                check(self.lib.yond_vst_fwd_raw16(ptr(frames[b0:b0 + n]), None, ptr(z[:n]), ptr(ub[:n]), n, H, W, pl, pr, pt, pb, ptr(pch),
+                                                  ptr(chain["rows"]), ptr(chain["xnodes"]), chain["stride"], st,
+                                                  ptr(raw[b0 // fps * RAW_REC.itemsize:]), fps))
             else:
                 check(self.lib.yond_vst_fwd(ptr(frames[b0:b0 + n]), ptr(z[:n]), ptr(ub[:n]), n, H, W, pl, pr, pt, pb, ptr(pch),
                                             ptr(chain["rows"]), ptr(chain["xnodes"]), chain["stride"], st))
@@ -207,7 +278,8 @@ class YondEngine:
 
     # ------------------------------------------------------------------------------------------
     def vst_denoise(self, bayer, gains, sigmas, scale, bias_corr="pre", vst_type="exact", clip01=True, table_bound=None, fixed_table=None, out=None):
-        """VST_Denoiser (YOND_SIDD.py:250-299) for a batch: bayer (B,H,W) CUDA f32 -> (B,H,W) CUDA f32."""
+        """VST_Denoiser (YOND_SIDD.py:250-299) for a batch: bayer (B,H,W) CUDA f32 -> (B,H,W) CUDA f32.  gains, sigmas and scale:
+        one value or one per frame."""
         B, H, W = bayer.shape
         dev = bayer.device
         h, w = H // 2, W // 2
@@ -215,13 +287,14 @@ class YondEngine:
         hp, wp = h + pt + pb, w + pl + pr
         gains = np.broadcast_to(np.asarray(gains, np.float64), (B,))
         sigmas = np.broadcast_to(np.asarray(sigmas, np.float64), (B,))
+        scale = np.broadcast_to(np.asarray(scale, np.float64), (B,))
         # upper bound of a fallback table: the caller's bound (YOND_SIDD.py:393-395: one table per image, up to the image
         # max) or, like VST_Denoiser / BiasLUT.get_lut on their own, each frame's max in DN (float32 product)
         if table_bound is not None:
             frame_max = lambda: np.full(B, np.float32(table_bound), np.float32)
         else:
-            frame_max = lambda: (bayer.amax(dim=(1, 2)).clamp_min(0).cpu().numpy().astype(np.float32) * np.float32(scale))
-        params, rows, xnodes, stride, t = self.make_params(gains, sigmas, float(scale), bias_corr, vst_type, frame_max, dev, fixed_table)
+            frame_max = lambda: (bayer.amax(dim=(1, 2)).clamp_min(0).cpu().numpy().astype(np.float32) * scale.astype(np.float32))
+        params, rows, xnodes, stride, t = self.make_params(gains, sigmas, scale, bias_corr, vst_type, frame_max, dev, fixed_table)
         if out is None:
             out = torch.empty_like(bayer)
         cb = self.default_chunk(B, hp, wp)
@@ -467,20 +540,30 @@ class YOND_SIDD:
 
         raw = (black, white, ratio[, clip]): x is the uint16 SENSOR mosaic (16-bit integer tensor) and the dataset normalisation
         (raw - black) * ratio / (white - black) of the 14-bit drivers (data_process/yond_datasets.py:955-961, :1053-1056) is applied
-        on load by the estimator and the VST front end — the float32 frame never exists (SURVEY 8(f)-1)."""
+        on load by the estimator and the VST front end — the float32 frame never exists (SURVEY 8(f)-1).
+
+        Exposure per image: p['wp'], p['bl'], p['scale'] and each entry of raw are a scalar (every image) or one value per image
+        (batch_exposure; ValueError before anything is launched), so a batch may mix white / black levels and ratios.  They reach the
+        device in one small copy; scalars take the same path."""
         pipe = self.pipe
         n_collab = collab_rounds(pipe)
         if raw is not None:
             assert x.dtype in (torch.int16, torch.uint16) and lr_full is None
-            raw = _lib.RawNorm(float(raw[0]), float(raw[1]), float(raw[2]), int(bool(raw[3])) if len(raw) > 3 else 0)
         assert pipe["full_est"] and "simple" in pipe["est_type"]
         nimg, nblk, H, W = x.shape
         dev = x.device
         eng = self.engine
-        scale_est = p["wp"] - p["bl"]
-        scale = p.get("scale", scale_est)
         k, bias_corr, vst_type = pipe["k"], pipe["bias_corr"], pipe.get("vst_type", "exact")
         full_dn = bool(pipe["full_dn"])
+        scale_est, scale, raw_rec = batch_exposure(p, nimg, raw)
+        # (scale_est, scale, bound) per image for round 1 and for the collab rounds.  The bound of a fallback bias table: full_dn
+        # round 1 = the frame's max in DN of p['scale'] (:256); everything else lr_raw.max()*(wp-bl) (:393, :449)
+        scales1 = np.stack([scale_est, scale, scale if full_dn else scale_est], 1)
+        scales_c = np.stack([scale_est, scale, scale_est], 1)
+        buf, offs = _upload([scales1, scales_c] + ([raw_rec] if raw is not None else []), dev)
+        s1_dev = buf[offs[0]:offs[1]].view(torch.float64)
+        sc_dev = buf[offs[1]:offs[1] + scales_c.nbytes].view(torch.float64)
+        raw = buf[offs[2]:] if raw is not None else None
         est = nlf._estimator()
 
         def mark(name):  # optional stage timing (synchronising; for profiling only)
@@ -524,9 +607,7 @@ class YOND_SIDD:
             if need_max:
                 seg_max = x.amax().clamp_min(0).reshape(1)
         mark("estimate_self")
-        # the bound of a fallback bias table: full_dn round 1 = the frame's max in DN of p['scale'] (:256); everything else
-        # lr_raw.max()*(wp-bl) (:393, :449)
-        ch = eng.chain_params(regs, seg_max, nimg, nblk, scale_est, scale, scale if full_dn else scale_est, 1, bias_corr, vst_type)
+        ch = eng.chain_params(regs, seg_max, nimg, nblk, *scales1.T, 1, bias_corr, vst_type, scales_dev=s1_dev)
         frames = x.reshape(nimg * nblk, H, W)
         out = torch.empty((nimg, H, nblk * W), device=dev, dtype=torch.float32)
         eng.vst_denoise_dev(frames, ch, out, frames_per_row=nblk, fps=nblk, raw=raw)
@@ -540,7 +621,7 @@ class YOND_SIDD:
                 est.lr_var_dev(cx, lr_var, k, split_blocks=sidd, x_mosaic=c_mosaic, nblk=cnb, raw=raw)
             regs = est.estimate_collab_cached(out, lr_var, cnb, k, split_blocks=sidd, y_mosaic=True)
             mark("estimate_collab")
-            ch = eng.chain_params(regs, seg_max, nimg, nblk, scale_est, scale, scale_est, r, bias_corr, vst_type, prev=ch)
+            ch = eng.chain_params(regs, seg_max, nimg, nblk, *scales_c.T, r, bias_corr, vst_type, prev=ch, scales_dev=sc_dev)
             prev_out, out = out, torch.empty_like(out)
             eng.vst_denoise_dev(frames, ch, out, frames_per_row=nblk, fps=nblk, select=True, fallback=prev_out, raw=raw)
             mark(f"denoise_round{r}")
@@ -612,9 +693,11 @@ class YOND_SIDD:
         the next batch first, so its first upload runs under the tail of this one (bench.py's e2e keeps two in flight).
         `lanes` is accepted for compatibility and ignored (round 1 needed host threads to hide the estimator's read-backs).
         raw = (black, white, ratio[, clip]): host_in holds uint16 sensor mosaics (int16 / uint16 tensor, half the H2D bytes), see
-        iter_denoise_dev."""
+        iter_denoise_dev.  Per-image values of p / raw (one per image of host_in) are sliced for each group."""
         assert host_in.is_pinned() and host_out.is_pinned(), "pinned host buffers required for asynchronous copies"
         nimg = host_in.shape[0]
+        batch_exposure(p, nimg, raw)  # malformed values raise before the first copy
+        part = lambda v, a, b: v[a:b] if np.ndim(v) == 1 else v
         dev = self.device
         cur = torch.cuda.current_stream(dev)
         sizes = [min(group, nimg - a) for a in range(0, nimg, group)] if isinstance(group, int) else [int(g) for g in group]
@@ -650,7 +733,8 @@ class YOND_SIDD:
                 stage_in(g + 1)
             slot = ring[(seq0 + g) % 3]
             cur.wait_event(in_ready[g])
-            res = self.iter_denoise_dev(slot["buf"][:b - a], dict(p), raw=raw)
+            pg = {key: part(v, a, b) if key in ("wp", "bl", "scale") else v for key, v in p.items()}
+            res = self.iter_denoise_dev(slot["buf"][:b - a], pg, raw=None if raw is None else tuple(part(v, a, b) for v in raw))
             done = torch.cuda.Event()
             done.record(cur)
             slot["free"] = done
