@@ -1,6 +1,5 @@
 """Times the estimator stages (CUDA events, device-resident) on N synthetic 12 MP frames: maps (box filters) and fit
-(radix select + score3 + masked sums), self and collab.  Environment switches of the kernels (YOND_BOX_ROWS, ...) are read
-once per process: run one process per setting."""
+(radix select + score3 + masked sums), self and collab."""
 import os
 import sys
 

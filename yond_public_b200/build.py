@@ -13,8 +13,6 @@ LIB = os.path.join(HERE, "libyond_b200.so")
 SOURCES = ["api.cu", "isp_kernels.cu", "nlf_kernels.cu", "chain_kernels.cu", "net_kernels.cu", "conv_tc.cu", "conv_ref.cu", "net.cu", "metrics_kernels.cu", "render_kernels.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
-if os.environ.get("YOND_CONV_TIMING"):  # cycle counters in the conv kernel's producer / issuer loops (printed with YOND_CONV_DBG=8)
-    NVCC_FLAGS.append("-DYOND_CONV_TIMING")
 
 
 def _nvcc():

@@ -19,20 +19,12 @@
 // absolute shared-memory address, so any pixel-aligned start reads consistently).  T sub-tiles of 128 pixels
 // (stacked rows, or T images) share every weight tile, which cuts weight traffic from L2 by T.  Two builds:
 // conv_tc_kernel<false> (one CTA per SM) and conv_tc_kernel<true> (cluster of 2, cta_group::2: each CTA holds its own
-// pixels and half of every weight tile).  Modes: 3x3 s1, 3x3 s2, 1x1 (on up to two concatenated sources), ConvT 2x2,
-// and the fused ConvT 2x2 + 1x1-on-concat hand-over of the decoder (CONV_UPSC).  See DESIGN.md section 4.
+// pixels and half of every weight tile; the 3x3 layers that stream their weights with N tiles >= 128).  Modes: 3x3 s1,
+// 3x3 s2, 1x1 (on up to two concatenated sources), ConvT 2x2, and the fused ConvT 2x2 + 1x1-on-concat hand-over of the
+// decoder (CONV_UPSC).  See DESIGN.md section 4.
 #include "conv_tc.cuh"
 
-#include <cstdlib>
 #include <mutex>
-
-// -DYOND_CONV_TIMING: cycle counters in the producer / issuer loops, printed with YOND_CONV_DBG=8 (six clock reads per tile in the
-// issuer otherwise cost ~5 % of a narrow layer)
-#ifdef YOND_CONV_TIMING
-#define YOND_TICK() clock64()
-#else
-#define YOND_TICK() 0LL
-#endif
 
 namespace {
 
@@ -41,6 +33,12 @@ constexpr int kThreads = 64 + 32 * kEpiWarps;  // 2 control warps + the epilogue
 constexpr int kMaxStagesA = 8;
 constexpr int kMaxStagesB = 8;
 constexpr int kMaxT = 4;
+// The MMA issuer instantiates its loops for T = 1, 2 and 4 only (T is a power of two <= kMaxT).
+static_assert(kMaxT == 4, "conv_tc: the issuer dispatches T in {1, 2, 4}");
+constexpr int kMaxNT = 256;      // largest UMMA N
+constexpr int kCta2MinNT = 128;  // smallest N tile of a streamed layer that runs as a CTA pair
+// Resident-weight layers other than 3x3 stride 1 tabulate their stage decode (16 B per stage) in the 1 KB output-conv table.
+constexpr int kMaxTabStages = 64;
 
 // Division by a run-time constant as multiply-high + shift (n < 2^31): the epilogue and the tile decode run once per
 // tile in every warp, and a 32-bit integer division is ~20 instructions.
@@ -71,7 +69,6 @@ struct TcParams {
   int CB;     // channel block (32 | 64)
   int ncb0, ncb1;
   int mode;
-  int slab;   // 3x3 stride-1: 1 = one halo slab per channel block (9 taps by descriptor offset); 0 = three W-shifted slabs
   int wres;   // weights resident in smem
   int SA, SB; // pipeline depths
   uint32_t a_stage_bytes, a_tx_bytes, b_stage_bytes;  // stage pitch (1024-aligned), bytes one slab load writes, weight tile
@@ -91,7 +88,6 @@ struct TcParams {
   int paired;      // pixel-pair formulation of a 32 -> 32 channel 3x3 conv (conv_tc.cuh): N = CB = 64 over (H, W/2)
   int cvec;        // channels of the bias / scale / shift vectors (= Cout, or 32 in the paired formulation)
   uint32_t cmask;  // paired: 31 (output column n = o*32 + co uses vector entry co), else all ones
-  int dbg;    // bring-up switches (YOND_CONV_DBG): 1 = skip global stores, 2 = skip the epilogue math, 4 = skip residual loads
   const float* bias;
   const float* scale;
   const float* shift;
@@ -279,29 +275,19 @@ struct AStage {
   int dw, dh;    // tile-origin offsets of the load
   int ntaps;     // weight tiles consumed from this stage
   int widx0;     // first weight-tile index
-  int sx;        // fixed horizontal tap of this stage (three-slab mode), else -1
+  int sx;        // CONV_UPSC skip part: output parity of this stage, else -1
 };
 __device__ __forceinline__ AStage decode_astage(const TcParams& p, int ai) {
   AStage s;
   s.sx = -1;
-  if (p.mode == CONV_3X3_S1) {
-    int cbg, src;
-    if (p.slab) {
-      cbg = ai;
-      s.dw = -1;
-      s.ntaps = 9;
-      s.widx0 = cbg * 9;
-    } else {
-      cbg = ai / 3;
-      s.sx = ai - cbg * 3;
-      s.dw = s.sx - 1;
-      s.ntaps = 3;
-      s.widx0 = cbg * 9 + s.sx;  // tap = r*3 + sx
-    }
-    src = cbg >= p.ncb0;
+  if (p.mode == CONV_3X3_S1) {  // one halo slab per channel block: all nine taps
+    const int src = ai >= p.ncb0;
     s.map = src;
-    s.c = (src ? cbg - p.ncb0 : cbg) * p.CB;
+    s.c = (src ? ai - p.ncb0 : ai) * p.CB;
+    s.dw = -1;
     s.dh = -1;
+    s.ntaps = 9;
+    s.widx0 = ai * 9;
   } else if (p.mode == CONV_3X3_S2) {
     int cbg = ai / 9, tap = ai - cbg * 9;
     int r = tap / 3, sx = tap - r * 3;
@@ -339,9 +325,9 @@ __device__ __forceinline__ AStage decode_astage(const TcParams& p, int ai) {
   }
   return s;
 }
-__device__ __forceinline__ int num_astages(const TcParams& p) {
+__host__ __device__ __forceinline__ int num_astages(const TcParams& p) {
   int ncb = p.ncb0 + p.ncb1;
-  if (p.mode == CONV_3X3_S1) return p.slab ? ncb : ncb * 3;
+  if (p.mode == CONV_3X3_S1) return ncb;
   if (p.mode == CONV_UPSC) return p.ncb0 + 4 * p.ncb1;
   return p.mode == CONV_3X3_S2 ? ncb * 9 : ncb;
 }
@@ -460,7 +446,7 @@ __device__ __forceinline__ void issue_tap(uint32_t d_tmem, uint32_t nt, uint32_t
 }
 
 // K steps [K0, K1) of one tap (pixel-pair formulation: the other steps multiply all-zero weights)
-template <int K0, int K1, int TT, bool kP = false>  // kP: cta_group::2 MMAs (CTA pair)
+template <int K0, int K1, int TT>
 __device__ __forceinline__ void issue_tap_range(uint32_t d_tmem, uint32_t nt, uint32_t a_lo0, uint32_t sub_step, uint32_t b_lo0,
                                                 uint32_t a_hi, uint32_t b_hi, uint32_t idesc, uint32_t accum) {
   uint32_t al = a_lo0 + 2u * K0, dt = d_tmem;
@@ -468,32 +454,29 @@ __device__ __forceinline__ void issue_tap_range(uint32_t d_tmem, uint32_t nt, ui
   for (int t = 0; t < TT; ++t) {
     uint32_t bl = b_lo0 + 2u * K0;
 #pragma unroll
-    for (int k = K0; k < K1; ++k) {
-      if (kP) umma_step_pair(dt, al, a_hi, bl, b_hi, idesc, k > K0 ? 1u : accum);
-      else umma_step(dt, al, a_hi, bl, b_hi, idesc, k > K0 ? 1u : accum);
-    }
+    for (int k = K0; k < K1; ++k) umma_step(dt, al, a_hi, bl, b_hi, idesc, k > K0 ? 1u : accum);
     al += sub_step - 2u * (K1 - K0);
     dt += nt;
   }
 }
 // Nine taps of a pixel-pair slab (CB = 64: K steps 0,1 = first pixel of the pair, 2,3 = second): the left neighbour pair
 // contributes only its second pixel, the right neighbour pair only its first.
-template <int TT, bool kP = false>
+template <int TT>
 __device__ __forceinline__ void issue_slab_paired(uint32_t d_tmem, uint32_t nt, uint32_t a_stage_lo, uint32_t tap_r16, uint32_t px16,
                                                   uint32_t sub_step, uint32_t b_lo_first, uint32_t b_step16, uint32_t a_hi,
                                                   uint32_t b_hi, uint32_t idesc, uint32_t first_accum) {
 #pragma unroll
   for (int r = 0; r < 3; ++r) {
     const uint32_t a0 = a_stage_lo + (uint32_t)r * tap_r16, b0 = b_lo_first + (uint32_t)(r * 3) * b_step16;
-    issue_tap_range<2, 4, TT, kP>(d_tmem, nt, a0, sub_step, b0, a_hi, b_hi, idesc, r ? 1u : first_accum);
-    issue_tap_range<0, 4, TT, kP>(d_tmem, nt, a0 + px16, sub_step, b0 + b_step16, a_hi, b_hi, idesc, 1u);
-    issue_tap_range<0, 2, TT, kP>(d_tmem, nt, a0 + 2u * px16, sub_step, b0 + 2u * b_step16, a_hi, b_hi, idesc, 1u);
+    issue_tap_range<2, 4, TT>(d_tmem, nt, a0, sub_step, b0, a_hi, b_hi, idesc, r ? 1u : first_accum);
+    issue_tap_range<0, 4, TT>(d_tmem, nt, a0 + px16, sub_step, b0 + b_step16, a_hi, b_hi, idesc, 1u);
+    issue_tap_range<0, 2, TT>(d_tmem, nt, a0 + 2u * px16, sub_step, b0 + 2u * b_step16, a_hi, b_hi, idesc, 1u);
   }
 }
 
 // All nine taps of one halo slab as straight-line code (resident weights): the only run-time inputs are a handful of
 // uniform bases and strides, everything else is an immediate.
-template <int KS, int TT, bool kP = false>
+template <int KS, int TT>
 __device__ __forceinline__ void issue_slab_resident(uint32_t d_tmem, uint32_t nt, uint32_t a_stage_lo, uint32_t tap_r16, uint32_t px16,
                                                     uint32_t sub_step, uint32_t b_lo_first, uint32_t b_step16, uint32_t a_hi,
                                                     uint32_t b_hi, uint32_t idesc, uint32_t first_accum) {
@@ -501,8 +484,8 @@ __device__ __forceinline__ void issue_slab_resident(uint32_t d_tmem, uint32_t nt
   for (int r = 0; r < 3; ++r)
 #pragma unroll
     for (int sx = 0; sx < 3; ++sx)
-      issue_tap_range<0, KS, TT, kP>(d_tmem, nt, a_stage_lo + (uint32_t)r * tap_r16 + (uint32_t)sx * px16, sub_step,
-                                     b_lo_first + (uint32_t)(r * 3 + sx) * b_step16, a_hi, b_hi, idesc, (r | sx) ? 1u : first_accum);
+      issue_tap_range<0, KS, TT>(d_tmem, nt, a_stage_lo + (uint32_t)r * tap_r16 + (uint32_t)sx * px16, sub_step,
+                                 b_lo_first + (uint32_t)(r * 3 + sx) * b_step16, a_hi, b_hi, idesc, (r | sx) ? 1u : first_accum);
 }
 
 // 256-bit global accesses (sm_100): one lane moves a whole 32-byte sector per instruction, so a pixel-per-lane store of
@@ -669,84 +652,76 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& p, uint32_t tmem_b
 #pragma unroll
       for (int k = 0; k < kV; ++k) {
         const int ci = part + nparts * (k0 + k);
-        if (ci < nvis && !(p.dbg & 128)) {  // dbg 128: the epilogue does not touch TMEM
-          const int t = ci >> p.lg_nchunk, c = (ci & nchunk_m1) << 4;
-          uint32_t v[16];
-          tmem_ld16(tmem_row + (uint32_t)((as * p.T + t) * p.NT + c), v);
-          tmem_ld_wait();
-          if (!(p.dbg & 2) && ((vmask >> k) & 1u)) {
-            float f[16];
-            if (kRegP) {
+        if (ci >= nvis) break;  // visits are in increasing order: the rest of the group is past the end too
+        const int t = ci >> p.lg_nchunk, c = (ci & nchunk_m1) << 4;
+        uint32_t v[16];
+        tmem_ld16(tmem_row + (uint32_t)((as * p.T + t) * p.NT + c), v);
+        tmem_ld_wait();
+        if ((vmask >> k) & 1u) {
+          float f[16];
+          if (kRegP) {
 #pragma unroll
-              for (int j = 0; j < 16; ++j) f[j] = kScale ? fmaf(__uint_as_float(v[j]), pa[j], pb[j]) : __uint_as_float(v[j]) + pb[j];
-            } else if (fixed) {
-              const uint32_t pt = ptab + 128u * (uint32_t)((k0 + k) & (nsets - 1));
+            for (int j = 0; j < 16; ++j) f[j] = kScale ? fmaf(__uint_as_float(v[j]), pa[j], pb[j]) : __uint_as_float(v[j]) + pb[j];
+          } else if (fixed) {
+            const uint32_t pt = ptab + 128u * (uint32_t)((k0 + k) & (nsets - 1));
 #pragma unroll
-              for (int g = 0; g < 4; ++g) {
-                const float4 bc = lds_f4(pt + 64 + 16 * g);
-                if (kScale) {
-                  const float4 a = lds_f4(pt + 16 * g);
-                  f[g * 4 + 0] = fmaf(__uint_as_float(v[g * 4 + 0]), a.x, bc.x); f[g * 4 + 1] = fmaf(__uint_as_float(v[g * 4 + 1]), a.y, bc.y);
-                  f[g * 4 + 2] = fmaf(__uint_as_float(v[g * 4 + 2]), a.z, bc.z); f[g * 4 + 3] = fmaf(__uint_as_float(v[g * 4 + 3]), a.w, bc.w);
-                } else {
-                  f[g * 4 + 0] = __uint_as_float(v[g * 4 + 0]) + bc.x; f[g * 4 + 1] = __uint_as_float(v[g * 4 + 1]) + bc.y;
-                  f[g * 4 + 2] = __uint_as_float(v[g * 4 + 2]) + bc.z; f[g * 4 + 3] = __uint_as_float(v[g * 4 + 3]) + bc.w;
-                }
-              }
-            } else {
-              const uint32_t n = (uint32_t)(tc.n0 + c);
-              const uint32_t co = (convt ? n - fdiv(n, p.fd_cout) * p.Cout : n) & p.cmask;
-              const float4* b4 = reinterpret_cast<const float4*>(p.bias + co);
-#pragma unroll
-              for (int g = 0; g < 4; ++g) {
-                const float4 bi = __ldg(b4 + g);
-                f[g * 4 + 0] = __uint_as_float(v[g * 4 + 0]) + bi.x; f[g * 4 + 1] = __uint_as_float(v[g * 4 + 1]) + bi.y;
-                f[g * 4 + 2] = __uint_as_float(v[g * 4 + 2]) + bi.z; f[g * 4 + 3] = __uint_as_float(v[g * 4 + 3]) + bi.w;
-              }
+            for (int g = 0; g < 4; ++g) {
+              const float4 bc = lds_f4(pt + 64 + 16 * g);
               if (kScale) {
-                int b = p.t_along_h ? bb : bb + t;
-                if (b > p.B - 1) b = p.B - 1;
-                const float4* s4 = reinterpret_cast<const float4*>(p.scale + (size_t)b * p.cvec + co);
-                const float4* h4 = p.shift ? reinterpret_cast<const float4*>(p.shift + (size_t)b * p.cvec + co) : nullptr;
-#pragma unroll
-                for (int g = 0; g < 4; ++g) {
-                  const float4 sc = __ldg(s4 + g), sh = h4 ? __ldg(h4 + g) : make_float4(0.f, 0.f, 0.f, 0.f);
-                  f[g * 4 + 0] = fmaf(f[g * 4 + 0], sc.x, sh.x); f[g * 4 + 1] = fmaf(f[g * 4 + 1], sc.y, sh.y);
-                  f[g * 4 + 2] = fmaf(f[g * 4 + 2], sc.z, sh.z); f[g * 4 + 3] = fmaf(f[g * 4 + 3], sc.w, sh.w);
-                }
+                const float4 a = lds_f4(pt + 16 * g);
+                f[g * 4 + 0] = fmaf(__uint_as_float(v[g * 4 + 0]), a.x, bc.x); f[g * 4 + 1] = fmaf(__uint_as_float(v[g * 4 + 1]), a.y, bc.y);
+                f[g * 4 + 2] = fmaf(__uint_as_float(v[g * 4 + 2]), a.z, bc.z); f[g * 4 + 3] = fmaf(__uint_as_float(v[g * 4 + 3]), a.w, bc.w);
+              } else {
+                f[g * 4 + 0] = __uint_as_float(v[g * 4 + 0]) + bc.x; f[g * 4 + 1] = __uint_as_float(v[g * 4 + 1]) + bc.y;
+                f[g * 4 + 2] = __uint_as_float(v[g * 4 + 2]) + bc.z; f[g * 4 + 3] = __uint_as_float(v[g * 4 + 3]) + bc.w;
               }
             }
-            if (kSilu) {
+          } else {
+            const uint32_t n = (uint32_t)(tc.n0 + c);
+            const uint32_t co = (convt ? n - fdiv(n, p.fd_cout) * p.Cout : n) & p.cmask;
+            const float4* b4 = reinterpret_cast<const float4*>(p.bias + co);
 #pragma unroll
-              for (int j = 0; j < 16; ++j) f[j] = fast_silu(f[j]);
-            } else if (lrelu) {  // slope < 1: LeakyReLU(x) = max(x, slope * x)
-#pragma unroll
-              for (int j = 0; j < 16; ++j) f[j] = fmaxf(f[j], f[j] * slope);
+            for (int g = 0; g < 4; ++g) {
+              const float4 bi = __ldg(b4 + g);
+              f[g * 4 + 0] = __uint_as_float(v[g * 4 + 0]) + bi.x; f[g * 4 + 1] = __uint_as_float(v[g * 4 + 1]) + bi.y;
+              f[g * 4 + 2] = __uint_as_float(v[g * 4 + 2]) + bi.z; f[g * 4 + 3] = __uint_as_float(v[g * 4 + 3]) + bi.w;
             }
-            if (kRes) {
+            if (kScale) {
+              int b = p.t_along_h ? bb : bb + t;
+              if (b > p.B - 1) b = p.B - 1;
+              const float4* s4 = reinterpret_cast<const float4*>(p.scale + (size_t)b * p.cvec + co);
+              const float4* h4 = p.shift ? reinterpret_cast<const float4*>(p.shift + (size_t)b * p.cvec + co) : nullptr;
 #pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                const float2 a = unpack_bf16x2(rr[k].v[j]);
-                f[2 * j] += a.x;
-                f[2 * j + 1] += a.y;
+              for (int g = 0; g < 4; ++g) {
+                const float4 sc = __ldg(s4 + g), sh = h4 ? __ldg(h4 + g) : make_float4(0.f, 0.f, 0.f, 0.f);
+                f[g * 4 + 0] = fmaf(f[g * 4 + 0], sc.x, sh.x); f[g * 4 + 1] = fmaf(f[g * 4 + 1], sc.y, sh.y);
+                f[g * 4 + 2] = fmaf(f[g * 4 + 2], sc.z, sh.z); f[g * 4 + 3] = fmaf(f[g * 4 + 3], sc.w, sh.w);
               }
             }
-            if (p.dbg & 1) {  // dbg 1: no global stores (keep the math alive)
-              float acc = 0.f;
+          }
+          if (kSilu) {
 #pragma unroll
-              for (int j = 0; j < 16; ++j) acc += f[j];
-              if (acc == 123.456f) p.out0[0] = __float2bfloat16_rn(acc);
-            } else {
-              U8 o;
+            for (int j = 0; j < 16; ++j) f[j] = fast_silu(f[j]);
+          } else if (lrelu) {  // slope < 1: LeakyReLU(x) = max(x, slope * x)
 #pragma unroll
-              for (int j = 0; j < 8; ++j) o.v[j] = pack_bf16x2(f[2 * j], f[2 * j + 1]);
-              stg256(p.out0 + off[k], o);
-              if (p.out1) {
+            for (int j = 0; j < 16; ++j) f[j] = fmaxf(f[j], f[j] * slope);
+          }
+          if (kRes) {
 #pragma unroll
-                for (int j = 0; j < 8; ++j) o.v[j] = pack_bf16x2(fast_silu(f[2 * j]), fast_silu(f[2 * j + 1]));
-                stg256(p.out1 + off[k], o);
-              }
+            for (int j = 0; j < 8; ++j) {
+              const float2 a = unpack_bf16x2(rr[k].v[j]);
+              f[2 * j] += a.x;
+              f[2 * j + 1] += a.y;
             }
+          }
+          U8 o;
+#pragma unroll
+          for (int j = 0; j < 8; ++j) o.v[j] = pack_bf16x2(f[2 * j], f[2 * j + 1]);
+          stg256(p.out0 + off[k], o);
+          if (p.out1) {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) o.v[j] = pack_bf16x2(fast_silu(f[2 * j]), fast_silu(f[2 * j + 1]));
+            stg256(p.out1 + off[k], o);
           }
         }
       }
@@ -942,12 +917,6 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
         mbar_expect_tx(w_full, p.ncb0 * p.b_stage_bytes + p.ncb1 * p.b2_stage_bytes);
         for (int i = 0; i < p.ncb0; ++i) tma_load_2d(smem_b + i * p.b_stage_bytes, &maps.w, w_full, 0, i * p.N);
         for (int i = 0; i < p.ncb1; ++i) tma_load_2d(smem_b + p.b2_off + i * p.b2_stage_bytes, &maps.w2, w_full, 0, i * p.Cout);
-      } else if (p.wres && kPair) {  // CTA pair: this CTA keeps its HALF (NT/2 rows) of every weight tile
-        const int nwt = num_wtiles(p);
-        const uint32_t w_full_sig = mapa_shared(w_full, 0);
-        if (sched.rank == 0) mbar_expect_tx(w_full, 2 * nwt * p.b_stage_bytes);
-        for (int i = 0; i < nwt; ++i)
-          tma_load_2d_pair(smem_b + i * p.b_stage_bytes, &maps.w, w_full_sig, 0, i * p.N + sched.rank * (p.NT / 2));
       } else if (p.wres) {  // all weight tiles of this layer stay in smem for the kernel's lifetime
         const int nwt = num_wtiles(p);
         mbar_expect_tx(w_full, nwt * p.b_stage_bytes);
@@ -956,7 +925,6 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
     }
     __syncwarp();
     int sa = 0, pa = 0, sb = 0, pb = 0;
-    long long t_wait = 0, t_begin = YOND_TICK();
     // CTA pair: "data landed" is counted on the LEADER's barriers (its MMA consumes both CTAs' stages); the leader
     // expects the bytes of both CTAs, the peer only issues its loads.  "Stage free" arrives on each CTA's own barrier
     // through the multicast commit.
@@ -967,13 +935,9 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
       const TileCoord tc = decode_tile(p, sched_tile(p, sched, u));
       for (int ai = 0; ai < n_ast; ++ai) {
         const AStage s = decode_astage(p, ai);
-        const long long tw0 = YOND_TICK();
         mbar_wait(a_empty + 8 * sa, pa ^ 1);
-        t_wait += YOND_TICK() - tw0;
         if (is_leader) {
-          if (p.dbg & 16) {  // bring-up: no activation loads (MMA-rate experiment; results are garbage)
-            mbar_arrive(a_full + 8 * sa);
-          } else if (kPair) {
+          if (kPair) {
             if (pair_leader) mbar_expect_tx(a_full + 8 * sa, 2 * p.a_tx_bytes);
             tma_load_4d_pair(smem_a + sa * p.a_stage_bytes, &maps.a[s.map], a_full_sig + 8 * sa, s.c, tc.w0 + s.dw, tc.b0, tc.h0 + s.dh);
           } else {
@@ -985,7 +949,7 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
         if (++sa == p.SA) { sa = 0; pa ^= 1; }
         if (!p.wres) {
           for (int j = 0; j < s.ntaps; ++j) {
-            const int widx = s.widx0 + (s.sx >= 0 ? j * 3 : j);
+            const int widx = s.widx0 + j;
             mbar_wait(b_empty + 8 * sb, pb ^ 1);
             if (is_leader) {
               if (kPair) {
@@ -1002,8 +966,6 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
         }
       }
     }
-    if ((p.dbg & 8) && blockIdx.x == 0 && is_leader)
-      printf("[conv dbg] producer: total %lld cyc, waiting for a free A stage %lld cyc\n", YOND_TICK() - t_begin, t_wait);
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     // The whole warp stays converged and ONE elected lane issues the tcgen05 instructions.  tcgen05.mma takes its
@@ -1032,18 +994,16 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
     const uint32_t tap_r16 = p.tap_r_off >> 4, px16 = row_bytes >> 4;
     const uint32_t nt = (uint32_t)p.NT;
     const bool leader = elect_one() != 0;
-    if (p.wres && (!kPair || pair_leader)) mbar_wait(uw_full, 0);  // pair: both halves are counted on the leader's barrier
+    if (p.wres) mbar_wait(uw_full, 0);
     int sa = 0, pa = 0, sb = 0, pb = 0, as = 0, pacc = 0;
-    long long t_acc = 0, t_a = 0, t_issue = 0, t_dec = 0, t_begin = YOND_TICK();
     // The commonest shape — 3x3 stride 1, weights resident, ONE halo slab per tile (32 / 64 input channels: the four layers of
     // each full- and half-resolution block) — gets a loop of its own.  A single warp retires roughly one dependent instruction
     // every 5 cycles, and tcgen05.mma issue blocks once a few MMAs are queued, so whatever this warp executes between the last
     // MMA of a tile and the first of the next is time the tensor pipe drains and idles: the generic loop below spends up to
-    // ~1100 cycles per tile there (stage decode, the dispatch on T / K steps / pairing, ring bookkeeping; as seen by the cycle
-    // counters of the YOND_CONV_TIMING build, their own cost included) against 4500-5700 cycles for a tile of these layers.  Here everything tile-invariant is hoisted and the dispatch
-    // happens once, outside the loop.
-    const bool fast_slab1 = p.wres && p.slab && p.mode == CONV_3X3_S1 && n_ast == 1 && !kPair && !(p.dbg & (8 | 16 | 32 | 256 | 512)) &&  // dbg 512: generic loop (A/B of this path)
-                            (p.T == 1 || p.T == 2 || p.T == 4);
+    // ~1100 cycles per tile there (stage decode, the dispatch on T / K steps / pairing, ring bookkeeping; measured with cycle
+    // counters, their own cost included) against 4500-5700 cycles for a tile of these layers.  Here everything tile-invariant is
+    // hoisted and the dispatch happens once, outside the loop.
+    const bool fast_slab1 = p.wres && p.mode == CONV_3X3_S1 && n_ast == 1 && !kPair;
     if (fast_slab1) {
       const uint32_t b_first = (((u_smem_b) & 0x3FFFFu) >> 4) | lo_flags;  // the slab's channel block is 0: widx0 = 0
       const uint32_t b_step16 = p.b_stage_bytes >> 4;
@@ -1066,17 +1026,17 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
       };
 #define YOND_SLAB1(FN) run([&](uint32_t d, uint32_t a_lo) { FN(d, nt, a_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, 0u); })
       if (p.paired) {
-        if (p.T == 1) YOND_SLAB1((issue_slab_paired<1, kPair>));
-        else if (p.T == 2) YOND_SLAB1((issue_slab_paired<2, kPair>));
-        else YOND_SLAB1((issue_slab_paired<4, kPair>));
+        if (p.T == 1) YOND_SLAB1((issue_slab_paired<1>));
+        else if (p.T == 2) YOND_SLAB1((issue_slab_paired<2>));
+        else YOND_SLAB1((issue_slab_paired<4>));
       } else if (ksteps == 4) {
-        if (p.T == 1) YOND_SLAB1((issue_slab_resident<4, 1, kPair>));
-        else if (p.T == 2) YOND_SLAB1((issue_slab_resident<4, 2, kPair>));
-        else YOND_SLAB1((issue_slab_resident<4, 4, kPair>));
+        if (p.T == 1) YOND_SLAB1((issue_slab_resident<4, 1>));
+        else if (p.T == 2) YOND_SLAB1((issue_slab_resident<4, 2>));
+        else YOND_SLAB1((issue_slab_resident<4, 4>));
       } else {
-        if (p.T == 1) YOND_SLAB1((issue_slab_resident<2, 1, kPair>));
-        else if (p.T == 2) YOND_SLAB1((issue_slab_resident<2, 2, kPair>));
-        else YOND_SLAB1((issue_slab_resident<2, 4, kPair>));
+        if (p.T == 1) YOND_SLAB1((issue_slab_resident<2, 1>));
+        else if (p.T == 2) YOND_SLAB1((issue_slab_resident<2, 2>));
+        else YOND_SLAB1((issue_slab_resident<2, 4>));
       }
 #undef YOND_SLAB1
     }
@@ -1084,10 +1044,8 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
     // activation stage, 2-36 stages per tile.  Their stage decode (weight-tile address, and for the skip part of CONV_UPSC a
     // narrower N and a column offset into the accumulator) does not depend on the tile: it is tabulated once in shared memory
     // (the unused output-conv table region) and the per-stage work of this warp shrinks to a barrier wait, one 16-byte load and
-    // the MMAs.
-    constexpr int kMaxTabStages = 64;
-    const bool fast_tab = p.wres && p.mode != CONV_3X3_S1 && !kPair && n_ast <= kMaxTabStages && p.tail_w == nullptr &&
-                          !(p.dbg & (8 | 16 | 32 | 512)) && (p.T == 1 || p.T == 2 || p.T == 4);
+    // the MMAs.  (conv_tc_launch bounds n_ast by kMaxTabStages; the fused output conv, whose table shares the region, is 3x3 only.)
+    const bool fast_tab = p.wres && p.mode != CONV_3X3_S1 && !kPair;
     if (fast_tab) {
       const uint32_t tab = smem_base + p.smem_tail_off;
       for (int ai = lane; ai < n_ast; ai += 32) {
@@ -1139,8 +1097,7 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
     // Streamed weights, one halo slab per 64-channel block (the 128- to 512-channel 3x3 layers, normally as CTA pairs): nine taps
     // per stage, each waiting for its weight tile and handing the ring slot back.  Same hoisting: T is dispatched once, the
     // stage needs no decode at all (the slab is the whole story for this warp; weight tiles arrive in ring order).
-    const bool fast_stream = !p.wres && p.slab && p.mode == CONV_3X3_S1 && ksteps == 4 && !(p.dbg & (8 | 16 | 32 | 512)) &&
-                             (p.T == 1 || p.T == 2 || p.T == 4);
+    const bool fast_stream = !p.wres && p.mode == CONV_3X3_S1 && ksteps == 4;
     if (fast_stream && (!kPair || pair_leader)) {
       const uint32_t a_bytes = p.a_stage_bytes, b_bytes = p.b_stage_bytes, acc_cols = (uint32_t)p.T * nt;
       const int SA = p.SA, SB = p.SB, nacc = p.acc_stages;
@@ -1190,112 +1147,45 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
       else YOND_STREAM(4);
 #undef YOND_STREAM
     }
-    // CTA pair: only the leader CTA issues (its MMAs drive both SMs' tensor cores); the peer's warp 1 idles
-    for (int u = (fast_slab1 || fast_tab || fast_stream || (kPair && !pair_leader)) ? sched.n_units : sched.first; u < sched.n_units;
-         u += sched.step) {
-      long long tw0 = YOND_TICK();
-      mbar_wait(uacc_empty + 8 * as, pacc ^ 1);
-      t_acc += YOND_TICK() - tw0;
-      tc_fence_after();
-      const uint32_t d_tmem = u_tmem + (uint32_t)(as * p.T) * nt;
-      const uint32_t d_tmem_tile = d_tmem;
-      for (int ai = 0; ai < n_ast; ++ai) {
-        const long long td0 = YOND_TICK();
-        const AStage s = decode_astage(p, ai);
-        tw0 = YOND_TICK();
-        t_dec += tw0 - td0;
-        mbar_wait(ua_full + 8 * sa, pa);
-        t_a += YOND_TICK() - tw0;
+    // Everything no loop above takes: resident-weight 3x3 layers with several halo slabs (a concatenation of two 32-channel
+    // sources), and streamed layers with one weight tile per stage (stride-2 3x3, 1x1 / ConvT / fused up-sampling too wide to stay
+    // resident, and 3x3 with 32-channel blocks).  Every CTA-pair plan takes fast_stream, where the peer CTA's warp 1 idles.
+    if (!kPair && !fast_slab1 && !fast_tab && !fast_stream) {
+      for (int u = sched.first; u < sched.n_units; u += sched.step) {
+        mbar_wait(uacc_empty + 8 * as, pacc ^ 1);
         tc_fence_after();
-        const uint32_t a_stage_lo = (((u_smem_a + (uint32_t)sa * p.a_stage_bytes) & 0x3FFFFu) >> 4) | lo_flags;
-        const long long ti0 = YOND_TICK();
-        if (leader && p.wres && p.slab && p.mode == CONV_3X3_S1 && !(p.dbg & 32)) {
-          // resident weights, single slab: 9 taps x T sub-tiles x K steps as one straight-line burst
-          const uint32_t b_first = (((u_smem_b + (uint32_t)s.widx0 * p.b_stage_bytes) & 0x3FFFFu) >> 4) | lo_flags;
-          const uint32_t b_step16 = p.b_stage_bytes >> 4;
-          const uint32_t acc0 = ai ? 1u : 0u;
-          if (p.paired && !(p.dbg & 256)) {  // dbg 256: keep the all-zero K steps (cross-check of the skip)
-            if (p.T == 1) issue_slab_paired<1, kPair>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
-            else if (p.T == 2) issue_slab_paired<2, kPair>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
-            else issue_slab_paired<4, kPair>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
-          } else if (ksteps == 4) {
-            if (p.T == 1) issue_slab_resident<4, 1, kPair>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
-            else if (p.T == 2) issue_slab_resident<4, 2, kPair>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
-            else issue_slab_resident<4, 4, kPair>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
-          } else {
-            if (p.T == 1) issue_slab_resident<2, 1, kPair>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
-            else if (p.T == 2) issue_slab_resident<2, 2, kPair>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
-            else issue_slab_resident<2, 4, kPair>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
-          }
-          if (kPair) umma_commit_pair(ua_empty + 8 * sa);  // frees the stage in both CTAs
-          else umma_commit(ua_empty + 8 * sa);
-        } else if (leader && p.wres && p.mode != CONV_3X3_S1 && !(p.dbg & 32)) {
-          // resident weights, one tap per stage (stride-2 / 1x1 / transposed / fused up-sampling): one straight-line burst
-          uint32_t b_lo0 = (((u_smem_b + (uint32_t)s.widx0 * p.b_stage_bytes) & 0x3FFFFu) >> 4) | lo_flags;
-          const uint32_t acc0 = ai ? 1u : 0u;
-          uint32_t idesc = idesc_full, d_tmem = d_tmem_tile;
-          if (p.mode == CONV_UPSC && s.sx >= 0) {  // skip part: N = Cout, accumulate into parity s.sx's columns
-            b_lo0 = (((u_smem_b + p.b2_off + (uint32_t)s.widx0 * p.b2_stage_bytes) & 0x3FFFFu) >> 4) | lo_flags;
-            idesc = (idesc_full & ~(0x3Fu << 17)) | ((uint32_t)(p.Cout >> 3) << 17);
-            d_tmem = d_tmem_tile + (uint32_t)(s.sx * p.Cout);
-          }
-          if (ksteps == 4) {
-            if (p.T == 1) issue_tap<4, 1>(d_tmem, nt, a_stage_lo, sub_step, b_lo0, a_hi, b_hi, idesc, acc0);
-            else if (p.T == 2) issue_tap<4, 2>(d_tmem, nt, a_stage_lo, sub_step, b_lo0, a_hi, b_hi, idesc, acc0);
-            else issue_tap<4, 4>(d_tmem, nt, a_stage_lo, sub_step, b_lo0, a_hi, b_hi, idesc, acc0);
-          } else {
-            if (p.T == 1) issue_tap<2, 1>(d_tmem, nt, a_stage_lo, sub_step, b_lo0, a_hi, b_hi, idesc, acc0);
-            else if (p.T == 2) issue_tap<2, 2>(d_tmem, nt, a_stage_lo, sub_step, b_lo0, a_hi, b_hi, idesc, acc0);
-            else issue_tap<2, 4>(d_tmem, nt, a_stage_lo, sub_step, b_lo0, a_hi, b_hi, idesc, acc0);
-          }
-          umma_commit(ua_empty + 8 * sa);
-        } else if (leader && !p.wres && p.slab && p.mode == CONV_3X3_S1 && ksteps == 4 && !(p.dbg & 32)) {
-          // streamed weights, single slab, 64-channel blocks: nine taps with a compile-time trip count; each waits for
-          // its weight tile (CTA pair: both halves, counted on this CTA's barrier) and frees the stage (in both CTAs)
-          int lsb = sb, lpb = pb;
-#pragma unroll
-          for (int j = 0; j < 9; ++j) {
-            const uint32_t r = j / 3, sx = j % 3;
-            mbar_wait(ub_full + 8 * lsb, lpb);
-            tc_fence_after();
-            const uint32_t a_lo0 = a_stage_lo + r * tap_r16 + sx * px16;
-            const uint32_t b_lo0 = (((u_smem_b + (uint32_t)lsb * p.b_stage_bytes) & 0x3FFFFu) >> 4) | lo_flags;
-            const uint32_t accum = (ai | j) ? 1u : 0u;
-            if (kPair) {
-              if (p.T == 1) issue_tap_pair<4, 1>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
-              else if (p.T == 2) issue_tap_pair<4, 2>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
-              else issue_tap_pair<4, 4>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
-              umma_commit_pair(ub_empty + 8 * lsb);
+        const uint32_t d_tmem = u_tmem + (uint32_t)(as * p.T) * nt;
+        for (int ai = 0; ai < n_ast; ++ai) {
+          const AStage s = decode_astage(p, ai);
+          mbar_wait(ua_full + 8 * sa, pa);
+          tc_fence_after();
+          const uint32_t a_stage_lo = (((u_smem_a + (uint32_t)sa * p.a_stage_bytes) & 0x3FFFFu) >> 4) | lo_flags;
+          if (leader && p.wres) {
+            // resident weights, 3x3 stride 1: 9 taps x T sub-tiles x K steps of this slab as one straight-line burst
+            const uint32_t b_first = (((u_smem_b + (uint32_t)s.widx0 * p.b_stage_bytes) & 0x3FFFFu) >> 4) | lo_flags;
+            const uint32_t b_step16 = p.b_stage_bytes >> 4;
+            const uint32_t acc0 = ai ? 1u : 0u;
+            if (ksteps == 4) {
+              if (p.T == 1) issue_slab_resident<4, 1>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
+              else if (p.T == 2) issue_slab_resident<4, 2>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
+              else issue_slab_resident<4, 4>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
             } else {
-              if (p.T == 1) issue_tap<4, 1>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
-              else if (p.T == 2) issue_tap<4, 2>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
-              else issue_tap<4, 4>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
-              umma_commit(ub_empty + 8 * lsb);
+              if (p.T == 1) issue_slab_resident<2, 1>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
+              else if (p.T == 2) issue_slab_resident<2, 2>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
+              else issue_slab_resident<2, 4>(d_tmem, nt, a_stage_lo, tap_r16, px16, sub_step, b_first, b_step16, a_hi, b_hi, idesc, acc0);
             }
-            if (++lsb == p.SB) { lsb = 0; lpb ^= 1; }
-          }
-          if (kPair) umma_commit_pair(ua_empty + 8 * sa);
-          else umma_commit(ua_empty + 8 * sa);
-        } else if (leader) {
-          int lsb = sb, lpb = pb;  // weight-ring position of this stage's first tap (uniform on entry)
-          for (int j = 0; j < s.ntaps; ++j) {
-            uint32_t r = 0, sx = 0, widx = (uint32_t)(s.widx0 + j);
-            if (p.mode == CONV_3X3_S1) {
-              if (s.sx >= 0) { r = j; widx = (uint32_t)(s.widx0 + j * 3); }   // three-slab mode: the stage fixes sx
-              else { r = (j >= 3) + (j >= 6); sx = j - r * 3; }             // single slab: all nine taps
-            }
-            uint32_t b_base;
-            if (p.wres) {
-              b_base = u_smem_b + widx * p.b_stage_bytes;
-            } else {
+            umma_commit(ua_empty + 8 * sa);
+          } else if (leader) {
+            // streamed weights: each tap waits for its weight tile and hands the ring slot back
+            int lsb = sb, lpb = pb;  // weight-ring position of this stage's first tap (uniform on entry)
+            for (int j = 0; j < s.ntaps; ++j) {
+              uint32_t r = 0, sx = 0;
+              if (p.mode == CONV_3X3_S1) { r = (j >= 3) + (j >= 6); sx = j - r * 3; }
               mbar_wait(ub_full + 8 * lsb, lpb);
               tc_fence_after();
-              b_base = u_smem_b + (uint32_t)lsb * p.b_stage_bytes;
-            }
-            const uint32_t a_lo0 = a_stage_lo + r * tap_r16 + sx * px16;
-            const uint32_t b_lo0 = ((b_base & 0x3FFFFu) >> 4) | lo_flags;
-            const uint32_t accum = (ai | j) ? 1u : 0u;
-            if (!(p.dbg & 32)) {  // dbg 32: no MMAs (TMA-rate experiment)
+              const uint32_t a_lo0 = a_stage_lo + r * tap_r16 + sx * px16;
+              const uint32_t b_lo0 = (((u_smem_b + (uint32_t)lsb * p.b_stage_bytes) & 0x3FFFFu) >> 4) | lo_flags;
+              const uint32_t accum = (ai | j) ? 1u : 0u;
               if (ksteps == 4) {
                 if (p.T == 1) issue_tap<4, 1>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
                 else if (p.T == 2) issue_tap<4, 2>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
@@ -1305,32 +1195,23 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
                 else if (p.T == 2) issue_tap<2, 2>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
                 else issue_tap<2, 4>(d_tmem, nt, a_lo0, sub_step, b_lo0, a_hi, b_hi, idesc, accum);
               }
-            }
-            if (!p.wres) {
               umma_commit(ub_empty + 8 * lsb);
               if (++lsb == p.SB) { lsb = 0; lpb ^= 1; }
             }
+            umma_commit(ua_empty + 8 * sa);
           }
-          umma_commit(ua_empty + 8 * sa);
+          __syncwarp();
+          if (!p.wres) {  // advance the weight ring by this stage's taps, in converged code
+            sb += s.ntaps;
+            while (sb >= p.SB) { sb -= p.SB; pb ^= 1; }
+          }
+          if (++sa == p.SA) { sa = 0; pa ^= 1; }
         }
+        if (leader) umma_commit(uacc_full + 8 * as);
         __syncwarp();
-        t_issue += YOND_TICK() - ti0;
-        if (!p.wres) {  // advance the weight ring by this stage's taps, in converged code
-          sb += s.ntaps;
-          while (sb >= p.SB) { sb -= p.SB; pb ^= 1; }
-        }
-        if (++sa == p.SA) { sa = 0; pa ^= 1; }
+        if (++as == p.acc_stages) { as = 0; pacc ^= 1; }
       }
-      if (leader) {
-        if (kPair) umma_commit_pair(uacc_full + 8 * as);
-        else umma_commit(uacc_full + 8 * as);
-      }
-      __syncwarp();
-      if (++as == p.acc_stages) { as = 0; pacc ^= 1; }
     }
-    if ((p.dbg & 8) && blockIdx.x == 0 && leader)
-      printf("[conv dbg] issuer: total %lld cyc; issue regions %lld; waiting: accumulator %lld, activations %lld; stage decode %lld; tiles %d, A stages/tile %d, SA %d SB %d T %d NT %d\n",
-             YOND_TICK() - t_begin, t_issue, t_acc, t_a, t_dec, (total_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x, n_ast, p.SA, p.SB, p.T, p.NT);
   } else {
     // ===================== epilogue (warps 2..2+kEpiWarps) =====================
     const bool silu = p.act == ACT_SILU;
@@ -1345,12 +1226,12 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
       else epilogue_tail<false, false>(p, tmem_base, acc_full, acc_empty, ptab, tailtab, warp, lane, total_tiles);
     }
     else if (p.scale && p.res) { if (silu) YOND_EPI(true, true, true, 2); else YOND_EPI(true, true, false, 2); }
-    else if (p.scale && epilogue_single_set(p) && !(p.dbg & 1024)) {  // dbg 1024: parameters from shared memory (A/B)
+    else if (p.scale && epilogue_single_set(p)) {
       if (silu) epilogue_loop<true, false, true, 4, kPair, true>(p, tmem_base, acc_full, acc_empty, ptab, warp, lane, total_tiles);
       else epilogue_loop<true, false, false, 4, kPair, true>(p, tmem_base, acc_full, acc_empty, ptab, warp, lane, total_tiles);
     }
     else if (p.scale) { if (silu) YOND_EPI(true, false, true, 4); else YOND_EPI(true, false, false, 4); }
-    else if (p.res && epilogue_single_set(p) && !(p.dbg & 1024)) {
+    else if (p.res && epilogue_single_set(p)) {
 #define YOND_EPI_R(A, V) epilogue_loop<false, true, A, V, kPair, true>(p, tmem_base, acc_full, acc_empty, ptab, warp, lane, total_tiles)
       if (few) { if (silu) YOND_EPI_R(true, 2); else YOND_EPI_R(false, 2); }
       else { if (silu) YOND_EPI_R(true, 4); else YOND_EPI_R(false, 4); }
@@ -1360,7 +1241,7 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
       if (few) { if (silu) YOND_EPI(false, true, true, 2); else YOND_EPI(false, true, false, 2); }
       else { if (silu) YOND_EPI(false, true, true, 4); else YOND_EPI(false, true, false, 4); }
     }
-    else if (epilogue_single_set(p) && !(p.dbg & 1024)) {
+    else if (epilogue_single_set(p)) {
       if (silu) epilogue_loop<false, false, true, 4, kPair, true>(p, tmem_base, acc_full, acc_empty, ptab, warp, lane, total_tiles);
       else epilogue_loop<false, false, false, 4, kPair, true>(p, tmem_base, acc_full, acc_empty, ptab, warp, lane, total_tiles);
     }
@@ -1437,13 +1318,6 @@ int pow2_ceil(int v) {
   return p;
 }
 
-// Debug / bring-up switches (environment): YOND_CONV_SLAB=0 selects the three-slab 3x3 path, YOND_CONV_T caps the
-// number of sub-tiles sharing a weight tile.
-int env_int(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return v ? atoi(v) : dflt;
-}
-
 }  // namespace
 
 int conv_tc_channel_block(int Cin0, int Cin1) {
@@ -1472,11 +1346,10 @@ void conv_tc_pack_paired(const float* w, bf16* out) {
 
 int conv_tc_launch(const ConvLayer& Lin, cudaStream_t stream) {
   ConvLayer L = Lin;
-  static const int env_paired = env_int("YOND_CONV_PAIRED", 1);
   // (layers with a residual input are bound by their 3 x 64 B per pixel of HBM traffic, not by the MMAs: measured 930 us plain
   // vs 990-1030 us paired for 24.8 M pixels, so they keep the N = 32 form)
-  const bool paired = env_paired && L.wpaired && L.mode == CONV_3X3_S1 && L.Cin0 == 32 && L.Cin1 == 0 && L.Cout == 32 && L.Win % 2 == 0 &&
-                      (L.res == nullptr || env_paired > 1) && L.tail_w == nullptr;
+  const bool paired = L.wpaired && L.mode == CONV_3X3_S1 && L.Cin0 == 32 && L.Cin1 == 0 && L.Cout == 32 && L.Win % 2 == 0 &&
+                      L.res == nullptr && L.tail_w == nullptr;
   if (paired) {  // (B,H,W,32) is (B,H,W/2,64): same memory, pixel pairs as 64-channel pixels
     L.Win /= 2;
     L.Cin0 = 64;
@@ -1486,9 +1359,6 @@ int conv_tc_launch(const ConvLayer& Lin, cudaStream_t stream) {
   YOND_REQUIRE(L.Cin0 % 32 == 0 && L.Cin1 % 32 == 0 && L.Cin0 > 0, "conv_tc: Cin must be a multiple of 32 (got %d,%d)",
                L.Cin0, L.Cin1);
   YOND_REQUIRE(L.Cout % 32 == 0, "conv_tc: Cout must be a multiple of 32 (got %d)", L.Cout);
-  static const int env_slab = env_int("YOND_CONV_SLAB", 1);
-  static const int env_T = env_int("YOND_CONV_T", kMaxT);
-  static const int env_dbg = env_int("YOND_CONV_DBG", 0);
   YOND_REQUIRE((double)L.B * L.Hin * L.Win * ((L.mode == CONVT_2X2 || L.mode == CONV_UPSC) ? 4.0 : 1.0) * L.Cout < 4294967296.0,
                "conv_tc: output of %d x %d x %d x %d elements exceeds the 32-bit offset range; split the batch", L.B, L.Hin, L.Win, L.Cout);
   YOND_REQUIRE(L.scale != nullptr || L.shift == nullptr, "conv_tc: a shift vector needs a scale vector");
@@ -1512,13 +1382,11 @@ int conv_tc_launch(const ConvLayer& Lin, cudaStream_t stream) {
   p.CB = conv_tc_channel_block(L.Cin0, L.Cin1);
   p.ncb0 = L.Cin0 / p.CB;
   p.ncb1 = L.Cin1 / p.CB;
-  static const int env_nt = env_int("YOND_CONV_NT", 256);
-  p.NT = p.N < env_nt ? p.N : env_nt;
+  p.NT = p.N < kMaxNT ? p.N : kMaxNT;
   YOND_REQUIRE(p.N % p.NT == 0 && (p.NT & (p.NT - 1)) == 0, "conv_tc: unsupported N=%d", p.N);
   p.tiles_n = p.N / p.NT;
   const uint32_t row_bytes = p.CB * 2;
   const bool conv3 = L.mode == CONV_3X3_S1;
-  p.slab = conv3 ? env_slab : 0;
 
   // sub-tile: TH rows x NB images x TW columns = 128 GEMM rows.  3x3 convs use 8-pixel-wide tiles so that every
   // 8-row swizzle group is one image row of the slab (uniform stride between groups whatever the halo width).
@@ -1541,17 +1409,13 @@ int conv_tc_launch(const ConvLayer& Lin, cudaStream_t stream) {
                  "conv_tc: fused up-sampling is built for resident weights (Cout <= 64); got Cout=%d", L.Cout);
   }
   p.wres = (p.tiles_n == 1 && wres_bytes <= 80 * 1024) ? 1 : 0;
+  YOND_REQUIRE(!p.wres || conv3 || num_astages(p) <= kMaxTabStages, "conv_tc: %d resident-weight stages exceed the stage table (%d)",
+               num_astages(p), kMaxTabStages);
   // CTA pairs for the layers that stream their weights (>= 128 channels): halves the per-SM weight traffic and the
   // shared-memory reads of the B operand, which is what bounds those layers with single-CTA MMAs.
-  static const int env_cta2 = env_int("YOND_CONV_CTA2", 128);  // smallest N tile that runs as a CTA pair (0: never)
-  p.cta2 = (conv3 && p.slab && !p.wres && p.CB == 64 && p.NT >= env_cta2 && env_cta2 > 0 && yond_num_sms() >= 2) ? 1 : 0;
-  // ... and for the resident-weight 64-channel 3x3 layers (incl. the pixel-pair layers): an N = 64 MMA reads 4 KB of A and 2 KB of B
-  // per 48 cycles — exactly the 128 B/clk of shared memory — and runs at 57-60 cycles under TMA-write contention; the pair halves B.
-  static const int env_cta2res = env_int("YOND_CONV_CTA2_RES", 0);
-  if (env_cta2res && conv3 && p.slab && p.wres && p.CB == 64 && p.NT == 64 && L.tail_w == nullptr && yond_num_sms() >= 2) {
-    p.cta2 = 1;
-    wres_bytes /= 2;
-  }
+  // (Resident-weight layers stay single-CTA: at N = 64 the A operand is 4 of the 6 KB an MMA reads, so halving B buys less than
+  // the pair's cross-CTA hand-shakes cost; measured 25 % slower, DESIGN.md section 4.)
+  p.cta2 = (conv3 && !p.wres && p.CB == 64 && p.NT >= kCta2MinNT && yond_num_sms() >= 2) ? 1 : 0;
   if (p.cta2) p.b_stage_bytes /= 2;  // each CTA of the pair holds NT/2 rows of every weight tile
   // T sub-tiles share each weight tile (and one halo slab): stacked along H when the map is tall enough, else along
   // the batch (sub-tile t = images t, t+T, ... of the tile, so that the 8-row groups keep a uniform stride).  T is
@@ -1562,11 +1426,8 @@ int conv_tc_launch(const ConvLayer& Lin, cudaStream_t stream) {
   // Stride-2 / 1x1 / transposed layers stack their sub-tiles along H only (a taller box of whole 128-row tiles).
   int T = 1;
   {
-    static const int env_pair_double = env_int("YOND_CONV_PAIR_DOUBLE", 1);
-    static const int env_acc1 = env_int("YOND_CONV_ACC1", 1);  // 0: never trade the second accumulator stage for a larger T
     // (a CTA pair already halves the weight traffic per SM: it keeps both accumulator stages)
-    int tmax = (p.wres || !env_acc1 || (p.cta2 && env_pair_double)) ? 512 / (2 * p.NT) : 512 / p.NT;
-    if (tmax > env_T) tmax = env_T;
+    int tmax = (p.wres || p.cta2) ? 512 / (2 * p.NT) : 512 / p.NT;
     if (tmax > kMaxT) tmax = kMaxT;
     if (p.NB == 1) {
       while (T * 2 <= tmax && (p.H >= p.TH * T * 2 || (conv3 && p.B >= T * 2))) T *= 2;
@@ -1584,7 +1445,7 @@ int conv_tc_launch(const ConvLayer& Lin, cudaStream_t stream) {
     p.tiles_w = ceil_div(p.W, p.TW);
     p.tiles_h = ceil_div(p.H, SH);
     p.tiles_b = ceil_div(p.B, SBt);
-    slab_w = (conv3 && p.slab) ? p.TW + 2 : p.TW;
+    slab_w = conv3 ? p.TW + 2 : p.TW;
     slab_h = conv3 ? SH + 2 : SH;
     const uint32_t line = (uint32_t)slab_w * row_bytes;  // one image row of one image inside a stage
     p.a_tx_bytes = (uint32_t)slab_h * SBt * line;
@@ -1624,16 +1485,13 @@ int conv_tc_launch(const ConvLayer& Lin, cudaStream_t stream) {
   p.smem_tail_off = p.smem_epi_off + kEpiWarps * 256;
   const size_t smem_bytes = p.smem_tail_off + 1024 + 1024;  // barriers, parameter rows, output-conv table, alignment slack
   p.acc_stages = 2 * p.T * p.NT <= 512 ? 2 : 1;
-  static const int env_split = env_int("YOND_CONV_EPI_SPLIT", 1);
   // Measured inside a GuidedResUnet forward on 8 x 12 MP frames (ncu, profiles/r02_conv_layers_pairing.txt): the pixel-pair
   // layers 890 -> 767 us; every other layer is within +-2 % or loses 4 % (64-channel FiLM layers, residual layers), and the wide
   // layers (N tile >= 128: many visits per warp) lose up to 10 % in isolation — so only the paired layers split.
-  p.epi_split = (env_split && p.acc_stages == 2 && (p.paired || env_split > 1)) ? 1 : 0;
+  p.epi_split = (p.acc_stages == 2 && p.paired) ? 1 : 0;
   p.tmem_cols = p.acc_stages * p.T * p.NT < 32 ? 32 : p.acc_stages * p.T * p.NT;
-  if ((env_dbg & 64) && p.tmem_cols <= 256) p.tmem_cols = 512;
   YOND_REQUIRE(p.tmem_cols <= 512, "conv_tc: TMEM budget exceeded");
 
-  p.dbg = env_dbg;
   p.fd_tiles_n = make_fastdiv((uint32_t)p.tiles_n);
   p.fd_tiles_w = make_fastdiv((uint32_t)p.tiles_w);
   p.fd_tiles_h = make_fastdiv((uint32_t)p.tiles_h);

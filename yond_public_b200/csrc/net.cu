@@ -533,10 +533,10 @@ int forward_selfres(yond_net* n, const float* z, const float* ub, const float* t
 
 // One forward pass; with ws == nullptr only measures workspace bytes and FLOPs.
 //
-// Schedule: the two full-resolution levels (0 and 1) hold ~85 % of the activation bytes; they CAN run in sub-batches
-// small enough for a producer's output to still be in the 126 MB L2 when its consumer reads it (encoder: first conv
-// .. second down-sampling; decoder: second up-sampling .. last 1x1) while the three coarse levels run once over the
-// whole batch.  See the measurement note at SBn below: the split is off by default.
+// Every layer runs once over the whole batch.  The two full-resolution levels hold ~85 % of the activation bytes, and running
+// them in sub-batches small enough for a producer's output to still be in the 126 MB L2 when its consumer reads it was
+// measured on B200 (bench.py, 1280 blocks): the split costs more in launch tails than L2 residency returns (43.7 ms/step
+// unsplit vs 49-60 ms at 16-48 blocks).
 int forward_impl(yond_net* n, const float* z, const float* ub, const float* t, float* y, int B, int H, int W, void* ws,
                  size_t* ws_bytes, double* flops, cudaStream_t s) {
   if (n->arch == YOND_ARCH_SELFRES || n->arch == YOND_ARCH_GSELF) return forward_selfres(n, z, ub, t, y, B, H, W, ws, ws_bytes, flops, s);
@@ -554,16 +554,8 @@ int forward_impl(yond_net* n, const float* z, const float* ub, const float* t, f
   if (!dry && !unet && !res2 && t == nullptr) return yond_set_error(YOND_ERR_INVALID, "guided network needs the per-sample t vector");
   const double head_tail_flops = 2.0 * B * H * W * (36.0 * nf + 4.0 * nf);
   auto px = [&](int lv) { return (size_t)(H >> lv) * (W >> lv); };
-  // Sub-batch of the full-resolution levels.  Measured on B200 (bench.py, 1280 blocks): splitting costs more in
-  // launch tails than L2 residency returns (43.7 ms/step unsplit vs 49-60 ms at 16-48 blocks), so the default is the
-  // whole batch; YOND_SUB_BATCH=n re-enables the split for experiments.
-  static const int env_fuse = getenv("YOND_FUSE_UPSC") ? atoi(getenv("YOND_FUSE_UPSC")) : 1;
-  const bool fuse_up = env_fuse && !n->conv_impl;  // the CUDA-core cross-check path keeps the two reference layers
-  static const int env_sub = getenv("YOND_SUB_BATCH") ? atoi(getenv("YOND_SUB_BATCH")) : 0;
-  int SBn = env_sub > 0 ? env_sub : B;
-  if (SBn < 1) SBn = 1;
-  if (SBn > B) SBn = B;
-  auto buf = [&](int nb, int lv, int C) { return bump.take<bf16>((size_t)nb * px(lv) * C); };
+  const bool fuse_up = !n->conv_impl;  // the CUDA-core cross-check path keeps the two reference layers
+  auto buf = [&](int lv, int C) { return bump.take<bf16>((size_t)B * px(lv) * C); };
 
 #define RUN(expr)                                       \
   do {                                                  \
@@ -619,50 +611,42 @@ int forward_impl(yond_net* n, const float* z, const float* ub, const float* t, f
       film_pending = true;
     }
   }
-  // One residual block on `nb` images starting at image b0 (FiLM rows are per image): x raw, xs = SiLU(x).
-  auto block = [&](int l, int lv, int b0, int nb, const bf16* x, const bf16* xs, bf16* zb, bf16* out, const TailArgs* tail = nullptr) {
-    const int C = n->ch(lv), h = H >> lv, w = W >> lv;
+  // One residual block (FiLM rows are per image): x raw, xs = SiLU(x).
+  auto block = [&](int l, int lv, const bf16* x, const bf16* xs, bf16* zb, bf16* out, const TailArgs* tail = nullptr) {
+    const int h = H >> lv, w = W >> lv;
     const std::string p = "conv" + std::to_string(l);
-    const float* a = va[l] ? va[l] + (size_t)b0 * C : nullptr;
-    const float* bb = vb[l] ? vb[l] + (size_t)b0 * C : nullptr;
+    const float* a = va[l];
+    const float* bb = vb[l];
     if (guided || res2) {  // z = SiLU(conv1(SiLU(x)) * tk + tb); out = conv2(z) + x   (ResUnet2: tk = 1, tb = 0)
-      R.conv(p + ".conv1", nb, h, w, xs, nullptr, a, bb, ACT_SILU, 0.f, nullptr, zb, nullptr);
-      R.conv(p + ".conv2", nb, h, w, zb, nullptr, nullptr, nullptr, ACT_NONE, 0.f, x, out, nullptr, tail);
+      R.conv(p + ".conv1", B, h, w, xs, nullptr, a, bb, ACT_SILU, 0.f, nullptr, zb, nullptr);
+      R.conv(p + ".conv2", B, h, w, zb, nullptr, nullptr, nullptr, ACT_NONE, 0.f, x, out, nullptr, tail);
     } else {  // SNR: z = SiLU(conv1(SiLU(x)) * a1); out = conv2(z) * a2 + x
-      R.conv(p + ".conv1", nb, h, w, xs, nullptr, a, nullptr, ACT_SILU, 0.f, nullptr, zb, nullptr);
-      R.conv(p + ".conv2", nb, h, w, zb, nullptr, bb, nullptr, ACT_NONE, 0.f, x, out, nullptr, tail);
+      R.conv(p + ".conv1", B, h, w, xs, nullptr, a, nullptr, ACT_SILU, 0.f, nullptr, zb, nullptr);
+      R.conv(p + ".conv2", B, h, w, zb, nullptr, bb, nullptr, ACT_NONE, 0.f, x, out, nullptr, tail);
     }
   };
   // The 1x1 output conv (+ input residual, x ub) rides in the epilogue of the last 3x3 layer: its 64 B/px input is never stored.
-  static const int env_tail = getenv("YOND_FUSE_TAIL") ? atoi(getenv("YOND_FUSE_TAIL")) : 1;
-  const bool fuse_tail = env_tail && !n->conv_impl && nf == 32 && H >= 16;
+  const bool fuse_tail = !n->conv_impl && nf == 32 && H >= 16;
   const int C0 = n->ch(0), C1 = n->ch(1), C2 = n->ch(2), C3 = n->ch(3), C4 = n->ch(4);
   const int H1 = H >> 1, W1 = W >> 1, H2 = H >> 2, W2 = W >> 2, H3 = H >> 3, W3 = W >> 3, H4 = H >> 4, W4 = W >> 4;
   // skips of the full-resolution levels (whole batch) and the level-2 hand-over tensors
-  bf16* skip0 = buf(B, 0, C0);
-  bf16* skip1 = buf(B, 1, C1);
+  bf16* skip0 = buf(0, C0);
+  bf16* skip1 = buf(1, C1);
 
   if (unet) {
-    bf16* p2 = buf(B, 2, C1);  // pooled level-1 output
-    // sub-batch temporaries
-    bf16* a0 = buf(SBn, 0, C0);
-    bf16* p1 = buf(SBn, 1, C0);
-    bf16* a1 = buf(SBn, 1, C1);
-    for (int b0 = 0; b0 < B; b0 += SBn) {
-      const int nb = B - b0 < SBn ? B - b0 : SBn;
-      bf16* s0 = skip0 + (size_t)b0 * px(0) * C0;
-      bf16* s1 = skip1 + (size_t)b0 * px(1) * C1;
-      RUN(head_conv_launch(z + (size_t)b0 * px(0) * 4, ubn ? ubn + b0 : nullptr, n->head_w, n->f32["conv1_1.bias"], nb, H, W, nf, 0.2f, a0, nullptr, s));
-      R.conv("conv1_2", nb, H, W, a0, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, s0, nullptr);
-      RUN(maxpool2_launch(s0, p1, nb, H, W, C0, s));
-      R.conv("conv2_1", nb, H1, W1, p1, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, a1, nullptr);
-      R.conv("conv2_2", nb, H1, W1, a1, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, s1, nullptr);
-      RUN(maxpool2_launch(s1, p2 + (size_t)b0 * px(2) * C1, nb, H1, W1, C1, s));
-    }
-    // coarse levels, whole batch
-    bf16* a2 = buf(B, 2, C2); bf16* c3 = buf(B, 2, C2); bf16* p3 = buf(B, 3, C2);
-    bf16* a3 = buf(B, 3, C3); bf16* c4 = buf(B, 3, C3); bf16* p4 = buf(B, 4, C3);
-    bf16* a4 = buf(B, 4, C4); bf16* c5 = buf(B, 4, C4);
+    bf16* p2 = buf(2, C1);  // pooled level-1 output
+    bf16* a0 = buf(0, C0);
+    bf16* p1 = buf(1, C0);
+    bf16* a1 = buf(1, C1);
+    RUN(head_conv_launch(z, ubn, n->head_w, n->f32["conv1_1.bias"], B, H, W, nf, 0.2f, a0, nullptr, s));
+    R.conv("conv1_2", B, H, W, a0, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, skip0, nullptr);
+    RUN(maxpool2_launch(skip0, p1, B, H, W, C0, s));
+    R.conv("conv2_1", B, H1, W1, p1, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, a1, nullptr);
+    R.conv("conv2_2", B, H1, W1, a1, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, skip1, nullptr);
+    RUN(maxpool2_launch(skip1, p2, B, H1, W1, C1, s));
+    bf16* a2 = buf(2, C2); bf16* c3 = buf(2, C2); bf16* p3 = buf(3, C2);
+    bf16* a3 = buf(3, C3); bf16* c4 = buf(3, C3); bf16* p4 = buf(4, C3);
+    bf16* a4 = buf(4, C4); bf16* c5 = buf(4, C4);
     R.conv("conv3_1", B, H2, W2, p2, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, a2, nullptr);
     R.conv("conv3_2", B, H2, W2, a2, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c3, nullptr);
     RUN(maxpool2_launch(c3, p3, B, H2, W2, C2, s));
@@ -671,94 +655,77 @@ int forward_impl(yond_net* n, const float* z, const float* ub, const float* t, f
     RUN(maxpool2_launch(c4, p4, B, H3, W3, C3, s));
     R.conv("conv5_1", B, H4, W4, p4, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, a4, nullptr);
     R.conv("conv5_2", B, H4, W4, a4, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c5, nullptr);
-    bf16* u6 = buf(B, 3, C3); bf16* t6 = buf(B, 3, C3); bf16* c6 = buf(B, 3, C3);
+    bf16* u6 = buf(3, C3); bf16* t6 = buf(3, C3); bf16* c6 = buf(3, C3);
     R.conv("upv6", B, H4, W4, c5, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u6, nullptr);
     R.conv("conv6_1", B, H3, W3, u6, c4, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, t6, nullptr);
     R.conv("conv6_2", B, H3, W3, t6, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c6, nullptr);
-    bf16* u7 = buf(B, 2, C2); bf16* t7 = buf(B, 2, C2); bf16* c7 = buf(B, 2, C2);
+    bf16* u7 = buf(2, C2); bf16* t7 = buf(2, C2); bf16* c7 = buf(2, C2);
     R.conv("upv7", B, H3, W3, c6, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u7, nullptr);
     R.conv("conv7_1", B, H2, W2, u7, c3, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, t7, nullptr);
     R.conv("conv7_2", B, H2, W2, t7, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c7, nullptr);
-    // decoder of the full-resolution levels, per sub-batch
-    bf16* u8 = buf(SBn, 1, C1); bf16* t8 = buf(SBn, 1, C1); bf16* c8 = buf(SBn, 1, C1);
-    bf16* u9 = buf(SBn, 0, C0); bf16* t9 = buf(SBn, 0, C0); bf16* c9 = buf(SBn, 0, C0);
-    for (int b0 = 0; b0 < B; b0 += SBn) {
-      const int nb = B - b0 < SBn ? B - b0 : SBn;
-      R.conv("upv8", nb, H2, W2, c7 + (size_t)b0 * px(2) * C2, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u8, nullptr);
-      R.conv("conv8_1", nb, H1, W1, u8, skip1 + (size_t)b0 * px(1) * C1, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, t8, nullptr);
-      R.conv("conv8_2", nb, H1, W1, t8, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c8, nullptr);
-      R.conv("upv9", nb, H1, W1, c8, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u9, nullptr);
-      R.conv("conv9_1", nb, H, W, u9, skip0 + (size_t)b0 * px(0) * C0, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, t9, nullptr);
-      if (fuse_tail) {
-        const TailArgs ta{n->tail_w, dry ? nullptr : n->f32["conv10_1.bias"], z + (size_t)b0 * px(0) * 4, ubn ? ubn + b0 : nullptr,
-                          y + (size_t)b0 * px(0) * 4, n->res};
-        R.conv("conv9_2", nb, H, W, t9, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c9, nullptr, &ta);
-      } else {
-        R.conv("conv9_2", nb, H, W, t9, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c9, nullptr);
-        RUN(tail_conv_launch(c9, n->tail_w, n->f32["conv10_1.bias"], z + (size_t)b0 * px(0) * 4, ubn ? ubn + b0 : nullptr, n->res, nb,
-                             H, W, nf, y + (size_t)b0 * px(0) * 4, s));
-      }
+    bf16* u8 = buf(1, C1); bf16* t8 = buf(1, C1); bf16* c8 = buf(1, C1);
+    bf16* u9 = buf(0, C0); bf16* t9 = buf(0, C0); bf16* c9 = buf(0, C0);
+    R.conv("upv8", B, H2, W2, c7, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u8, nullptr);
+    R.conv("conv8_1", B, H1, W1, u8, skip1, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, t8, nullptr);
+    R.conv("conv8_2", B, H1, W1, t8, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c8, nullptr);
+    R.conv("upv9", B, H1, W1, c8, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u9, nullptr);
+    R.conv("conv9_1", B, H, W, u9, skip0, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, t9, nullptr);
+    if (fuse_tail) {
+      const TailArgs ta{n->tail_w, dry ? nullptr : n->f32["conv10_1.bias"], z, ubn, y, n->res};
+      R.conv("conv9_2", B, H, W, t9, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c9, nullptr, &ta);
+    } else {
+      R.conv("conv9_2", B, H, W, t9, nullptr, nullptr, nullptr, ACT_LRELU, 0.2f, nullptr, c9, nullptr);
+      RUN(tail_conv_launch(c9, n->tail_w, n->f32["conv10_1.bias"], z, ubn, n->res, B, H, W, nf, y, s));
     }
   } else {
-    bf16* x2 = buf(B, 2, C2);   // pool2 output (raw) and its SiLU: inputs of the level-2 block
-    bf16* x2s = buf(B, 2, C2);
-    bf16* x0 = buf(SBn, 0, C0); bf16* x0s = buf(SBn, 0, C0); bf16* z0 = buf(SBn, 0, C0);
-    bf16* x1 = buf(SBn, 1, C1); bf16* x1s = buf(SBn, 1, C1); bf16* z1 = buf(SBn, 1, C1);
-    for (int b0 = 0; b0 < B; b0 += SBn) {
-      const int nb = B - b0 < SBn ? B - b0 : SBn;
-      bf16* s0 = skip0 + (size_t)b0 * px(0) * C0;
-      bf16* s1 = skip1 + (size_t)b0 * px(1) * C1;
-      RUN(head_conv_launch(z + (size_t)b0 * px(0) * 4, ubn ? ubn + b0 : nullptr, n->head_w, n->f32["conv_in.bias"], nb, H, W, nf, res2 ? 0.2f : 0.01f, x0, x0s, s));
-      film_join();
-      block(1, 0, b0, nb, x0, x0s, z0, s0);
-      // stride-2 conv, no activation (modules.py:117-125); the dual store feeds the next block
-      R.conv("pool1.conv", nb, H, W, s0, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x1, x1s);
-      block(2, 1, b0, nb, x1, x1s, z1, s1);
-      R.conv("pool2.conv", nb, H1, W1, s1, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x2 + (size_t)b0 * px(2) * C2,
-             x2s + (size_t)b0 * px(2) * C2);
-    }
-    bf16* zb2 = buf(B, 2, C2); bf16* c3 = buf(B, 2, C2);
-    bf16* x3 = buf(B, 3, C3); bf16* x3s = buf(B, 3, C3); bf16* zb3 = buf(B, 3, C3); bf16* c4 = buf(B, 3, C3);
-    bf16* x4 = buf(B, 4, C4); bf16* x4s = buf(B, 4, C4); bf16* zb4 = buf(B, 4, C4); bf16* c5 = buf(B, 4, C4);
-    block(3, 2, 0, B, x2, x2s, zb2, c3);
+    bf16* x2 = buf(2, C2);   // pool2 output (raw) and its SiLU: inputs of the level-2 block
+    bf16* x2s = buf(2, C2);
+    bf16* x0 = buf(0, C0); bf16* x0s = buf(0, C0); bf16* z0 = buf(0, C0);
+    bf16* x1 = buf(1, C1); bf16* x1s = buf(1, C1); bf16* z1 = buf(1, C1);
+    RUN(head_conv_launch(z, ubn, n->head_w, n->f32["conv_in.bias"], B, H, W, nf, res2 ? 0.2f : 0.01f, x0, x0s, s));
+    film_join();
+    block(1, 0, x0, x0s, z0, skip0);
+    // stride-2 conv, no activation (modules.py:117-125); the dual store feeds the next block
+    R.conv("pool1.conv", B, H, W, skip0, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x1, x1s);
+    block(2, 1, x1, x1s, z1, skip1);
+    R.conv("pool2.conv", B, H1, W1, skip1, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x2, x2s);
+    bf16* zb2 = buf(2, C2); bf16* c3 = buf(2, C2);
+    bf16* x3 = buf(3, C3); bf16* x3s = buf(3, C3); bf16* zb3 = buf(3, C3); bf16* c4 = buf(3, C3);
+    bf16* x4 = buf(4, C4); bf16* x4s = buf(4, C4); bf16* zb4 = buf(4, C4); bf16* c5 = buf(4, C4);
+    block(3, 2, x2, x2s, zb2, c3);
     R.conv("pool3.conv", B, H2, W2, c3, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x3, x3s);
-    block(4, 3, 0, B, x3, x3s, zb3, c4);
+    block(4, 3, x3, x3s, zb3, c4);
     R.conv("pool4.conv", B, H3, W3, c4, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x4, x4s);
-    block(5, 4, 0, B, x4, x4s, zb4, c5);
-    bf16* u6 = buf(B, 3, C3); bf16* c6 = buf(B, 3, C3);
+    block(5, 4, x4, x4s, zb4, c5);
+    bf16* u6 = buf(3, C3); bf16* c6 = buf(3, C3);
     R.conv("upv6", B, H4, W4, c5, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u6, nullptr);
     R.conv("conv6.short_cut.0", B, H3, W3, u6, c4, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x3, x3s);  // x3/x3s are free again
-    block(6, 3, 0, B, x3, x3s, zb3, c6);
-    bf16* u7 = buf(B, 2, C2); bf16* c7 = buf(B, 2, C2);
+    block(6, 3, x3, x3s, zb3, c6);
+    bf16* u7 = buf(2, C2); bf16* c7 = buf(2, C2);
     R.conv("upv7", B, H3, W3, c6, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u7, nullptr);
     R.conv("conv7.short_cut.0", B, H2, W2, u7, c3, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x2, x2s);
-    block(7, 2, 0, B, x2, x2s, zb2, c7);
-    bf16* u8 = buf(SBn, 1, C1); bf16* c8 = buf(SBn, 1, C1);
-    bf16* u9 = buf(SBn, 0, C0); bf16* c9 = buf(SBn, 0, C0);
-    for (int b0 = 0; b0 < B; b0 += SBn) {
-      const int nb = B - b0 < SBn ? B - b0 : SBn;
-      if (fuse_up && n->conv.count("conv8.upsc")) {
-        R.conv("conv8.upsc", nb, H2, W2, c7 + (size_t)b0 * px(2) * C2, skip1 + (size_t)b0 * px(1) * C1, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x1, x1s);
-      } else {
-        R.conv("upv8", nb, H2, W2, c7 + (size_t)b0 * px(2) * C2, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u8, nullptr);
-        R.conv("conv8.short_cut.0", nb, H1, W1, u8, skip1 + (size_t)b0 * px(1) * C1, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x1, x1s);
-      }
-      block(8, 1, b0, nb, x1, x1s, z1, c8);
-      if (fuse_up && n->conv.count("conv9.upsc")) {
-        R.conv("conv9.upsc", nb, H1, W1, c8, skip0 + (size_t)b0 * px(0) * C0, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x0, x0s);
-      } else {
-        R.conv("upv9", nb, H1, W1, c8, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u9, nullptr);
-        R.conv("conv9.short_cut.0", nb, H, W, u9, skip0 + (size_t)b0 * px(0) * C0, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x0, x0s);
-      }
-      if (fuse_tail) {
-        const TailArgs ta{n->tail_w, dry ? nullptr : n->f32["conv10.bias"], z + (size_t)b0 * px(0) * 4, ubn ? ubn + b0 : nullptr,
-                          y + (size_t)b0 * px(0) * 4, n->res};
-        block(9, 0, b0, nb, x0, x0s, z0, c9, &ta);
-      } else {
-        block(9, 0, b0, nb, x0, x0s, z0, c9);
-        RUN(tail_conv_launch(c9, n->tail_w, n->f32["conv10.bias"], z + (size_t)b0 * px(0) * 4, ubn ? ubn + b0 : nullptr, n->res, nb, H, W,
-                             nf, y + (size_t)b0 * px(0) * 4, s));
-      }
+    block(7, 2, x2, x2s, zb2, c7);
+    bf16* u8 = buf(1, C1); bf16* c8 = buf(1, C1);
+    bf16* u9 = buf(0, C0); bf16* c9 = buf(0, C0);
+    if (fuse_up && n->conv.count("conv8.upsc")) {
+      R.conv("conv8.upsc", B, H2, W2, c7, skip1, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x1, x1s);
+    } else {
+      R.conv("upv8", B, H2, W2, c7, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u8, nullptr);
+      R.conv("conv8.short_cut.0", B, H1, W1, u8, skip1, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x1, x1s);
+    }
+    block(8, 1, x1, x1s, z1, c8);
+    if (fuse_up && n->conv.count("conv9.upsc")) {
+      R.conv("conv9.upsc", B, H1, W1, c8, skip0, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x0, x0s);
+    } else {
+      R.conv("upv9", B, H1, W1, c8, nullptr, nullptr, nullptr, ACT_NONE, 0.f, nullptr, u9, nullptr);
+      R.conv("conv9.short_cut.0", B, H, W, u9, skip0, nullptr, nullptr, ACT_NONE, 0.f, nullptr, x0, x0s);
+    }
+    if (fuse_tail) {
+      const TailArgs ta{n->tail_w, dry ? nullptr : n->f32["conv10.bias"], z, ubn, y, n->res};
+      block(9, 0, x0, x0s, z0, c9, &ta);
+    } else {
+      block(9, 0, x0, x0s, z0, c9);
+      RUN(tail_conv_launch(c9, n->tail_w, n->f32["conv10.bias"], z, ubn, n->res, B, H, W, nf, y, s));
     }
   }
   film_join();
@@ -918,23 +885,6 @@ int yond_conv2d(int mode, int impl, int B, int Hin, int Win, int Cin0, int Cin1,
   c.scale = scale; c.shift = shift; c.act = act; c.slope = slope; c.res = (const bf16*)res;
   c.out0 = (bf16*)out0; c.out1 = (bf16*)out1;
   int rc = impl ? conv_ref_launch(c, (cudaStream_t)stream) : conv_tc_launch(c, (cudaStream_t)stream);
-  if (const char* reps_s = getenv("YOND_CONV_REPS")) {  // bring-up micro-benchmark: time back-to-back launches
-    const int reps = atoi(reps_s);
-    cudaEvent_t e0, e1;
-    cudaEventCreate(&e0);
-    cudaEventCreate(&e1);
-    for (int i = 0; i < 3 && !rc; ++i) rc = conv_tc_launch(c, (cudaStream_t)stream);
-    cudaEventRecord(e0, (cudaStream_t)stream);
-    for (int i = 0; i < reps && !rc; ++i) rc = conv_tc_launch(c, (cudaStream_t)stream);
-    cudaEventRecord(e1, (cudaStream_t)stream);
-    cudaEventSynchronize(e1);
-    float ms = 0;
-    cudaEventElapsedTime(&ms, e0, e1);
-    fprintf(stderr, "conv2d_bench mode=%d B=%d HxW=%dx%d Cin=%d+%d Cout=%d: %.2f us/launch\n", mode, B, Hin, Win, Cin0, Cin1, Cout,
-            1e3 * ms / (reps > 0 ? reps : 1));
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-  }
   cudaError_t e = cudaStreamSynchronize((cudaStream_t)stream);
   cudaFree(dw);
   if (dwp) cudaFree(dwp);

@@ -59,7 +59,8 @@ __device__ __forceinline__ int reflect_once(int i, int n) {
 // of the round are issued up front), stores the kRows sets of column sums, the scan warps prefix kRows x NQ rows of the
 // staging array (two at a time, interleaved), the writers emit kRows image rows: three block barriers per kRows rows
 // instead of two per row, and kRows-fold more independent work between them.
-template <bool kSq, int kCols, bool kBayer, bool kNarrow, int kRows>  // kCols = 256, or 160 when a whole row plus both halos fits
+constexpr int kRows = 4;
+template <bool kSq, int kCols, bool kBayer, bool kNarrow>  // kCols = 256, or 160 when a whole row plus both halos fits
 __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, float4* __restrict__ out0,
                                                                 float4* __restrict__ out1, int B, int h, int w, int k, int op,
                                                                 int rows_per_strip, const float4* aux,  // may alias out2
@@ -884,29 +885,27 @@ BoxSrc packed_src(const float* x, int h, int w) {
   return s;
 }
 
-template <bool SQ, int COLS, bool BAYER, bool NARROW, int R>
+template <bool SQ, int COLS, bool BAYER, bool NARROW>
 int launch_box(dim3 g, cudaStream_t s, const BoxSrc& src, float4* o0, float4* o1, int B, int h, int w, int k, int op, int rows_per_strip,
                const float4* ax, float4* o2) {
-  constexpr size_t bytes = (size_t)R * (SQ ? 8 : 4) * (COLS == 256 ? COLS : COLS + 33) * sizeof(double);  // = [kRows][NQ][PITCH]
+  constexpr size_t bytes = (size_t)kRows * (SQ ? 8 : 4) * (COLS == 256 ? COLS : COLS + 33) * sizeof(double);  // = [kRows][NQ][PITCH]
   static std::once_flag once;
   static cudaError_t err = cudaSuccess;
   std::call_once(once, [] {
-    err = cudaFuncSetAttribute(box_fused_kernel<SQ, COLS, BAYER, NARROW, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    err = cudaFuncSetAttribute(box_fused_kernel<SQ, COLS, BAYER, NARROW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
   });
   if (err != cudaSuccess) return yond_set_error(YOND_ERR_CUDA, "box filter: cudaFuncSetAttribute failed: %s", cudaGetErrorString(err));
-  box_fused_kernel<SQ, COLS, BAYER, NARROW, R><<<g, kBoxThreads, bytes, s>>>(src, o0, o1, B, h, w, k, op, rows_per_strip, ax, o2);
+  box_fused_kernel<SQ, COLS, BAYER, NARROW><<<g, kBoxThreads, bytes, s>>>(src, o0, o1, B, h, w, k, op, rows_per_strip, ax, o2);
   return YOND_OK;
 }
 
 int box_pass(const BoxSrc& src, bool bayer, float* out0, float* out1, int B, int h, int w, int k, bool with_sq, int op,
              cudaStream_t s, const float* aux = nullptr, float* out2 = nullptr) {
-  static const int env_rows = getenv("YOND_BOX_ROWS") ? atoi(getenv("YOND_BOX_ROWS")) : 0;
-  static const int env_narrow = getenv("YOND_BOX_NARROW") ? atoi(getenv("YOND_BOX_NARROW")) : 1;
   const int r = k / 2;
   // narrow images (SIDD blocks): 256 / w whole images per block, no halo threads; needs a single reflection (r < w - 1)
-  const bool multi = env_narrow && 2 * w <= 256 && w >= 2 * r + 2;
+  const bool multi = 2 * w <= 256 && w >= 2 * r + 2;
   const bool narrow = !multi && w + 2 * r <= 160;
-  const int rows_per_strip = env_rows > 0 ? env_rows : 64;
+  const int rows_per_strip = 64;
   const int cols = narrow ? 160 : 256;
   const int outc = cols - 2 * r;
   dim3 g(ceil_div(w, outc), ceil_div(h, rows_per_strip), B);
@@ -917,15 +916,8 @@ int box_pass(const BoxSrc& src, bool bayer, float* out0, float* out1, int B, int
   const float4* ax = reinterpret_cast<const float4*>(aux);
   float4* o2 = reinterpret_cast<float4*>(out2);
   const int opx = with_sq ? op : OP_MEAN;
-  static const int env_r = getenv("YOND_BOX_R") ? atoi(getenv("YOND_BOX_R")) : 4;  // image rows per barrier round
-#define YOND_BOX_R(SQ, COLS, BAYER, NARROW, R) \
-  rc = launch_box<SQ, COLS, BAYER, NARROW, R>(g, s, src, o0, o1, B, h, w, k, opx, rows_per_strip, ax, o2)
-#define YOND_BOX(SQ, COLS, BAYER, NARROW)                          \
-  do {                                                             \
-    if (env_r >= 4) YOND_BOX_R(SQ, COLS, BAYER, NARROW, 4);        \
-    else if (env_r >= 2) YOND_BOX_R(SQ, COLS, BAYER, NARROW, 2);   \
-    else YOND_BOX_R(SQ, COLS, BAYER, NARROW, 1);                   \
-  } while (0)
+#define YOND_BOX(SQ, COLS, BAYER, NARROW) \
+  rc = launch_box<SQ, COLS, BAYER, NARROW>(g, s, src, o0, o1, B, h, w, k, opx, rows_per_strip, ax, o2)
 #define YOND_BOX_B(SQ, COLS, NARROW)                        \
   do {                                                      \
     if (bayer) YOND_BOX(SQ, COLS, true, NARROW);            \
@@ -943,7 +935,6 @@ int box_pass(const BoxSrc& src, bool bayer, float* out0, float* out1, int B, int
   }
 #undef YOND_BOX_B
 #undef YOND_BOX
-#undef YOND_BOX_R
   if (rc) return rc;
   YOND_LAUNCH_CHECK();
   return YOND_OK;
