@@ -214,6 +214,35 @@ size_t yond_nlf_fit_work_bytes(int nseg);
 int yond_nlf_fit(const float* var, const float* mean, const float* lap, size_t seg_len, int nseg, const double* quants_host,
                  int nq, double* regs_dev, double* detail_dev, void* work, void* stream);
 
+/* ---- the self estimate of frames of different sizes in one pass — YOND_SIDD.py:338-341 (round 1 of IterDenoise on the
+ * full-resolution frame `lr_path_full` when it exists), :62-71 (SelfNLF), :22-49 (score3), :77-86 + utils/isp_algos.py:345-365 (fit).
+ * yond_frame_geom: one record per frame, in DEVICE memory.  Frame i's packed maps (H/2, W/2, 4) sit at float offset `off` of the
+ *   concatenated var / mean / lap buffers (off = sum of H*W over the frames before it).
+ * yond_nlf_maps_frames: the self maps (mode 0 of yond_nlf_maps_bayer) of `nframes` float32 Bayer frames given by `frames_dev`, in
+ *   one launch per box pass whatever the sizes.  max_H / max_W: the largest H and W of the records (they size the grid; CTAs past a
+ *   smaller frame's extent return at once).  Every frame needs even H, W with H/2 and W/2 larger than k/2; frames narrower than the
+ *   box filter's block take the same wide layout as large frames.  `work`: 16 bytes per packed pixel of all frames (sum of H*W*4
+ *   bytes), 16-byte aligned.
+ * yond_nlf_fit_ragged: yond_nlf_fit over segments of different lengths: segment s is [seg_off_dev[s], seg_off_dev[s + 1]) of the
+ *   maps (a DEVICE array of nseg + 1 float offsets, multiples of 4).  max_seg_len (host) is the longest segment; it sizes the grids.
+ *   The percentile ranks and weights are computed per segment on the device.  `work`: yond_nlf_fit_ragged_work_bytes(nseg), 256-byte
+ *   aligned.  Same outputs and arithmetic as yond_nlf_fit.
+ * yond_seg_max: seg_max[s] = max(x, 0) over the nseg contiguous segments of seg_len floats of x (the blocks of image s) — the bound
+ *   of the fallback bias table when round 1 estimated on the full frame (:393-395: the maximum of the blocks, not of lr_full).
+ *   seg_len a multiple of 4, x 16-byte aligned. */
+typedef struct yond_frame_geom {
+  const float* base; /* the (H, W) float32 Bayer frame */
+  int H, W;
+  long long off;
+} yond_frame_geom;
+int yond_nlf_maps_frames(const yond_frame_geom* frames_dev, int nframes, int max_H, int max_W, float* var, float* mean, float* lap,
+                         int k, void* work, void* stream);
+size_t yond_nlf_fit_ragged_work_bytes(int nseg);
+int yond_nlf_fit_ragged(const float* var, const float* mean, const float* lap, const unsigned long long* seg_off_dev,
+                        size_t max_seg_len, int nseg, const double* quants_host, int nq, double* regs_dev, double* detail_dev,
+                        void* work, void* stream);
+int yond_seg_max(const float* x, size_t seg_len, int nseg, float* seg_max, void* stream);
+
 /* ---- the VST parameter chain on the device — YOND_SIDD.py:356 (round 1) / :438-447 (round 2 guards), :252-269,
  * :284-285 (bias source, VST(0), VST(scale), t = nsr*1.03), utils/isp_algos.py:179-231 (sigma row of the BiasLUT),
  * :49-140 (get_bias: the numeric Poisson (*) Gaussian fallback table — SURVEY 8(f)-2, generated on the device).

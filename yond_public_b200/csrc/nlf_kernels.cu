@@ -60,11 +60,15 @@ __device__ __forceinline__ int reflect_once(int i, int n) {
 // staging array (two at a time, interleaved), the writers emit kRows image rows: three block barriers per kRows rows
 // instead of two per row, and kRows-fold more independent work between them.
 constexpr int kRows = 4;
-template <bool kSq, int kCols, bool kBayer, bool kNarrow>  // kCols = 256, or 160 when a whole row plus both halos fits
+// kRagged (wide layout): blockIdx.z picks a frame record (yond_frame_geom: its own h, w, Bayer source and map offset; a packed source
+// is `src.base` + that offset) instead of an image of one (B, h, w) geometry.  The grid is sized by the largest frame; the CTAs past
+// a smaller frame's column blocks or strips return before the first barrier.  The arithmetic is the uniform form's.
+template <bool kSq, int kCols, bool kBayer, bool kNarrow, bool kRagged = false>  // kCols = 256, or 160 when a whole row plus both halos fits
 __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, float4* __restrict__ out0,
                                                                 float4* __restrict__ out1, int B, int h, int w, int k, int op,
                                                                 int rows_per_strip, const float4* aux,  // may alias out2
-                                                                float4* __restrict__ out2) {
+                                                                float4* __restrict__ out2, const yond_frame_geom* frames) {
+  static_assert(!(kRagged && kNarrow), "frames of different sizes take the wide layout");
   constexpr int NQ = kSq ? 8 : 4;
   constexpr int CH = kCols / 32;           // columns per scan chunk (8 or 5)
   // Staging rows.  kCols = 256: 16-byte slots (column pairs) XOR-swizzled, slot s -> s ^ ((s >> 3) & 3): 64-bit accesses of 16
@@ -76,6 +80,19 @@ __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, floa
   extern __shared__ __align__(16) double S[];  // [kRows][NQ][PITCH]
   const int r = k / 2;
   const int outc = kCols - 2 * r;
+  size_t frame_px = 0;  // kRagged: the frame's first packed pixel in the concatenated outputs
+  // `if constexpr` keeps the ragged code out of the uniform instantiations' IR: a plain `if` on kRagged changes their schedule
+  if constexpr (kRagged) {  // read once per CTA; the frame is its own image 0 of the source and of the outputs
+    const yond_frame_geom f = frames[blockIdx.z];
+    h = f.H / 2;
+    w = f.W / 2;
+    if ((int)blockIdx.x * outc >= w || (int)blockIdx.y * rows_per_strip >= h) return;
+    src.base = kBayer ? f.base : src.base + f.off;
+    src.row_len = kBayer ? f.W : 4 * w;
+    src.blk_w = w;
+    src.img_stride = 0;
+    frame_px = f.off / 4;
+  }
   const int c = threadIdx.x, lane = c & 31, warp = c >> 5;
   int b, col_out, col_src, img0 = 0;
   bool colthread, writer;
@@ -93,6 +110,7 @@ __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, floa
     colthread = c < kCols;
     writer = (c >= r) && (c < r + outc) && (col_out < w);
   }
+  if constexpr (kRagged) b = 0;
   // Wide layout: the thread that WRITES output column oc is thread oc + r, so that its upper window end P[oc + r] sits at its own
   // (aligned) position; only the lower end P[oc - r - 1] is an unaligned access.
   int col_w = col_out;
@@ -272,7 +290,8 @@ __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, floa
           a[q] = Sq[hi_idx] - (lo_idx >= 0 ? Sq[lo_idx] : 0.0);
           if (kNarrow && e1_idx >= 0) a[q] += Sq[e1_idx] - Sq[e0_idx];
         }
-        const size_t o = ((size_t)b * h + (i + j)) * w + col_w;
+        size_t o = ((size_t)b * h + (i + j)) * w + col_w;
+        if constexpr (kRagged) o += frame_px;
         const float4 m = make_float4((float)(a[0] * inv), (float)(a[1] * inv), (float)(a[2] * inv), (float)(a[3] * inv));
         if (!kSq || op == OP_MEAN) {
           out0[o] = m;
@@ -360,13 +379,24 @@ __device__ __forceinline__ void stream_f4(const float4* __restrict__ d4, size_t 
   }
 }
 
+// Segments of the fit: uniform, segment s = [s*n, (s+1)*n); kRagged, [seg_off[s], seg_off[s+1]) (n becomes that segment's length).
+template <bool kRagged>
+__device__ __forceinline__ size_t seg_begin(size_t& n, const unsigned long long* seg_off, int s) {
+  if (!kRagged) return (size_t)s * n;
+  const size_t o = seg_off[s];
+  n = seg_off[s + 1] - o;
+  return o;
+}
+
 // First level, optionally fused with the score3 bin pass (get_threshold 'score3', YOND_SIDD.py:34-43): npeaks[i] counts
 // the `mean` bins that hold a pixel with lap <= ths[i], i.e. the bins whose SMALLEST lap is <= ths[i] — so the pass only
 // needs the per-bin minimum of lap and does not depend on the thresholds: it rides along with the first histogram.
-template <bool kBinMin>
+template <bool kBinMin, bool kRagged>
 __global__ void __launch_bounds__(256) hist0_kernel(const float* __restrict__ d, const float* __restrict__ mean, size_t n,
-                                                    SelectWork* wk, unsigned int* __restrict__ binmin) {
-  d += (size_t)blockIdx.y * n;  // one segment (image) per blockIdx.y
+                                                    SelectWork* wk, unsigned int* __restrict__ binmin,
+                                                    const unsigned long long* seg_off) {
+  const size_t seg0 = seg_begin<kRagged>(n, seg_off, blockIdx.y);
+  d += seg0;  // one segment (image) per blockIdx.y
   if (wk) wk += blockIdx.y;
   if (kBinMin) binmin += (size_t)blockIdx.y * 1024;  // smallest lap key per `mean` bin, ~0u = bin empty
   __shared__ unsigned int h[2048];
@@ -379,7 +409,7 @@ __global__ void __launch_bounds__(256) hist0_kernel(const float* __restrict__ d,
   if (!kBinMin) {
     stream_f4(d4, n / 4, [&](float e) { atomicAdd(&h[f2key(e) >> 21], 1u); });
   } else {
-    const float4* m4 = reinterpret_cast<const float4*>(mean + (size_t)blockIdx.y * n);
+    const float4* m4 = reinterpret_cast<const float4*>(mean + seg0);
     auto one = [&](float l, float m) {
       const uint32_t k = f2key(l);
       if (wk) atomicAdd(&h[k >> 21], 1u);
@@ -448,8 +478,10 @@ __device__ __forceinline__ int find_bin(const unsigned int* __restrict__ pre, in
   return lo;
 }
 
+template <bool kRagged>  // kRagged: one row of kMaxRanks ranks per segment
 __global__ void __launch_bounds__(1024) select0_kernel(SelectWork* wk, const unsigned long long* __restrict__ ranks, int nranks) {
   wk += blockIdx.x;
+  if (kRagged) ranks += (size_t)blockIdx.x * kMaxRanks;
   __shared__ unsigned int pre[2048];
   __shared__ unsigned int wsum[32];
   __shared__ int s_bin[kMaxRanks];
@@ -489,10 +521,12 @@ __device__ __forceinline__ void load_slot_table(const SelectWork* wk, signed cha
   const int nq = wk->nq_live;
   if ((int)threadIdx.x < nq) s1tab[wk->q_prefix[threadIdx.x] >> ((wk->level - 1) * 11)] = (signed char)wk->q_slot1[threadIdx.x];
 }
-__global__ void __launch_bounds__(kHist1Threads) hist1_kernel(const float* __restrict__ d, size_t n, SelectWork* wk) {
+template <bool kRagged>
+__global__ void __launch_bounds__(kHist1Threads) hist1_kernel(const float* __restrict__ d, size_t n, SelectWork* wk,
+                                                              const unsigned long long* seg_off) {
   extern __shared__ unsigned int hs[];  // [kHist1Slots][2048] counters, then the 2048-entry prefix -> slot table (int8)
   signed char* s1tab = reinterpret_cast<signed char*>(hs + kHist1Slots * 2048);
-  d += (size_t)blockIdx.y * n;
+  d += seg_begin<kRagged>(n, seg_off, blockIdx.y);
   wk += blockIdx.y;
   const int nsh = min(wk->nslot1, kHist1Slots);
   for (int i = threadIdx.x; i < nsh * 2048; i += blockDim.x) hs[i] = 0u;
@@ -597,16 +631,18 @@ __global__ void __launch_bounds__(1024) select1_kernel(SelectWork* wk, int nrank
 // the other one is due: sparse hits (natural data: ~0.2 %) take the lean form with 6 blocks per SM, dense hits the privatised one.
 constexpr int kHist2Slots = 16;
 __device__ __forceinline__ bool hist2_dense(const SelectWork* wk, size_t n) { return (size_t)wk->hist2_hits > n / 16; }
-template <bool privatise>
-__global__ void __launch_bounds__(256) hist2_kernel(const float* __restrict__ d, size_t n, SelectWork* wk) {
+template <bool privatise, bool kRagged>  // kRagged: the dense / sparse choice is made per segment, on its own length
+__global__ void __launch_bounds__(256) hist2_kernel(const float* __restrict__ d, size_t n, SelectWork* wk,
+                                                    const unsigned long long* seg_off) {
   extern __shared__ unsigned int hs2[];  // [kHist2Slots][1024] when privatise
+  const size_t seg0 = seg_begin<kRagged>(n, seg_off, blockIdx.y);
   if (hist2_dense(wk + blockIdx.y, n) != privatise) return;
   __shared__ signed char s1tab[2048];
   __shared__ unsigned int bm[kMaxRanks * 64];
   __shared__ uint32_t qpre[kMaxRanks];
   __shared__ int qs2[kMaxRanks];
   __shared__ int nq;
-  d += (size_t)blockIdx.y * n;
+  d += seg0;
   wk += blockIdx.y;
   const int ns1 = wk->nslot1;
   const int nsh = privatise ? min(wk->nslot2, kHist2Slots) : 0;
@@ -726,14 +762,16 @@ __global__ void score3_count_kernel(const unsigned int* __restrict__ binmin, con
 }
 
 // ------------------------------------------------------------------ masked regression sums
+template <bool kRagged>
 __global__ void __launch_bounds__(256) masked_sums_kernel(const float* __restrict__ lap, const float* __restrict__ mean,
                                                           const float* __restrict__ var, size_t n,
                                                           const double* __restrict__ ths, double* __restrict__ sums,
-                                                          const int* __restrict__ active) {
+                                                          const int* __restrict__ active, const unsigned long long* seg_off) {
   if (active && !active[blockIdx.y]) return;  // second pass of the device-side estimator: only the segments that redo
-  lap += (size_t)blockIdx.y * n;
-  mean += (size_t)blockIdx.y * n;
-  var += (size_t)blockIdx.y * n;
+  const size_t seg0 = seg_begin<kRagged>(n, seg_off, blockIdx.y);
+  lap += seg0;
+  mean += seg0;
+  var += seg0;
   sums += (size_t)blockIdx.y * 12;
   const double th = ths[blockIdx.y];
   double s[12];
@@ -784,9 +822,18 @@ struct QuantList {
 };
 // np.percentile(method='linear'): virtual index (n-1)*q/100, bracketing order statistics, gamma (numpy _quantile).
 // ranks: [lo_0..lo_nq | hi_0..hi_nq] with entry nq = the 25th percentile of the empty-mask fallback (:82).
-__global__ void ranks_kernel(QuantList ql, unsigned long long n, unsigned long long* __restrict__ ranks, double* __restrict__ gamma) {
+// kRagged: block s fills row s (kMaxRanks ranks, kGammaRow weights) from the length of segment s.
+constexpr int kGammaRow = 2 * kMaxQ;
+template <bool kRagged>
+__global__ void ranks_kernel(QuantList ql, unsigned long long n, unsigned long long* __restrict__ ranks, double* __restrict__ gamma,
+                             const unsigned long long* seg_off) {
   const int i = threadIdx.x;
   if (i > ql.nq) return;
+  if (kRagged) {
+    n = seg_off[blockIdx.x + 1] - seg_off[blockIdx.x];
+    ranks += (size_t)blockIdx.x * kMaxRanks;
+    gamma += (size_t)blockIdx.x * kGammaRow;
+  }
   const double q = i < ql.nq ? ql.q[i] : 25.0;
   const double vi = __dmul_rn((double)(n - 1), __ddiv_rn(q, 100.0));
   const double lo = floor(vi);
@@ -802,10 +849,12 @@ __device__ __forceinline__ double np_lerp(float a, float b, double t) {
   if (t >= 0.5) return __dsub_rn((double)b, __dmul_rn(diff, __dsub_rn(1.0, t)));
   return __dadd_rn((double)a, __dmul_rn(diff, t));
 }
+template <bool kRagged>
 __global__ void pct_kernel(const float* __restrict__ stats, const double* __restrict__ gamma, int nq, double* __restrict__ ths,
                            double* __restrict__ th25) {
   const int s = blockIdx.x, i = threadIdx.x;
   if (i > nq) return;
+  if (kRagged) gamma += (size_t)s * kGammaRow;
   const float* st = stats + (size_t)s * (2 * (nq + 1));
   const double v = np_lerp(st[i], st[nq + 1 + i], gamma[i]);
   if (i < nq) ths[(size_t)s * nq + i] = v;
@@ -885,17 +934,17 @@ BoxSrc packed_src(const float* x, int h, int w) {
   return s;
 }
 
-template <bool SQ, int COLS, bool BAYER, bool NARROW>
+template <bool SQ, int COLS, bool BAYER, bool NARROW, bool RAGGED = false>
 int launch_box(dim3 g, cudaStream_t s, const BoxSrc& src, float4* o0, float4* o1, int B, int h, int w, int k, int op, int rows_per_strip,
-               const float4* ax, float4* o2) {
+               const float4* ax, float4* o2, const yond_frame_geom* frames = nullptr) {
   constexpr size_t bytes = (size_t)kRows * (SQ ? 8 : 4) * (COLS == 256 ? COLS : COLS + 33) * sizeof(double);  // = [kRows][NQ][PITCH]
   static std::once_flag once;
   static cudaError_t err = cudaSuccess;
   std::call_once(once, [] {
-    err = cudaFuncSetAttribute(box_fused_kernel<SQ, COLS, BAYER, NARROW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    err = cudaFuncSetAttribute(box_fused_kernel<SQ, COLS, BAYER, NARROW, RAGGED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
   });
   if (err != cudaSuccess) return yond_set_error(YOND_ERR_CUDA, "box filter: cudaFuncSetAttribute failed: %s", cudaGetErrorString(err));
-  box_fused_kernel<SQ, COLS, BAYER, NARROW><<<g, kBoxThreads, bytes, s>>>(src, o0, o1, B, h, w, k, op, rows_per_strip, ax, o2);
+  box_fused_kernel<SQ, COLS, BAYER, NARROW, RAGGED><<<g, kBoxThreads, bytes, s>>>(src, o0, o1, B, h, w, k, op, rows_per_strip, ax, o2, frames);
   return YOND_OK;
 }
 
@@ -935,6 +984,21 @@ int box_pass(const BoxSrc& src, bool bayer, float* out0, float* out1, int B, int
   }
 #undef YOND_BOX_B
 #undef YOND_BOX
+  if (rc) return rc;
+  YOND_LAUNCH_CHECK();
+  return YOND_OK;
+}
+
+// One box pass over `nframes` frames of different sizes (wide layout, one frame per blockIdx.z): a Bayer source comes from the records, a
+// packed one is `src.base` plus each record's offset; the outputs are the concatenated maps.
+template <bool SQ, bool BAYER>
+int box_pass_frames(const BoxSrc& src, float* out0, float* out1, const yond_frame_geom* frames, int nframes, int max_h, int max_w, int k,
+                    int op, cudaStream_t s) {
+  const int r = k / 2, rows_per_strip = 64;
+  const dim3 g(ceil_div(max_w, 256 - 2 * r), ceil_div(max_h, rows_per_strip), nframes);
+  YOND_REQUIRE(g.z <= 65535, "box filter: at most 65535 frames per call");
+  const int rc = launch_box<SQ, 256, BAYER, false, true>(g, s, src, reinterpret_cast<float4*>(out0), reinterpret_cast<float4*>(out1),
+                                                         nframes, max_h, max_w, k, op, rows_per_strip, nullptr, nullptr, frames);
   if (rc) return rc;
   YOND_LAUNCH_CHECK();
   return YOND_OK;
@@ -1094,12 +1158,37 @@ int yond_nlf_maps_collab_cached(const float* y, int y_mosaic, const float* lr_va
   return collab_from_lr_var(bayer_src(y, y_mosaic, nblk, H, W, split_blocks), true, lr_var, var, mean, lap, B, h, w, k, s);
 }
 
+// SelfNLF's maps of frames of different sizes: the three box passes of nlf_maps_impl mode 0, one launch each for all frames.
+int yond_nlf_maps_frames(const yond_frame_geom* frames_dev, int nframes, int max_H, int max_W, float* var, float* mean, float* lap, int k,
+                         void* work, void* stream) {
+  YOND_REQUIRE(frames_dev && var && mean && lap && work, "yond_nlf_maps_frames: null argument");
+  YOND_REQUIRE(nframes > 0 && nframes <= 65535, "yond_nlf_maps_frames: 1..65535 frames");
+  YOND_REQUIRE(k % 2 == 1 && k >= 3 && k <= kMaxK, "yond_nlf_maps_frames: odd k <= %d required (got %d)", kMaxK, k);
+  YOND_REQUIRE(max_H > 0 && max_W > 0 && max_H % 2 == 0 && max_W % 2 == 0, "yond_nlf_maps_frames: H,W must be even");
+  YOND_REQUIRE((uintptr_t)work % 16 == 0, "yond_nlf_maps_frames: work must be 16-byte aligned");
+  cudaStream_t s = (cudaStream_t)stream;
+  const int h = max_H / 2, w = max_W / 2, k2 = k / 3 * 2 + 1;
+  float* tmp = reinterpret_cast<float*>(work);
+  BoxSrc bayer{};  // base, strides and row length come from the records
+  bayer.imgs_per_seg = 1;
+  BoxSrc packed = bayer;
+  packed.base = tmp;
+  YondProfScope prof("nlf_maps_frames (3 box_fused passes)", s, 0.0);  // no byte count: the frame sizes are in device memory
+  int rc;
+  // mean = blur_k(x), var = std_k(x)^2 ; blur_k2(x) -> tmp ; lap = std_k(blur_k2(x))  (YOND_SIDD.py:66-71)
+  if ((rc = box_pass_frames<true, true>(bayer, mean, var, frames_dev, nframes, h, w, k, OP_MEAN_VAR, s))) return rc;
+  if ((rc = box_pass_frames<false, true>(bayer, tmp, nullptr, frames_dev, nframes, h, w, k2, OP_MEAN, s))) return rc;
+  return box_pass_frames<true, false>(packed, lap, nullptr, frames_dev, nframes, h, w, k, OP_STD, s);
+}
+
 }  // extern "C"
 
 namespace {
-// data = lap; the first counting pass also collects the per-bin minimum of lap over the `mean` bins (score3) into `binmin`
+// data = lap; the first counting pass also collects the per-bin minimum of lap over the `mean` bins (score3) into `binmin`.
+// RAGGED: segment s is [seg_off[s], seg_off[s+1]) and seg_len the longest one (it sizes the grids).
+template <bool RAGGED>
 int order_stats_impl(const float* data, const float* mean, unsigned int* binmin, size_t seg_len, int nseg, const uint64_t* ranks_dev,
-                     int nranks, float* out_dev, void* work, cudaStream_t s) {
+                     int nranks, float* out_dev, void* work, cudaStream_t s, const unsigned long long* seg_off) {
   SelectWork* wk = reinterpret_cast<SelectWork*>(work);
   // one memset for all segments (the slot tables behind the histograms are rewritten by the select kernels anyway)
   YOND_CUDA_CHECK(cudaMemsetAsync(wk, 0, (size_t)nseg * sizeof(SelectWork), s));
@@ -1109,17 +1198,17 @@ int order_stats_impl(const float* data, const float* mean, unsigned int* binmin,
   YOND_CUDA_CHECK(cudaMemsetAsync(binmin, 0xff, (size_t)nseg * 1024 * sizeof(unsigned int), s));
   {
     YondProfScope prof("hist0+score3_binmin", s, 8.0 * nel);
-    hist0_kernel<true><<<g, 256, 0, s>>>(data, mean, seg_len, wk, binmin);
+    hist0_kernel<true, RAGGED><<<g, 256, 0, s>>>(data, mean, seg_len, wk, binmin, seg_off);
   }
   YOND_LAUNCH_CHECK();
-  select0_kernel<<<nseg, 1024, 0, s>>>(wk, reinterpret_cast<const unsigned long long*>(ranks_dev), nranks);
+  select0_kernel<RAGGED><<<nseg, 1024, 0, s>>>(wk, reinterpret_cast<const unsigned long long*>(ranks_dev), nranks);
   YOND_LAUNCH_CHECK();
   {
     static std::once_flag once;
     static cudaError_t attr_err = cudaSuccess;
     const size_t smem = (size_t)kHist1Slots * 2048 * sizeof(unsigned int) + 2048;
     std::call_once(once, [&] {
-      attr_err = cudaFuncSetAttribute(hist1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+      attr_err = cudaFuncSetAttribute(hist1_kernel<RAGGED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       if (attr_err == cudaSuccess)
         attr_err = cudaFuncSetAttribute(select1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 16 * (2048 + 32) * (int)sizeof(unsigned int));
     });
@@ -1129,7 +1218,7 @@ int order_stats_impl(const float* data, const float* mean, unsigned int* binmin,
     const size_t need = (seg_len / 4 + kHist1Threads - 1) / kHist1Threads;
     if ((size_t)bx > need) bx = (int)need;
     YondProfScope prof("hist1", s, 4.0 * nel);
-    hist1_kernel<<<dim3(bx, nseg), kHist1Threads, smem, s>>>(data, seg_len, wk);
+    hist1_kernel<RAGGED><<<dim3(bx, nseg), kHist1Threads, smem, s>>>(data, seg_len, wk, seg_off);
     YOND_LAUNCH_CHECK();
   }
   select1_kernel<<<nseg, 1024, 16 * (2048 + 32) * sizeof(unsigned int), s>>>(wk, nranks);
@@ -1138,11 +1227,11 @@ int order_stats_impl(const float* data, const float* mean, unsigned int* binmin,
     YondProfScope prof("hist2", s, 4.0 * nel);
     static std::once_flag h2_once;
     static cudaError_t h2_err = cudaSuccess;
-    std::call_once(h2_once, [] { h2_err = cudaFuncSetAttribute(hist2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHist2Slots * 1024 * 4); });
+    std::call_once(h2_once, [] { h2_err = cudaFuncSetAttribute(hist2_kernel<true, RAGGED>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHist2Slots * 1024 * 4); });
     if (h2_err != cudaSuccess) return yond_set_error(YOND_ERR_CUDA, "cudaFuncSetAttribute(hist2_kernel) failed: %s", cudaGetErrorString(h2_err));
-    hist2_kernel<false><<<g, 256, 0, s>>>(data, seg_len, wk);
+    hist2_kernel<false, RAGGED><<<g, 256, 0, s>>>(data, seg_len, wk, seg_off);
     YOND_LAUNCH_CHECK();
-    hist2_kernel<true><<<g, 256, kHist2Slots * 1024 * sizeof(unsigned int), s>>>(data, seg_len, wk);
+    hist2_kernel<true, RAGGED><<<g, 256, kHist2Slots * 1024 * sizeof(unsigned int), s>>>(data, seg_len, wk, seg_off);
   }
   YOND_LAUNCH_CHECK();
   select2_kernel<<<nseg, 1024, 0, s>>>(wk, nranks, out_dev);
@@ -1150,16 +1239,21 @@ int order_stats_impl(const float* data, const float* mean, unsigned int* binmin,
   return YOND_OK;
 }
 
-// sums_dev[s][0..5] = {N, Sx, Sy, Sxx, Sxy, Syy} over {lap < ths_dev[s]} (YOND_SIDD.py:77-78, strict), [6..11] the same over
-// {lap < th, 1e-4 < mean < 0.8} (polyfit's non-saturated subset, utils/isp_algos.py:348-350), float64
-int masked_sums(const float* lap, const float* mean, const float* var, size_t seg_len, int nseg, const double* ths_dev, double* sums_dev,
-                cudaStream_t s) {
-  YOND_CUDA_CHECK(cudaMemsetAsync(sums_dev, 0, (size_t)nseg * 12 * sizeof(double), s));
+inline dim3 sums_grid(size_t seg_len, int nseg) {
   dim3 g(stream_grid(seg_len), nseg);
   if ((size_t)g.x * nseg > (size_t)yond_num_sms() * 16) g.x = (unsigned)((yond_num_sms() * 16 + nseg - 1) / nseg);
+  return g;
+}
+
+// sums_dev[s][0..5] = {N, Sx, Sy, Sxx, Sxy, Syy} over {lap < ths_dev[s]} (YOND_SIDD.py:77-78, strict), [6..11] the same over
+// {lap < th, 1e-4 < mean < 0.8} (polyfit's non-saturated subset, utils/isp_algos.py:348-350), float64
+template <bool RAGGED>
+int masked_sums(const float* lap, const float* mean, const float* var, size_t seg_len, int nseg, const double* ths_dev, double* sums_dev,
+                cudaStream_t s, const unsigned long long* seg_off) {
+  YOND_CUDA_CHECK(cudaMemsetAsync(sums_dev, 0, (size_t)nseg * 12 * sizeof(double), s));
   {
     YondProfScope prof("masked_sums", s, 12.0 * (double)seg_len * nseg);
-    masked_sums_kernel<<<g, 256, 0, s>>>(lap, mean, var, seg_len, ths_dev, sums_dev, nullptr);
+    masked_sums_kernel<RAGGED><<<sums_grid(seg_len, nseg), 256, 0, s>>>(lap, mean, var, seg_len, ths_dev, sums_dev, nullptr, seg_off);
   }
   YOND_LAUNCH_CHECK();
   return YOND_OK;
@@ -1185,8 +1279,8 @@ FitWork carve_fit(void* base, int nseg) {
     return r;
   };
   w.sel = (SelectWork*)take((size_t)nseg * sizeof(SelectWork));
-  w.ranks = (unsigned long long*)take(kMaxRanks * 8);
-  w.gamma = (double*)take(kMaxQ * 2 * 8);
+  w.ranks = (unsigned long long*)take((size_t)nseg * kMaxRanks * 8);  // one row per segment (segments of different lengths)
+  w.gamma = (double*)take((size_t)nseg * kGammaRow * 8);
   w.ths = (double*)take((size_t)nseg * kMaxQ * 8);
   w.th25 = (double*)take((size_t)nseg * 8);
   w.th = (double*)take((size_t)nseg * 8);
@@ -1201,11 +1295,56 @@ FitWork carve_fit(void* base, int nseg) {
   w.bytes = align_up(off, 256);
   return w;
 }
+
+// yond_nlf_fit (RAGGED = false: nseg segments of seg_len) and yond_nlf_fit_ragged (segments from seg_off, seg_len = the longest)
+template <bool RAGGED>
+int nlf_fit_impl(const float* var, const float* mean, const float* lap, const unsigned long long* seg_off, size_t seg_len, int nseg,
+                 const double* quants_host, int nq, double* regs_dev, double* detail_dev, void* work, cudaStream_t s) {
+  const FitWork w = carve_fit(work, nseg);
+  QuantList ql{};
+  ql.nq = nq;
+  for (int i = 0; i < nq; ++i) ql.q[i] = quants_host[i];
+  for (int i = 1; i < nq; ++i) YOND_REQUIRE(ql.q[i] > ql.q[i - 1], "yond_nlf_fit: quantiles must ascend");
+  const int nranks = 2 * (nq + 1);
+  ranks_kernel<RAGGED><<<RAGGED ? nseg : 1, 32, 0, s>>>(ql, (unsigned long long)seg_len, w.ranks, w.gamma, seg_off);
+  YOND_LAUNCH_CHECK();
+  YOND_REQUIRE(seg_len < 0xffffffffull && seg_len % 4 == 0 && (uintptr_t)lap % 16 == 0 && (uintptr_t)mean % 16 == 0,
+               "yond_nlf_fit: segments must hold whole 4-channel pixels (16-byte aligned), fewer than 2^32 elements");
+  unsigned int* binmin = reinterpret_cast<unsigned int*>(w.minj);
+  // the first counting pass of the radix select also collects the per-bin minimum of lap (all score3 needs from the maps)
+  int rc = order_stats_impl<RAGGED>(lap, mean, binmin, seg_len, nseg, reinterpret_cast<const uint64_t*>(w.ranks), nranks, w.stats, w.sel, s,
+                                    seg_off);
+  if (rc) return rc;
+  pct_kernel<RAGGED><<<nseg, 32, 0, s>>>(w.stats, w.gamma, nq, w.ths, w.th25);
+  YOND_LAUNCH_CHECK();
+  score3_count_kernel<<<nseg, 256, 0, s>>>(binmin, w.ths, nq, w.npeaks);
+  YOND_LAUNCH_CHECK();
+  pick_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(ql, w.ths, w.npeaks, w.th, w.idx, nseg);
+  YOND_LAUNCH_CHECK();
+  if ((rc = masked_sums<RAGGED>(lap, mean, var, seg_len, nseg, w.th, w.sums, s, seg_off))) return rc;
+  backup_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(w.sums, w.th, w.th25, w.th2, w.redo, w.sums2, nseg);
+  YOND_LAUNCH_CHECK();
+  // second pass: only the segments whose mask came out empty do any work
+  masked_sums_kernel<RAGGED><<<sums_grid(seg_len, nseg), 256, 0, s>>>(lap, mean, var, seg_len, w.th2, w.sums2, w.redo, seg_off);
+  YOND_LAUNCH_CHECK();
+  solve_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(w.sums, w.sums2, w.redo, w.th2, w.idx, w.ths, w.npeaks, ql, regs_dev, detail_dev, nseg);
+  YOND_LAUNCH_CHECK();
+  return YOND_OK;
+}
+
+// seg_max[s] = max(x, 0) over segment s (the max of the bits of non-negative floats is their float maximum)
+__global__ void __launch_bounds__(256) seg_max_kernel(const float* __restrict__ x, size_t n, float* __restrict__ seg_max) {
+  float m = 0.f;
+  stream_f4(reinterpret_cast<const float4*>(x + (size_t)blockIdx.y * n), n / 4, [&](float e) { m = fmaxf(m, e); });
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(reinterpret_cast<int*>(seg_max + blockIdx.y), __float_as_int(m));
+}
 }  // namespace
 
 extern "C" {
 
 size_t yond_nlf_fit_work_bytes(int nseg) { return carve_fit(nullptr, nseg < 1 ? 1 : nseg).bytes + 256; }
+size_t yond_nlf_fit_ragged_work_bytes(int nseg) { return carve_fit(nullptr, nseg < 1 ? 1 : nseg).bytes + 256; }
 
 int yond_nlf_fit(const float* var, const float* mean, const float* lap, size_t seg_len, int nseg, const double* quants_host,
                  int nq, double* regs_dev, double* detail_dev, void* work, void* stream) {
@@ -1213,37 +1352,27 @@ int yond_nlf_fit(const float* var, const float* mean, const float* lap, size_t s
   YOND_REQUIRE(nq >= 1 && nq <= kMaxQ && 2 * (nq + 1) <= kMaxRanks, "yond_nlf_fit: 1..%d quantiles (got %d)", kMaxQ, nq);
   YOND_REQUIRE(seg_len > 0 && nseg > 0 && nseg <= 65535, "yond_nlf_fit: bad segment geometry");
   YOND_REQUIRE((uintptr_t)work % 256 == 0, "yond_nlf_fit: work must be 256-byte aligned");
+  return nlf_fit_impl<false>(var, mean, lap, nullptr, seg_len, nseg, quants_host, nq, regs_dev, detail_dev, work, (cudaStream_t)stream);
+}
+
+int yond_nlf_fit_ragged(const float* var, const float* mean, const float* lap, const unsigned long long* seg_off_dev,
+                        size_t max_seg_len, int nseg, const double* quants_host, int nq, double* regs_dev, double* detail_dev,
+                        void* work, void* stream) {
+  YOND_REQUIRE(var && mean && lap && seg_off_dev && regs_dev && work && quants_host, "yond_nlf_fit_ragged: null argument");
+  YOND_REQUIRE(nq >= 1 && nq <= kMaxQ && 2 * (nq + 1) <= kMaxRanks, "yond_nlf_fit_ragged: 1..%d quantiles (got %d)", kMaxQ, nq);
+  YOND_REQUIRE(max_seg_len > 0 && nseg > 0 && nseg <= 65535, "yond_nlf_fit_ragged: bad segment geometry");
+  YOND_REQUIRE((uintptr_t)work % 256 == 0, "yond_nlf_fit_ragged: work must be 256-byte aligned");
+  return nlf_fit_impl<true>(var, mean, lap, seg_off_dev, max_seg_len, nseg, quants_host, nq, regs_dev, detail_dev, work,
+                            (cudaStream_t)stream);
+}
+
+int yond_seg_max(const float* x, size_t seg_len, int nseg, float* seg_max, void* stream) {
+  YOND_REQUIRE(x && seg_max, "yond_seg_max: null argument");
+  YOND_REQUIRE(seg_len > 0 && seg_len % 4 == 0 && (uintptr_t)x % 16 == 0 && nseg > 0 && nseg <= 65535,
+               "yond_seg_max: 1..65535 segments of whole float4s, 16-byte aligned");
   cudaStream_t s = (cudaStream_t)stream;
-  const FitWork w = carve_fit(work, nseg);
-  QuantList ql{};
-  ql.nq = nq;
-  for (int i = 0; i < nq; ++i) ql.q[i] = quants_host[i];
-  for (int i = 1; i < nq; ++i) YOND_REQUIRE(ql.q[i] > ql.q[i - 1], "yond_nlf_fit: quantiles must ascend");
-  const int nranks = 2 * (nq + 1);
-  ranks_kernel<<<1, 32, 0, s>>>(ql, (unsigned long long)seg_len, w.ranks, w.gamma);
-  YOND_LAUNCH_CHECK();
-  YOND_REQUIRE(seg_len < 0xffffffffull && seg_len % 4 == 0 && (uintptr_t)lap % 16 == 0 && (uintptr_t)mean % 16 == 0,
-               "yond_nlf_fit: segments must hold whole 4-channel pixels (16-byte aligned), fewer than 2^32 elements");
-  unsigned int* binmin = reinterpret_cast<unsigned int*>(w.minj);
-  // the first counting pass of the radix select also collects the per-bin minimum of lap (all score3 needs from the maps)
-  int rc = order_stats_impl(lap, mean, binmin, seg_len, nseg, reinterpret_cast<const uint64_t*>(w.ranks), nranks, w.stats, w.sel, s);
-  if (rc) return rc;
-  pct_kernel<<<nseg, 32, 0, s>>>(w.stats, w.gamma, nq, w.ths, w.th25);
-  YOND_LAUNCH_CHECK();
-  score3_count_kernel<<<nseg, 256, 0, s>>>(binmin, w.ths, nq, w.npeaks);
-  YOND_LAUNCH_CHECK();
-  pick_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(ql, w.ths, w.npeaks, w.th, w.idx, nseg);
-  YOND_LAUNCH_CHECK();
-  if ((rc = masked_sums(lap, mean, var, seg_len, nseg, w.th, w.sums, s))) return rc;
-  backup_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(w.sums, w.th, w.th25, w.th2, w.redo, w.sums2, nseg);
-  YOND_LAUNCH_CHECK();
-  {  // second pass: only the segments whose mask came out empty do any work
-    dim3 g(stream_grid(seg_len), nseg);
-    if ((size_t)g.x * nseg > (size_t)yond_num_sms() * 16) g.x = (unsigned)((yond_num_sms() * 16 + nseg - 1) / nseg);
-    masked_sums_kernel<<<g, 256, 0, s>>>(lap, mean, var, seg_len, w.th2, w.sums2, w.redo);
-    YOND_LAUNCH_CHECK();
-  }
-  solve_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(w.sums, w.sums2, w.redo, w.th2, w.idx, w.ths, w.npeaks, ql, regs_dev, detail_dev, nseg);
+  YOND_CUDA_CHECK(cudaMemsetAsync(seg_max, 0, sizeof(float) * nseg, s));
+  seg_max_kernel<<<sums_grid(seg_len, nseg), 256, 0, s>>>(x, seg_len, seg_max);
   YOND_LAUNCH_CHECK();
   return YOND_OK;
 }

@@ -16,6 +16,41 @@ from . import _lib
 from ._lib import check, ptr, stream_ptr
 from .isp import _as_batch4, _dev, to_dev
 
+FRAME_GEOM = np.dtype([("base", "<u8"), ("H", "<i4"), ("W", "<i4"), ("off", "<i8")])  # yond_frame_geom
+assert FRAME_GEOM.itemsize == 24
+
+
+def check_frames(frames, nimg=None, k=29):
+    """Bayer frames of any even sizes as a list of (H, W) CUDA float32 tensors: a sequence of them, one (n, H, W) tensor or one (H, W)
+    frame.  Raises ValueError for a count other than `nimg` (when given), a frame that is not a contiguous 2-D CUDA float32 tensor, an
+    odd H or W, or a packed size (H/2, W/2) not larger than the filter radius k // 2 (the box filters reflect once at the border)."""
+    if isinstance(frames, torch.Tensor):
+        if frames.dim() not in (2, 3):
+            raise ValueError(f"frames: one (n, H, W) tensor or (H, W) frame expected, got shape {tuple(frames.shape)}")
+        frames = [frames] if frames.dim() == 2 else list(frames.unbind(0))
+    else:
+        try:
+            frames = list(frames)
+        except TypeError:
+            raise ValueError(f"frames: a sequence of (H, W) tensors or one (n, H, W) tensor expected, got {type(frames).__name__}") from None
+    if not frames or (nimg is not None and len(frames) != nimg):
+        raise ValueError(f"frames: {nimg if nimg is not None else 'at least one'} frame(s) expected, got {len(frames)}")
+    for i, f in enumerate(frames):
+        if not isinstance(f, torch.Tensor) or f.dim() != 2:
+            raise ValueError(f"frame {i}: a 2-D (H, W) tensor expected, got {getattr(f, 'shape', type(f).__name__)}")
+        H, W = f.shape
+        if H % 2 or W % 2:
+            raise ValueError(f"frame {i}: H and W must be even (Bayer 2x2 cells), got {H}x{W}")
+        if min(H, W) // 2 <= k // 2:
+            raise ValueError(f"frame {i}: packed size {H // 2}x{W // 2} must exceed the filter radius {k // 2}")
+        if f.dtype != torch.float32:
+            raise ValueError(f"frame {i}: float32 expected, got {f.dtype}")
+        if not f.is_contiguous():
+            raise ValueError(f"frame {i}: a contiguous tensor expected")
+        if not f.is_cuda:
+            raise ValueError(f"frame {i}: a CUDA tensor expected, got one on {f.device}")
+    return frames
+
 
 class NlfEstimator:
     """Blind (beta1, beta2) estimation, batched over `nimg` images: every device stage runs once for the whole batch
@@ -89,17 +124,59 @@ class NlfEstimator:
                                           H, W, int(bool(split_blocks)), int(k), mode, ptr(seg_max), ptr(work), stream_ptr()))
         return self._fit(var, mean, lap, nimg, details, step)
 
-    def _fit(self, var, mean, lap, nimg, details=False, step=5):
+    def _fit(self, var, mean, lap, nimg, details=False, step=5, segments=None):
+        """segments (optional): (seg_off, max_len), the device offsets (nimg + 1 uint64) of segments of different lengths and the
+        longest length; else the maps are nimg segments of equal length."""
         lib, dev = self.lib, var.device
         n_el = var.numel()
         quants = np.ascontiguousarray(np.linspace(step, 100, 100 // step, endpoint=True), np.float64)
         regs = torch.empty((nimg, 2), device=dev, dtype=torch.float64)
         detail = torch.empty((nimg, self.DETAIL), device=dev, dtype=torch.float64) if details else None
-        fwork = self._buf("fit", lib.yond_nlf_fit_work_bytes(nimg) + 256, dev)
-        off = (-fwork.data_ptr()) % 256
-        check(lib.yond_nlf_fit(ptr(var), ptr(mean), ptr(lap), n_el // nimg, nimg, quants.ctypes.data_as(C.POINTER(C.c_double)),
-                               len(quants), ptr(regs), ptr(detail), ptr(fwork[off:]), stream_ptr()))
+        qp = quants.ctypes.data_as(C.POINTER(C.c_double))
+        if segments is None:
+            fwork = self._buf("fit", lib.yond_nlf_fit_work_bytes(nimg) + 256, dev)
+            off = (-fwork.data_ptr()) % 256
+            check(lib.yond_nlf_fit(ptr(var), ptr(mean), ptr(lap), n_el // nimg, nimg, qp, len(quants), ptr(regs), ptr(detail),
+                                   ptr(fwork[off:]), stream_ptr()))
+        else:
+            seg_off, max_len = segments
+            fwork = self._buf("fit", lib.yond_nlf_fit_ragged_work_bytes(nimg) + 256, dev)
+            off = (-fwork.data_ptr()) % 256
+            check(lib.yond_nlf_fit_ragged(ptr(var), ptr(mean), ptr(lap), ptr(seg_off), int(max_len), nimg, qp, len(quants), ptr(regs),
+                                          ptr(detail), ptr(fwork[off:]), stream_ptr()))
         return (regs, detail) if details else regs
+
+    # -- the self estimate of frames of different sizes (round 1 of IterDenoise on the full-resolution frames) ----------------
+    def maps_frames(self, frames, k=29):
+        """SelfNLF maps of a list of (H, W) CUDA float32 Bayer frames of any even sizes (check_frames), every box pass one launch for
+        all of them.  Returns var, mean, lap: flat float32 maps, frame i's packed (H/2, W/2, 4) maps at float offsets
+        off[i]:off[i + 1] (off: the host array of the nframes + 1 offsets), then off and the device copy of the offsets (uint64)."""
+        from .pipeline import _upload
+        frames = check_frames(frames, None, k)
+        lib, dev = self.lib, frames[0].device
+        off = np.concatenate([[0], np.cumsum([f.numel() for f in frames])]).astype(np.uint64)
+        geom = np.zeros(len(frames), FRAME_GEOM)
+        geom["base"] = [f.data_ptr() for f in frames]
+        geom["H"] = [f.shape[0] for f in frames]
+        geom["W"] = [f.shape[1] for f in frames]
+        geom["off"] = off[:-1].astype(np.int64)
+        buf, offs = _upload([geom, off], dev)  # the records and the fit's segment offsets: one copy from pinned memory
+        n_el = int(off[-1])
+        maps = self._buf("maps3", 3 * n_el * 4, dev).view(torch.float32)
+        var, mean, lap = maps[:n_el], maps[n_el:2 * n_el], maps[2 * n_el:3 * n_el]
+        work = self._buf("maps", n_el * 4, dev)
+        check(lib.yond_nlf_maps_frames(ptr(buf), len(frames), int(geom["H"].max()), int(geom["W"].max()), ptr(var), ptr(mean), ptr(lap),
+                                       int(k), ptr(work), stream_ptr()))
+        return var, mean, lap, off, buf[offs[1]:offs[1] + off.nbytes].view(torch.int64)
+
+    def estimate_frames(self, frames, k=29, details=False, step=5):
+        """Batched SelfNLF (SimpleNLF 'self') of a list of (H, W) CUDA float32 Bayer frames of any even sizes, or one (n, H, W) tensor:
+        regs (nframes, 2) float64 on the device [, detail (nframes, DETAIL)], nothing read back.  The maps of all frames take one launch
+        per box pass and the fit one set of launches.  A frame wider than 160 - 2*(k//2) packed pixels (every full-resolution frame) gets
+        the same bits as estimate_dev on it alone; a narrower one takes the wide box-filter layout too and may differ from estimate_dev,
+        which packs such frames side by side, in the float64 rounding of the window sums."""
+        var, mean, lap, off, seg_off = self.maps_frames(frames, k)
+        return self._fit(var, mean, lap, len(off) - 1, details, step, segments=(seg_off, int(np.diff(off).max())))
 
     # -- the collab rounds of IterDenoise from cached noisy-frame statistics ---------------------------
     # Every collab round r >= 2 estimates on (lr, out_{r-1}) in the same geometry.  Its var map is stdfilt(lr, k)**2 -

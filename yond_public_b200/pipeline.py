@@ -544,11 +544,19 @@ class YOND_SIDD:
 
         Exposure per image: p['wp'], p['bl'], p['scale'] and each entry of raw are a scalar (every image) or one value per image
         (batch_exposure; ValueError before anything is launched), so a batch may mix white / black levels and ratios.  They reach the
-        device in one small copy; scalars take the same path."""
+        device in one small copy; scalars take the same path.
+
+        lr_full: the full-resolution noisy frame of every image (the shipped SIDD configuration estimates round 1 on it, :338-341) —
+        a sequence of nimg (H_i, W_i) CUDA float32 frames, of any even sizes, or one (nimg, H, W) tensor.  Round 1 is then one
+        estimate_frames call for the whole batch; the fallback bias-table bound stays the maximum of each image's blocks (:393), and
+        the collab rounds estimate on the blocks as without lr_full (:431).  ValueError before anything is launched for a wrong number
+        of frames, a malformed frame (nlf.check_frames) or lr_full together with raw, which is not supported."""
         pipe = self.pipe
         n_collab = collab_rounds(pipe)
+        if lr_full is not None and raw is not None:
+            raise ValueError("lr_full takes float32 frames and is not supported together with raw= (uint16 sensor input)")
         if raw is not None:
-            assert x.dtype in (torch.int16, torch.uint16) and lr_full is None
+            assert x.dtype in (torch.int16, torch.uint16)
         assert pipe["full_est"] and "simple" in pipe["est_type"]
         nimg, nblk, H, W = x.shape
         dev = x.device
@@ -556,6 +564,8 @@ class YOND_SIDD:
         k, bias_corr, vst_type = pipe["k"], pipe["bias_corr"], pipe.get("vst_type", "exact")
         full_dn = bool(pipe["full_dn"])
         scale_est, scale, raw_rec = batch_exposure(p, nimg, raw)
+        if lr_full is not None:
+            lr_full = nlf.check_frames(lr_full, nimg, k)
         # (scale_est, scale, bound) per image for round 1 and for the collab rounds.  The bound of a fallback bias table: full_dn
         # round 1 = the frame's max in DN of p['scale'] (:256); everything else lr_raw.max()*(wp-bl) (:393, :449)
         scales1 = np.stack([scale_est, scale, scale if full_dn else scale_est], 1)
@@ -602,10 +612,9 @@ class YOND_SIDD:
         if lr_full is None:
             regs = est.estimate_dev(x, None, k, split_blocks=False, seg_max=seg_max, raw=raw, var_map=lr_var if reuse else None)
         else:
-            assert nimg == 1
-            regs = est.estimate_dev(lr_full.reshape(1, 1, *lr_full.shape[-2:]), None, k)
-            if need_max:
-                seg_max = x.amax().clamp_min(0).reshape(1)
+            regs = est.estimate_frames(lr_full, k)
+            if need_max:  # the bound is the maximum of the image's blocks, not of its full frame (:393)
+                check(eng.lib.yond_seg_max(ptr(x), x[0].numel(), nimg, ptr(seg_max), stream_ptr()))
         mark("estimate_self")
         ch = eng.chain_params(regs, seg_max, nimg, nblk, *scales1.T, 1, bias_corr, vst_type, scales_dev=s1_dev)
         frames = x.reshape(nimg * nblk, H, W)
@@ -671,14 +680,15 @@ class YOND_SIDD:
             rounds += live[r]
         return regs, rounds, gains
 
-    def iter_denoise_batch(self, blocks, p, log=None, timings=None, raw=None):
+    def iter_denoise_batch(self, blocks, p, log=None, timings=None, raw=None, lr_full=None):
         """IterDenoise for a BATCH of SIDD-shaped images (or full frames, nblk = 1) at once: blocks (nimg, nblk, H, W) CUDA
         f32.  Same per-image algorithm and guards as the reference (YOND_SIDD.py:301-483); every device stage runs once for
         all images and the host reads back ONE small array at the end.
         Returns {'raw_dns': [(nimg,H,nblk*W) per round, max_iter + 1 of them], 'regs': [(nimg,2) per round; NaN rows in the
         rounds an image did not complete (a beta1 < 0 guard kept its previous result)], 'rounds': (nimg,) number of denoise rounds
-        each image completed}.  An image's entries of raw_dns beyond its rounds repeat its last completed round."""
-        res = self.iter_denoise_dev(blocks, p, timings=timings, raw=raw)
+        each image completed}.  An image's entries of raw_dns beyond its rounds repeat its last completed round.
+        lr_full (optional): the full-resolution frame of every image, sizes may differ (iter_denoise_dev): round 1 estimates on them."""
+        res = self.iter_denoise_dev(blocks, p, timings=timings, raw=raw, lr_full=lr_full)
         regs, rounds, _ = self.read_summary(res)
         return {"raw_dns": list(res["dns"]), "regs": regs, "rounds": rounds, "lr_raw": None, "dev": res}
 
@@ -769,7 +779,7 @@ class YOND_SIDD:
             return {"raw_dns": [dn], "regs": (0, 0), "lr_raw": mosaic}
         if "simple" not in pipe["est_type"]:
             raise NotImplementedError(f"est_type '{pipe['est_type']}' needs external estimate files / networks (YOND_SIDD.py:316-353)")
-        res = self.iter_denoise_dev(blk[None].contiguous(), p, lr_full=lr_full, after_round1=after_round1)
+        res = self.iter_denoise_dev(blk[None].contiguous(), p, lr_full=None if lr_full is None else [lr_full], after_round1=after_round1)
         if before_summary is not None:  # everything is enqueued; host work placed here overlaps the collab rounds
             before_summary()
         r4, live = self.host_numbers(res)
