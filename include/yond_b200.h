@@ -243,6 +243,32 @@ int yond_nlf_fit_ragged(const float* var, const float* mean, const float* lap, c
                         void* work, void* stream);
 int yond_seg_max(const float* x, size_t seg_len, int nseg, float* seg_max, void* stream);
 
+/* ---- IterDenoise over full frames of different sizes in one batch — YOND_SIDD.py:301-483 with the frame as the image (round 1
+ * :315/:338-341 self estimate, :356 + :252-269 VST constants, :419-472 collab rounds on (lr, previous output), :445-447 selection).
+ * Every record table below is in DEVICE memory, and the caller keeps every frame it points to alive and unchanged until the work
+ * is done.  A float32 frame must be 8-byte aligned (64-bit Bayer loads), a uint16 mosaic 4-byte aligned; these are not checked here.
+ * yond_nlf_maps_frames_max: yond_nlf_maps_frames plus `seg_max` (optional, nframes floats): max(x, 0) per frame from the first box
+ *   pass — the bound of the fallback bias table (:256, isp_algos.py:101).
+ * yond_nlf_maps_frames_raw16: the same self maps (and seg_max) with every record's `base` holding the address of a uint16 (H, W)
+ *   sensor mosaic, not a float32 frame: frame i is normalised on load with nrm_dev[i] (a DEVICE array of nframes entries), the same
+ *   float32 arithmetic as yond_nlf_maps_raw16_per_image (data_process/yond_datasets.py:955-961, :1053-1056).
+ * yond_nlf_maps_frames_collab_cached: the collab maps (yond_nlf_maps_collab_cached, :89-98 with stdfilt(lr, k)**2 cached) of every
+ *   frame in one launch: frame i of the round's output is the float32 Bayer frame at y + off_i (the flat layout of the maps, so a
+ *   round's outputs concatenated in record order), lr_var the var maps of the self estimate of the same records.  The records'
+ *   `base` is not read.  y and lr_var 16-byte aligned.
+ * yond_vst_fwd_frames: yond_vst_fwd (nrm_dev NULL, float32 frames) or yond_vst_fwd_raw16 (nrm_dev set: uint16 mosaics, frame b
+ *   normalised with nrm_dev[b]) over B records that all hold (H, W) frames: frame b is read from frames_dev[b].base, wherever it
+ *   lies.  z, ub, params_dev and the padding as in yond_vst_fwd. */
+int yond_nlf_maps_frames_max(const yond_frame_geom* frames_dev, int nframes, int max_H, int max_W, float* var, float* mean, float* lap,
+                             int k, void* work, void* stream, float* seg_max);
+int yond_nlf_maps_frames_raw16(const yond_frame_geom* frames_dev, const yond_raw_norm* nrm_dev, int nframes, int max_H, int max_W,
+                               float* var, float* mean, float* lap, int k, float* seg_max, void* work, void* stream);
+int yond_nlf_maps_frames_collab_cached(const float* y, const yond_frame_geom* frames_dev, int nframes, int max_H, int max_W,
+                                       const float* lr_var, float* var, float* mean, float* lap, int k, void* stream);
+int yond_vst_fwd_frames(const yond_frame_geom* frames_dev, const yond_raw_norm* nrm_dev, float* z, float* ub, int B, int H, int W,
+                        int pad_l, int pad_r, int pad_t, int pad_b, const yond_vst_params* params_dev, const float* rows,
+                        const float* xnodes, int row_stride, void* stream);
+
 /* ---- the VST parameter chain on the device — YOND_SIDD.py:356 (round 1) / :438-447 (round 2 guards), :252-269,
  * :284-285 (bias source, VST(0), VST(scale), t = nsr*1.03), utils/isp_algos.py:179-231 (sigma row of the BiasLUT),
  * :49-140 (get_bias: the numeric Poisson (*) Gaussian fallback table — SURVEY 8(f)-2, generated on the device).

@@ -67,6 +67,10 @@ SIGNATURES = {
     "yond_nlf_fit_ragged_work_bytes": (_SZ, [_I]),
     "yond_nlf_fit_ragged": (_I, [_P, _P, _P, _P, _SZ, _I, C.POINTER(_D), _I, _P, _P, _P, _P]),
     "yond_seg_max": (_I, [_P, _SZ, _I, _P, _P]),
+    "yond_nlf_maps_frames_max": (_I, [_P, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P]),
+    "yond_nlf_maps_frames_raw16": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P]),
+    "yond_nlf_maps_frames_collab_cached": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _I, _P]),
+    "yond_vst_fwd_frames": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P]),
     "yond_chain_work_bytes": (_SZ, [_I]),
     "yond_bias_table_nodes": (_I, [C.c_float]),
     "yond_vst_params_fill": (_I, [_P, _P, _I, _I, _D, _D, _D, _I, _I, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P]),

@@ -324,15 +324,22 @@ __device__ __forceinline__ float tab_lookup(float xq, uint32_t tab, int kind, in
   while (xq < e.x && g > 0) e = lds_v4f(tab + 16u * (uint32_t)(--g));
   return fmaf(fmaxf(xq - e.x, 0.f), e.z, e.y);
 }
-template <bool kVst>
+// kTable: frame b is the (H, W) frame of record frames[b] (yond_frame_geom), read once per CTA, instead of frame b of one (B, H, W)
+// tensor — the frames of one size of a batch stay where their owners keep them.  With raw_in.per_img set the record's `base` is a uint16
+// sensor mosaic, normalised with raw_in.per_img[b].  The arithmetic and the z / ub outputs are the uniform form's.
+template <bool kVst, bool kTable = false>
 __global__ void __launch_bounds__(kBlock, 5) vst_fwd_kernel(const float* __restrict__ bayer, float* __restrict__ z,
                                                          float* __restrict__ ub, int H, int W, int pl, int pt, int hp, int wp,
                                                          const yond_vst_params* __restrict__ params,
                                                          const float* __restrict__ rows, const float* __restrict__ xnodes,
-                                                         int row_stride, RawNorm raw_in) {
+                                                         int row_stride, RawNorm raw_in, const yond_frame_geom* frames) {
   extern __shared__ float4 tab[];
   __shared__ TabInfo ti;
   const int b = blockIdx.y;
+  if constexpr (kTable) {
+    bayer = frames[b].base;
+    if (raw_in.per_img) raw_in.base = reinterpret_cast<const uint16_t*>(bayer);
+  }
   const RawNorm raw = raw_norm_at(raw_in, b);  // every pixel of a CTA belongs to frame b
   const int h = H >> 1, w = W >> 1;
   VstConst c{};
@@ -380,7 +387,7 @@ __global__ void __launch_bounds__(kBlock, 5) vst_fwd_kernel(const float* __restr
   const int t_kind = ti.kind, t_n = ti.n;
   const float t_last = ti.last, t_ext = ti.ext;
   const float invK = kVst ? 1.0f / c.K : 0.f;
-  const float* frame = bayer + (size_t)b * H * W;
+  const float* frame = bayer + (kTable ? 0 : (size_t)b * H * W);
   float4* zo = reinterpret_cast<float4*>(z) + (size_t)b * hp * wp;
   const int npix = hp * wp;
   float vmax = 0.f;
@@ -393,7 +400,7 @@ __global__ void __launch_bounds__(kBlock, 5) vst_fwd_kernel(const float* __restr
     const size_t poff = (size_t)(2 * refl(i - pt, h)) * W + 2 * refl(j - pl, w);
     float v[4];
     if (raw.base) {  // uint16 sensor mosaic, normalised on load (SURVEY 8(f)-1)
-      const uint16_t* r16 = raw.base + (size_t)b * H * W + poff;
+      const uint16_t* r16 = raw.base + (kTable ? 0 : (size_t)b * H * W) + poff;
       const uint32_t a = __ldg(reinterpret_cast<const uint32_t*>(r16)), d = __ldg(reinterpret_cast<const uint32_t*>(r16 + W));
       v[0] = raw_norm(a & 0xffffu, raw); v[1] = raw_norm(a >> 16, raw); v[2] = raw_norm(d & 0xffffu, raw); v[3] = raw_norm(d >> 16, raw);
     } else {
@@ -647,7 +654,7 @@ int yond_table_apply(const float* x, float* bias, size_t n, const float* vals, c
 
 static int launch_fwd(bool vst, const float* bayer, float* z, float* ub, int B, int H, int W, int pl, int pr, int pt, int pb,
                       const yond_vst_params* params, const float* rows, const float* xnodes, int row_stride, void* stream,
-                      RawNorm raw = RawNorm{}) {
+                      RawNorm raw = RawNorm{}, const yond_frame_geom* frames = nullptr) {
   YOND_REQUIRE(B > 0 && H % 2 == 0 && W % 2 == 0 && H > 0 && W > 0, "vst_fwd: H,W must be even");
   const int h = H / 2, w = W / 2;
   YOND_REQUIRE(pl >= 0 && pr >= 0 && pt >= 0 && pb >= 0 && pl < w && pr < w && pt < h && pb < h,
@@ -662,14 +669,24 @@ static int launch_fwd(bool vst, const float* bayer, float* z, float* ub, int B, 
     const int tab_n = rows ? (row_stride > 1921 ? row_stride : 1921) : 0;
     const size_t smem = (size_t)tab_n * sizeof(float4);
     YOND_REQUIRE(smem <= 200 * 1024, "vst_fwd: bias tables of more than %d nodes are not supported (row_stride %d)", 200 * 1024 / 16, row_stride);
-    static std::once_flag once;
-    static cudaError_t attr_err = cudaSuccess;
-    std::call_once(once, [] { attr_err = cudaFuncSetAttribute(vst_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
-    if (attr_err != cudaSuccess) return yond_set_error(YOND_ERR_CUDA, "cudaFuncSetAttribute(vst_fwd_kernel) failed: %s", cudaGetErrorString(attr_err));
+    static std::once_flag once, once_tab;
+    static cudaError_t attr_err = cudaSuccess, attr_err_tab = cudaSuccess;
+    cudaError_t err;
+    if (frames) {
+      std::call_once(once_tab, [] { attr_err_tab = cudaFuncSetAttribute(vst_fwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
+      err = attr_err_tab;
+    } else {
+      std::call_once(once, [] { attr_err = cudaFuncSetAttribute(vst_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
+      err = attr_err;
+    }
+    if (err != cudaSuccess) return yond_set_error(YOND_ERR_CUDA, "cudaFuncSetAttribute(vst_fwd_kernel) failed: %s", cudaGetErrorString(err));
     YondProfScope prof("vst_fwd", s, 8.0 * (double)B * H * W);  // 4 R (Bayer f32) + 4 W (z f32) per Bayer pixel
-    vst_fwd_kernel<true><<<grid, kBlock, smem, s>>>(bayer, z, ub, H, W, pl, pt, hp, wp, params, rows, xnodes, row_stride, raw);
+    if (frames)
+      vst_fwd_kernel<true, true><<<grid, kBlock, smem, s>>>(nullptr, z, ub, H, W, pl, pt, hp, wp, params, rows, xnodes, row_stride, raw, frames);
+    else
+      vst_fwd_kernel<true><<<grid, kBlock, smem, s>>>(bayer, z, ub, H, W, pl, pt, hp, wp, params, rows, xnodes, row_stride, raw, nullptr);
   } else {
-    vst_fwd_kernel<false><<<grid, kBlock, 0, s>>>(bayer, z, ub, H, W, pl, pt, hp, wp, nullptr, nullptr, nullptr, 0, raw);
+    vst_fwd_kernel<false><<<grid, kBlock, 0, s>>>(bayer, z, ub, H, W, pl, pt, hp, wp, nullptr, nullptr, nullptr, 0, raw, nullptr);
   }
   YOND_LAUNCH_CHECK();
   return YOND_OK;
@@ -688,6 +705,15 @@ int yond_vst_fwd_raw16(const uint16_t* raw, const yond_raw_norm* nrm, float* z, 
                "yond_vst_fwd_raw16: bad normalisation / alignment");
   return launch_fwd(true, nullptr, z, ub, B, H, W, pad_l, pad_r, pad_t, pad_b, params_dev, rows, xnodes, row_stride, stream,
                     make_raw_norm(raw, nrm, nrm_dev, frames_per_img));
+}
+int yond_vst_fwd_frames(const yond_frame_geom* frames_dev, const yond_raw_norm* nrm_dev, float* z, float* ub, int B, int H, int W,
+                        int pad_l, int pad_r, int pad_t, int pad_b, const yond_vst_params* params_dev, const float* rows,
+                        const float* xnodes, int row_stride, void* stream) {
+  YOND_REQUIRE(frames_dev != nullptr && params_dev != nullptr, "yond_vst_fwd_frames: null argument");
+  RawNorm raw{};
+  raw.per_img = nrm_dev;  // uint16 records: the kernel takes each mosaic's address from its record
+  raw.units_per_img = 1;
+  return launch_fwd(true, nullptr, z, ub, B, H, W, pad_l, pad_r, pad_t, pad_b, params_dev, rows, xnodes, row_stride, stream, raw, frames_dev);
 }
 int yond_pack_pad(const float* bayer, float* z, float* ub, int B, int H, int W, int pad_l, int pad_r, int pad_t, int pad_b,
                   void* stream) {

@@ -63,6 +63,11 @@ constexpr int kRows = 4;
 // kRagged (wide layout): blockIdx.z picks a frame record (yond_frame_geom: its own h, w, Bayer source and map offset; a packed source
 // is `src.base` + that offset) instead of an image of one (B, h, w) geometry.  The grid is sized by the largest frame; the CTAs past
 // a smaller frame's column blocks or strips return before the first barrier.  The arithmetic is the uniform form's.
+// A ragged Bayer source is one of three, chosen once per CTA:
+//   - src.raw.per_img set: the record's `base` is a uint16 sensor mosaic, normalised on load with src.raw.per_img[blockIdx.z];
+//   - src.base set: the float32 frame at src.base + off of one flat buffer (a round's output, laid out like the maps);
+//   - neither: the record's `base` is a float32 frame.
+// src.seg_max (optional) is one slot per frame.
 template <bool kSq, int kCols, bool kBayer, bool kNarrow, bool kRagged = false>  // kCols = 256, or 160 when a whole row plus both halos fits
 __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, float4* __restrict__ out0,
                                                                 float4* __restrict__ out1, int B, int h, int w, int k, int op,
@@ -87,7 +92,13 @@ __global__ void __launch_bounds__(kBoxThreads) box_fused_kernel(BoxSrc src, floa
     h = f.H / 2;
     w = f.W / 2;
     if ((int)blockIdx.x * outc >= w || (int)blockIdx.y * rows_per_strip >= h) return;
-    src.base = kBayer ? f.base : src.base + f.off;
+    if (kBayer && src.raw.per_img) {
+      src.raw.base = reinterpret_cast<const uint16_t*>(f.base);
+      src.raw = raw_norm_at(src.raw, blockIdx.z);
+      src.raw.per_img = nullptr;
+    }
+    src.base = kBayer && !src.base ? f.base : src.base + f.off;
+    if (src.seg_max) src.seg_max += blockIdx.z;
     src.row_len = kBayer ? f.W : 4 * w;
     src.blk_w = w;
     src.img_stride = 0;
@@ -762,52 +773,85 @@ __global__ void score3_count_kernel(const unsigned int* __restrict__ binmin, con
 }
 
 // ------------------------------------------------------------------ masked regression sums
+// The float64 sums are formed in an order fixed by the segment's length alone, never by the grid or by atomics: segment s is cut into
+// chunks of sums_chunk(n/4) pixel quads (at most kSumsMaxChunks of them), each chunk is summed by one block in a fixed order (thread t
+// takes quads t, t + 256, ... of the chunk, then a fixed shuffle / warp tree), its 12 partial sums go to `part`, and the last block of
+// the segment to finish (a counter per segment) adds the chunk partials in chunk order.  The estimate of a frame is therefore the same
+// bits run after run, whether it is fitted alone or in a batch with frames of other sizes (whose longest segment sizes the grid).
+constexpr int kSumsMaxChunks = 4096;
+constexpr size_t kSumsChunkMin = 2048;  // pixel quads: 8 per thread
+__host__ __device__ __forceinline__ size_t sums_chunk(size_t n4) {
+  const size_t c = (n4 + kSumsMaxChunks - 1) / kSumsMaxChunks;
+  return c < kSumsChunkMin ? kSumsChunkMin : c;
+}
 template <bool kRagged>
 __global__ void __launch_bounds__(256) masked_sums_kernel(const float* __restrict__ lap, const float* __restrict__ mean,
                                                           const float* __restrict__ var, size_t n,
                                                           const double* __restrict__ ths, double* __restrict__ sums,
-                                                          const int* __restrict__ active, const unsigned long long* seg_off) {
+                                                          const int* __restrict__ active, const unsigned long long* seg_off,
+                                                          double* __restrict__ part, unsigned int* __restrict__ done) {
   if (active && !active[blockIdx.y]) return;  // second pass of the device-side estimator: only the segments that redo
   const size_t seg0 = seg_begin<kRagged>(n, seg_off, blockIdx.y);
+  const size_t n4 = n / 4, chunk = sums_chunk(n4), nch = (n4 + chunk - 1) / chunk;
+  if (blockIdx.x >= nch) return;  // a shorter segment of a ragged grid: these blocks take no part
   lap += seg0;
   mean += seg0;
   var += seg0;
   sums += (size_t)blockIdx.y * 12;
+  part += (size_t)blockIdx.y * kSumsMaxChunks * 12;
   const double th = ths[blockIdx.y];
-  double s[12];
-#pragma unroll
-  for (int i = 0; i < 12; ++i) s[i] = 0.0;
   const float4* l4 = reinterpret_cast<const float4*>(lap);
   const float4* m4 = reinterpret_cast<const float4*>(mean);
   const float4* v4 = reinterpret_cast<const float4*>(var);
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n / 4; i += (size_t)gridDim.x * blockDim.x) {
-    const float4 lv = ldg_stream_f4(l4 + i), mv = ldg_stream_f4(m4 + i), vv = ldg_stream_f4(v4 + i);
-    const float le[4] = {lv.x, lv.y, lv.z, lv.w}, me[4] = {mv.x, mv.y, mv.z, mv.w}, ve[4] = {vv.x, vv.y, vv.z, vv.w};
+  __shared__ double red[8][12];
+  __shared__ bool last;
+  for (size_t c = blockIdx.x; c < nch; c += gridDim.x) {
+    double s[12];
 #pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      if ((double)le[e] < th) {
-        const float xf = me[e];
-        const double x = xf, y = ve[e];
-        s[0] += 1.0; s[1] += x; s[2] += y; s[3] += x * x; s[4] += x * y; s[5] += y * y;
-        if (xf > 1e-4f && xf < 0.8f) {
-          s[6] += 1.0; s[7] += x; s[8] += y; s[9] += x * x; s[10] += x * y; s[11] += y * y;
+    for (int i = 0; i < 12; ++i) s[i] = 0.0;
+    const size_t end = min(n4, (c + 1) * chunk);
+    for (size_t i = c * chunk + threadIdx.x; i < end; i += blockDim.x) {
+      const float4 lv = ldg_stream_f4(l4 + i), mv = ldg_stream_f4(m4 + i), vv = ldg_stream_f4(v4 + i);
+      const float le[4] = {lv.x, lv.y, lv.z, lv.w}, me[4] = {mv.x, mv.y, mv.z, mv.w}, ve[4] = {vv.x, vv.y, vv.z, vv.w};
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        if ((double)le[e] < th) {
+          const float xf = me[e];
+          const double x = xf, y = ve[e];
+          s[0] += 1.0; s[1] += x; s[2] += y; s[3] += x * x; s[4] += x * y; s[5] += y * y;
+          if (xf > 1e-4f && xf < 0.8f) {
+            s[6] += 1.0; s[7] += x; s[8] += y; s[9] += x * x; s[10] += x * y; s[11] += y * y;
+          }
         }
       }
     }
-  }
-  __shared__ double red[8][12];
 #pragma unroll
-  for (int i = 0; i < 12; ++i) {
-    double v = s[i];
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5][i] = v;
+    for (int i = 0; i < 12; ++i) {
+      double v = s[i];
+      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5][i] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < 12) {
+      double v = 0;
+      for (int wq = 0; wq < 8; ++wq) v += red[wq][threadIdx.x];
+      part[c * 12 + threadIdx.x] = v;
+    }
+    __syncthreads();  // `red` is rewritten by the next chunk
   }
+  // the last block of the segment adds the chunk partials in chunk order
+  __threadfence();
   __syncthreads();
+  if (threadIdx.x == 0) last = atomicAdd(&done[blockIdx.y], 1u) == (unsigned)min((size_t)gridDim.x, nch) - 1;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
   if (threadIdx.x < 12) {
     double v = 0;
-    for (int wq = 0; wq < 8; ++wq) v += red[wq][threadIdx.x];
-    atomicAdd(&sums[threadIdx.x], v);
+    for (size_t c = 0; c < nch; ++c) v += __ldcg(part + c * 12 + threadIdx.x);
+    sums[threadIdx.x] = v;
   }
+  if (threadIdx.x == 0) done[blockIdx.y] = 0;  // ready for the next pass
 }
 
 // ------------------------------------------------------------------ device-resident estimator tail
@@ -993,12 +1037,13 @@ int box_pass(const BoxSrc& src, bool bayer, float* out0, float* out1, int B, int
 // packed one is `src.base` plus each record's offset; the outputs are the concatenated maps.
 template <bool SQ, bool BAYER>
 int box_pass_frames(const BoxSrc& src, float* out0, float* out1, const yond_frame_geom* frames, int nframes, int max_h, int max_w, int k,
-                    int op, cudaStream_t s) {
+                    int op, cudaStream_t s, const float* aux = nullptr, float* out2 = nullptr) {
   const int r = k / 2, rows_per_strip = 64;
   const dim3 g(ceil_div(max_w, 256 - 2 * r), ceil_div(max_h, rows_per_strip), nframes);
   YOND_REQUIRE(g.z <= 65535, "box filter: at most 65535 frames per call");
   const int rc = launch_box<SQ, 256, BAYER, false, true>(g, s, src, reinterpret_cast<float4*>(out0), reinterpret_cast<float4*>(out1),
-                                                         nframes, max_h, max_w, k, op, rows_per_strip, nullptr, nullptr, frames);
+                                                         nframes, max_h, max_w, k, op, rows_per_strip,
+                                                         reinterpret_cast<const float4*>(aux), reinterpret_cast<float4*>(out2), frames);
   if (rc) return rc;
   YOND_LAUNCH_CHECK();
   return YOND_OK;
@@ -1159,8 +1204,10 @@ int yond_nlf_maps_collab_cached(const float* y, int y_mosaic, const float* lr_va
 }
 
 // SelfNLF's maps of frames of different sizes: the three box passes of nlf_maps_impl mode 0, one launch each for all frames.
-int yond_nlf_maps_frames(const yond_frame_geom* frames_dev, int nframes, int max_H, int max_W, float* var, float* mean, float* lap, int k,
-                         void* work, void* stream) {
+// nrm_dev != nullptr: the records hold uint16 sensor mosaics, frame i normalised with nrm_dev[i].  seg_max (optional): max(x, 0) per frame
+// from the first pass.
+static int nlf_maps_frames_impl(const yond_frame_geom* frames_dev, const yond_raw_norm* nrm_dev, int nframes, int max_H, int max_W,
+                                float* var, float* mean, float* lap, int k, float* seg_max, void* work, void* stream) {
   YOND_REQUIRE(frames_dev && var && mean && lap && work, "yond_nlf_maps_frames: null argument");
   YOND_REQUIRE(nframes > 0 && nframes <= 65535, "yond_nlf_maps_frames: 1..65535 frames");
   YOND_REQUIRE(k % 2 == 1 && k >= 3 && k <= kMaxK, "yond_nlf_maps_frames: odd k <= %d required (got %d)", kMaxK, k);
@@ -1171,14 +1218,50 @@ int yond_nlf_maps_frames(const yond_frame_geom* frames_dev, int nframes, int max
   float* tmp = reinterpret_cast<float*>(work);
   BoxSrc bayer{};  // base, strides and row length come from the records
   bayer.imgs_per_seg = 1;
+  bayer.raw.per_img = nrm_dev;  // uint16 records: the kernel takes each mosaic's address from its record and entry i of nrm_dev
+  bayer.raw.units_per_img = 1;
   BoxSrc packed = bayer;
   packed.base = tmp;
+  packed.raw = RawNorm{};
+  BoxSrc first = bayer;
+  first.seg_max = seg_max;
+  if (seg_max) YOND_CUDA_CHECK(cudaMemsetAsync(seg_max, 0, sizeof(float) * nframes, s));
   YondProfScope prof("nlf_maps_frames (3 box_fused passes)", s, 0.0);  // no byte count: the frame sizes are in device memory
   int rc;
   // mean = blur_k(x), var = std_k(x)^2 ; blur_k2(x) -> tmp ; lap = std_k(blur_k2(x))  (YOND_SIDD.py:66-71)
-  if ((rc = box_pass_frames<true, true>(bayer, mean, var, frames_dev, nframes, h, w, k, OP_MEAN_VAR, s))) return rc;
+  if ((rc = box_pass_frames<true, true>(first, mean, var, frames_dev, nframes, h, w, k, OP_MEAN_VAR, s))) return rc;
   if ((rc = box_pass_frames<false, true>(bayer, tmp, nullptr, frames_dev, nframes, h, w, k2, OP_MEAN, s))) return rc;
   return box_pass_frames<true, false>(packed, lap, nullptr, frames_dev, nframes, h, w, k, OP_STD, s);
+}
+int yond_nlf_maps_frames(const yond_frame_geom* frames_dev, int nframes, int max_H, int max_W, float* var, float* mean, float* lap, int k,
+                         void* work, void* stream) {
+  return nlf_maps_frames_impl(frames_dev, nullptr, nframes, max_H, max_W, var, mean, lap, k, nullptr, work, stream);
+}
+int yond_nlf_maps_frames_max(const yond_frame_geom* frames_dev, int nframes, int max_H, int max_W, float* var, float* mean, float* lap,
+                             int k, void* work, void* stream, float* seg_max) {
+  return nlf_maps_frames_impl(frames_dev, nullptr, nframes, max_H, max_W, var, mean, lap, k, seg_max, work, stream);
+}
+int yond_nlf_maps_frames_raw16(const yond_frame_geom* frames_dev, const yond_raw_norm* nrm_dev, int nframes, int max_H, int max_W,
+                               float* var, float* mean, float* lap, int k, float* seg_max, void* work, void* stream) {
+  YOND_REQUIRE(nrm_dev != nullptr, "yond_nlf_maps_frames_raw16: null argument");
+  return nlf_maps_frames_impl(frames_dev, nrm_dev, nframes, max_H, max_W, var, mean, lap, k, seg_max, work, stream);
+}
+
+// CollabNLF's maps of frames of different sizes from the cached std_k(lr)^2 maps (yond_nlf_maps_collab_cached, one launch for all frames):
+// frame i of y is the float32 Bayer frame at y + off_i, the same offset as its maps.
+int yond_nlf_maps_frames_collab_cached(const float* y, const yond_frame_geom* frames_dev, int nframes, int max_H, int max_W,
+                                       const float* lr_var, float* var, float* mean, float* lap, int k, void* stream) {
+  YOND_REQUIRE(y && frames_dev && lr_var && var && mean && lap, "yond_nlf_maps_frames_collab_cached: null argument");
+  YOND_REQUIRE(nframes > 0 && nframes <= 65535, "yond_nlf_maps_frames_collab_cached: 1..65535 frames");
+  YOND_REQUIRE(k % 2 == 1 && k >= 3 && k <= kMaxK, "yond_nlf_maps_frames_collab_cached: odd k <= %d required (got %d)", kMaxK, k);
+  YOND_REQUIRE(max_H > 0 && max_W > 0 && max_H % 2 == 0 && max_W % 2 == 0, "yond_nlf_maps_frames_collab_cached: H,W must be even");
+  YOND_REQUIRE((uintptr_t)y % 16 == 0 && (uintptr_t)lr_var % 16 == 0, "yond_nlf_maps_frames_collab_cached: aligned buffers required");
+  cudaStream_t s = (cudaStream_t)stream;
+  BoxSrc flat{};
+  flat.base = y;
+  flat.imgs_per_seg = 1;
+  YondProfScope prof("nlf_maps_frames_collab (1 box_fused pass, lr statistics reused)", s, 0.0);
+  return box_pass_frames<true, true>(flat, mean, lap, frames_dev, nframes, max_H / 2, max_W / 2, k, OP_COLLAB, s, lr_var, var);
 }
 
 }  // extern "C"
@@ -1249,11 +1332,11 @@ inline dim3 sums_grid(size_t seg_len, int nseg) {
 // {lap < th, 1e-4 < mean < 0.8} (polyfit's non-saturated subset, utils/isp_algos.py:348-350), float64
 template <bool RAGGED>
 int masked_sums(const float* lap, const float* mean, const float* var, size_t seg_len, int nseg, const double* ths_dev, double* sums_dev,
-                cudaStream_t s, const unsigned long long* seg_off) {
-  YOND_CUDA_CHECK(cudaMemsetAsync(sums_dev, 0, (size_t)nseg * 12 * sizeof(double), s));
+                cudaStream_t s, const unsigned long long* seg_off, double* part, unsigned int* done) {
   {
     YondProfScope prof("masked_sums", s, 12.0 * (double)seg_len * nseg);
-    masked_sums_kernel<RAGGED><<<sums_grid(seg_len, nseg), 256, 0, s>>>(lap, mean, var, seg_len, ths_dev, sums_dev, nullptr, seg_off);
+    masked_sums_kernel<RAGGED><<<sums_grid(seg_len, nseg), 256, 0, s>>>(lap, mean, var, seg_len, ths_dev, sums_dev, nullptr, seg_off, part,
+                                                                        done);
   }
   YOND_LAUNCH_CHECK();
   return YOND_OK;
@@ -1263,9 +1346,10 @@ int masked_sums(const float* lap, const float* mean, const float* var, size_t se
 struct FitWork {
   SelectWork* sel;
   unsigned long long* ranks;
-  double *gamma, *ths, *th25, *th, *th2, *sums, *sums2;
+  double *gamma, *ths, *th25, *th, *th2, *sums, *sums2, *part;
   float* stats;
   int *npeaks, *minj, *idx, *redo;
+  unsigned int* done;
   size_t bytes;
 };
 FitWork carve_fit(void* base, int nseg) {
@@ -1292,6 +1376,8 @@ FitWork carve_fit(void* base, int nseg) {
   w.minj = (int*)take((size_t)nseg * 1024 * 4);
   w.idx = (int*)take((size_t)nseg * 4);
   w.redo = (int*)take((size_t)nseg * 4);
+  w.part = (double*)take((size_t)nseg * kSumsMaxChunks * 12 * 8);  // chunk partials of the masked sums
+  w.done = (unsigned int*)take((size_t)nseg * 4);
   w.bytes = align_up(off, 256);
   return w;
 }
@@ -1321,11 +1407,13 @@ int nlf_fit_impl(const float* var, const float* mean, const float* lap, const un
   YOND_LAUNCH_CHECK();
   pick_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(ql, w.ths, w.npeaks, w.th, w.idx, nseg);
   YOND_LAUNCH_CHECK();
-  if ((rc = masked_sums<RAGGED>(lap, mean, var, seg_len, nseg, w.th, w.sums, s, seg_off))) return rc;
+  YOND_CUDA_CHECK(cudaMemsetAsync(w.done, 0, (size_t)nseg * sizeof(unsigned int), s));  // the last block of a pass resets its counter
+  if ((rc = masked_sums<RAGGED>(lap, mean, var, seg_len, nseg, w.th, w.sums, s, seg_off, w.part, w.done))) return rc;
   backup_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(w.sums, w.th, w.th25, w.th2, w.redo, w.sums2, nseg);
   YOND_LAUNCH_CHECK();
   // second pass: only the segments whose mask came out empty do any work
-  masked_sums_kernel<RAGGED><<<sums_grid(seg_len, nseg), 256, 0, s>>>(lap, mean, var, seg_len, w.th2, w.sums2, w.redo, seg_off);
+  masked_sums_kernel<RAGGED><<<sums_grid(seg_len, nseg), 256, 0, s>>>(lap, mean, var, seg_len, w.th2, w.sums2, w.redo, seg_off, w.part,
+                                                                      w.done);
   YOND_LAUNCH_CHECK();
   solve_kernel<<<ceil_div(nseg, 64), 64, 0, s>>>(w.sums, w.sums2, w.redo, w.th2, w.idx, w.ths, w.npeaks, ql, regs_dev, detail_dev, nseg);
   YOND_LAUNCH_CHECK();

@@ -20,10 +20,15 @@ FRAME_GEOM = np.dtype([("base", "<u8"), ("H", "<i4"), ("W", "<i4"), ("off", "<i8
 assert FRAME_GEOM.itemsize == 24
 
 
-def check_frames(frames, nimg=None, k=29):
+RAW_DTYPES = (torch.int16, torch.uint16)
+
+
+def check_frames(frames, nimg=None, k=29, raw=False):
     """Bayer frames of any even sizes as a list of (H, W) CUDA float32 tensors: a sequence of them, one (n, H, W) tensor or one (H, W)
     frame.  Raises ValueError for a count other than `nimg` (when given), a frame that is not a contiguous 2-D CUDA float32 tensor, an
-    odd H or W, or a packed size (H/2, W/2) not larger than the filter radius k // 2 (the box filters reflect once at the border)."""
+    odd H or W, or a packed size (H/2, W/2) not larger than the filter radius k // 2 (the box filters reflect once at the border).
+    raw: the frames are int16 / uint16 sensor mosaics instead.  Also raises ValueError for a list that mixes dtypes and for a frame whose
+    data pointer is not aligned for the kernels' Bayer loads (8 bytes for float32, 4 for a 16-bit mosaic)."""
     if isinstance(frames, torch.Tensor):
         if frames.dim() not in (2, 3):
             raise ValueError(f"frames: one (n, H, W) tensor or (H, W) frame expected, got shape {tuple(frames.shape)}")
@@ -35,6 +40,9 @@ def check_frames(frames, nimg=None, k=29):
             raise ValueError(f"frames: a sequence of (H, W) tensors or one (n, H, W) tensor expected, got {type(frames).__name__}") from None
     if not frames or (nimg is not None and len(frames) != nimg):
         raise ValueError(f"frames: {nimg if nimg is not None else 'at least one'} frame(s) expected, got {len(frames)}")
+    dtypes = sorted({str(f.dtype) for f in frames if isinstance(f, torch.Tensor)})
+    if len(dtypes) > 1:
+        raise ValueError(f"frames: one dtype expected, the list mixes {', '.join(dtypes)}")
     for i, f in enumerate(frames):
         if not isinstance(f, torch.Tensor) or f.dim() != 2:
             raise ValueError(f"frame {i}: a 2-D (H, W) tensor expected, got {getattr(f, 'shape', type(f).__name__)}")
@@ -43,13 +51,49 @@ def check_frames(frames, nimg=None, k=29):
             raise ValueError(f"frame {i}: H and W must be even (Bayer 2x2 cells), got {H}x{W}")
         if min(H, W) // 2 <= k // 2:
             raise ValueError(f"frame {i}: packed size {H // 2}x{W // 2} must exceed the filter radius {k // 2}")
-        if f.dtype != torch.float32:
-            raise ValueError(f"frame {i}: float32 expected, got {f.dtype}")
+        if raw and f.dtype not in RAW_DTYPES:
+            raise ValueError(f"frame {i}: raw= given, so an int16 / uint16 sensor mosaic expected, got {f.dtype}")
+        if not raw and f.dtype != torch.float32:
+            hint = " (a 16-bit sensor mosaic needs raw=)" if f.dtype in RAW_DTYPES else ""
+            raise ValueError(f"frame {i}: float32 expected, got {f.dtype}{hint}")
         if not f.is_contiguous():
             raise ValueError(f"frame {i}: a contiguous tensor expected")
+        align = 4 if raw else 8
+        if f.data_ptr() % align:
+            raise ValueError(f"frame {i}: data pointer {f.data_ptr():#x} is not {align}-byte aligned (the Bayer loads of the kernels)")
         if not f.is_cuda:
             raise ValueError(f"frame {i}: a CUDA tensor expected, got one on {f.device}")
     return frames
+
+
+class FrameTable:
+    """Frames of any even sizes as the kernels address them: one yond_frame_geom record per frame (its address, H, W and the float offset
+    of its maps, which is also its offset in a flat buffer of the frames' outputs) and the fit's nframes + 1 segment offsets, copied to
+    the device together with the host arrays of `extra` in one non-blocking copy from pinned memory.  The frames are not copied: the
+    caller keeps them alive and unchanged while work that reads them is enqueued.
+    Attributes: geom / off (host), records / seg_off (device views), extra (device byte views, one per array of `extra`), nframes,
+    n_el (= off[-1]), max_H, max_W, device."""
+
+    def __init__(self, frames, extra=()):
+        from .pipeline import _upload
+        off = np.concatenate([[0], np.cumsum([f.numel() for f in frames])]).astype(np.uint64)
+        geom = np.zeros(len(frames), FRAME_GEOM)
+        geom["base"] = [f.data_ptr() for f in frames]
+        geom["H"] = [f.shape[0] for f in frames]
+        geom["W"] = [f.shape[1] for f in frames]
+        geom["off"] = off[:-1].astype(np.int64)
+        arrays = [geom, off] + list(extra)
+        buf, offs = _upload(arrays, frames[0].device)
+        views = [buf[o:o + np.asarray(a).nbytes] for o, a in zip(offs, arrays)]
+        self.geom, self.off = geom, off
+        self.records, self.seg_off, self.extra = views[0], views[1].view(torch.int64), views[2:]
+        self.nframes, self.n_el = len(frames), int(off[-1])
+        self.max_H, self.max_W = int(geom["H"].max()), int(geom["W"].max())
+        self.device = frames[0].device
+
+    def records_from(self, i):
+        """The device records of frames i, i + 1, ..."""
+        return self.records[i * FRAME_GEOM.itemsize:]
 
 
 class NlfEstimator:
@@ -147,36 +191,64 @@ class NlfEstimator:
         return (regs, detail) if details else regs
 
     # -- the self estimate of frames of different sizes (round 1 of IterDenoise on the full-resolution frames) ----------------
-    def maps_frames(self, frames, k=29):
+    def maps_frames(self, frames, k=29, var_map=None, seg_max=None, raw=None):
         """SelfNLF maps of a list of (H, W) CUDA float32 Bayer frames of any even sizes (check_frames), every box pass one launch for
         all of them.  Returns var, mean, lap: flat float32 maps, frame i's packed (H/2, W/2, 4) maps at float offsets
-        off[i]:off[i + 1] (off: the host array of the nframes + 1 offsets), then off and the device copy of the offsets (uint64)."""
-        from .pipeline import _upload
-        frames = check_frames(frames, None, k)
-        lib, dev = self.lib, frames[0].device
-        off = np.concatenate([[0], np.cumsum([f.numel() for f in frames])]).astype(np.uint64)
-        geom = np.zeros(len(frames), FRAME_GEOM)
-        geom["base"] = [f.data_ptr() for f in frames]
-        geom["H"] = [f.shape[0] for f in frames]
-        geom["W"] = [f.shape[1] for f in frames]
-        geom["off"] = off[:-1].astype(np.int64)
-        buf, offs = _upload([geom, off], dev)  # the records and the fit's segment offsets: one copy from pinned memory
-        n_el = int(off[-1])
+        off[i]:off[i + 1] (off: the host array of the nframes + 1 offsets), then off and the device copy of the offsets (uint64).
+        frames may also be a FrameTable of frames already checked and uploaded.
+        var_map (optional; float32 CUDA, at least off[-1] values): the var map goes there instead of the estimator's scratch, where no
+        later call overwrites it — the cached noisy-frame statistics of the collab rounds (estimate_collab_frames).
+        seg_max (optional, (nframes,) f32 CUDA): receives max(x, 0) per frame.
+        raw: the frames are uint16 / int16 sensor mosaics and raw the CUDA uint8 tensor of their nframes yond_raw_norm records (one per
+        frame, in the order of the frames): they are normalised on load."""
+        lib = self.lib
+        t = frames if isinstance(frames, FrameTable) else FrameTable(check_frames(frames, None, k, raw=raw is not None))
+        dev, n_el = t.device, t.n_el
         maps = self._buf("maps3", 3 * n_el * 4, dev).view(torch.float32)
         var, mean, lap = maps[:n_el], maps[n_el:2 * n_el], maps[2 * n_el:3 * n_el]
+        if var_map is not None:
+            assert var_map.dtype == torch.float32 and var_map.is_cuda and var_map.numel() >= n_el
+            var = var_map.reshape(-1)[:n_el]
         work = self._buf("maps", n_el * 4, dev)
-        check(lib.yond_nlf_maps_frames(ptr(buf), len(frames), int(geom["H"].max()), int(geom["W"].max()), ptr(var), ptr(mean), ptr(lap),
-                                       int(k), ptr(work), stream_ptr()))
-        return var, mean, lap, off, buf[offs[1]:offs[1] + off.nbytes].view(torch.int64)
+        args = (t.nframes, t.max_H, t.max_W, ptr(var), ptr(mean), ptr(lap), int(k))
+        if raw is not None:
+            assert isinstance(raw, torch.Tensor) and raw.is_cuda and raw.dtype == torch.uint8 and raw.numel() >= t.nframes * 16
+            check(lib.yond_nlf_maps_frames_raw16(ptr(t.records), ptr(raw), *args, ptr(seg_max), ptr(work), stream_ptr()))
+        elif seg_max is not None:
+            check(lib.yond_nlf_maps_frames_max(ptr(t.records), *args, ptr(work), stream_ptr(), ptr(seg_max)))
+        else:
+            check(lib.yond_nlf_maps_frames(ptr(t.records), *args, ptr(work), stream_ptr()))
+        return var, mean, lap, t.off, t.seg_off
 
-    def estimate_frames(self, frames, k=29, details=False, step=5):
+    def estimate_frames(self, frames, k=29, details=False, step=5, var_map=None, seg_max=None, raw=None):
         """Batched SelfNLF (SimpleNLF 'self') of a list of (H, W) CUDA float32 Bayer frames of any even sizes, or one (n, H, W) tensor:
         regs (nframes, 2) float64 on the device [, detail (nframes, DETAIL)], nothing read back.  The maps of all frames take one launch
         per box pass and the fit one set of launches.  A frame wider than 160 - 2*(k//2) packed pixels (every full-resolution frame) gets
         the same bits as estimate_dev on it alone; a narrower one takes the wide box-filter layout too and may differ from estimate_dev,
-        which packs such frames side by side, in the float64 rounding of the window sums."""
-        var, mean, lap, off, seg_off = self.maps_frames(frames, k)
+        which packs such frames side by side, in the float64 rounding of the window sums.  var_map, seg_max, raw and a FrameTable for
+        frames: see maps_frames."""
+        var, mean, lap, off, seg_off = self.maps_frames(frames, k, var_map, seg_max, raw)
         return self._fit(var, mean, lap, len(off) - 1, details, step, segments=(seg_off, int(np.diff(off).max())))
+
+    def collab_maps_frames(self, y, table, lr_var, k=29):
+        """CollabNLF maps (var, mean, lap) of frames of different sizes in one box pass: y is the flat float32 buffer of the frames of
+        `table` (a FrameTable; frame i at float offset off[i], the layout of the maps — a round's output of iter_denoise_frames_dev),
+        lr_var the var maps of the self estimate of the same table (maps_frames' var_map, read only)."""
+        n_el = table.n_el
+        assert y.is_cuda and y.dtype == torch.float32 and y.is_contiguous() and y.numel() >= n_el
+        assert lr_var.dtype == torch.float32 and lr_var.is_cuda and lr_var.numel() >= n_el
+        maps = self._buf("maps3", 3 * n_el * 4, y.device).view(torch.float32)
+        var, mean, lap = maps[:n_el], maps[n_el:2 * n_el], maps[2 * n_el:3 * n_el]
+        check(self.lib.yond_nlf_maps_frames_collab_cached(ptr(y), ptr(table.records), table.nframes, table.max_H, table.max_W,
+                                                          ptr(lr_var.reshape(-1)), ptr(var), ptr(mean), ptr(lap), int(k), stream_ptr()))
+        return var, mean, lap
+
+    def estimate_collab_frames(self, y, table, lr_var, k=29, details=False, step=5):
+        """CollabNLF (beta1, beta2) of a collab round of frames of different sizes (collab_maps_frames + the ragged fit): regs (nframes, 2)
+        float64 on the device."""
+        var, mean, lap = self.collab_maps_frames(y, table, lr_var, k)
+        off = table.off
+        return self._fit(var, mean, lap, table.nframes, details, step, segments=(table.seg_off, int(np.diff(off).max())))
 
     # -- the collab rounds of IterDenoise from cached noisy-frame statistics ---------------------------
     # Every collab round r >= 2 estimates on (lr, out_{r-1}) in the same geometry.  Its var map is stdfilt(lr, k)**2 -

@@ -243,12 +243,14 @@ class YondEngine:
                                        ptr(prev["ok"]) if prev is not None else None, ptr(scales_dev)))
         return out
 
-    def vst_denoise_dev(self, frames, chain, out, frames_per_row=1, fps=1, select=False, fallback=None, clip01=True, raw=None):
+    def vst_denoise_dev(self, frames, chain, out, frames_per_row=1, fps=1, select=False, fallback=None, clip01=True, raw=None, shape=None):
         """VST_Denoiser for frames (B,H,W) with device-filled parameters; writes `out` (plain (B,H,W) or the mosaic layout
         (B/n, H, n*W) for frames_per_row = n).  select: frames of images with chain['ok'] == 0 copy `fallback` instead.
         raw: frames is the uint16 sensor mosaic and raw the CUDA uint8 tensor of the yond_raw_norm records of its images (fps frames
-        each)."""
-        B, H, W = frames.shape
+        each).
+        shape = (B, H, W): frames is instead the device yond_frame_geom records (nlf.FrameTable) of B frames of that size, each read where
+        it lies (uint16 mosaics with raw; fps = 1)."""
+        B, H, W = frames.shape if shape is None else shape
         dev = frames.device
         h, w = H // 2, W // 2
         pl, pr, pt, pb = isp.get_p2d((B, 4, h, w), base=32)
@@ -264,7 +266,12 @@ class YondEngine:
         for b0 in range(0, B, cb):
             n = min(cb, B - b0)
             pch = params[b0 * psz:]
-            if raw is not None:  # uint16 sensor mosaic, normalised on load with each image's record (b0 starts an image)
+            if shape is not None:  # a table of frames of one size
+                check(self.lib.yond_vst_fwd_frames(ptr(frames[b0 * nlf.FRAME_GEOM.itemsize:]),
+                                                   ptr(raw[b0 * RAW_REC.itemsize:]) if raw is not None else None, ptr(z[:n]), ptr(ub[:n]),
+                                                   n, H, W, pl, pr, pt, pb, ptr(pch), ptr(chain["rows"]), ptr(chain["xnodes"]),
+                                                   chain["stride"], st))
+            elif raw is not None:  # uint16 sensor mosaic, normalised on load with each image's record (b0 starts an image)
                 check(self.lib.yond_vst_fwd_raw16(ptr(frames[b0:b0 + n]), None, ptr(z[:n]), ptr(ub[:n]), n, H, W, pl, pr, pt, pb, ptr(pch),
                                                   ptr(chain["rows"]), ptr(chain["xnodes"]), chain["stride"], st,
                                                   ptr(raw[b0 // fps * RAW_REC.itemsize:]), fps))
@@ -691,6 +698,106 @@ class YOND_SIDD:
         res = self.iter_denoise_dev(blocks, p, timings=timings, raw=raw, lr_full=lr_full)
         regs, rounds, _ = self.read_summary(res)
         return {"raw_dns": list(res["dns"]), "regs": regs, "rounds": rounds, "lr_raw": None, "dev": res}
+
+    # -- full frames of different sizes in one batch ---------------------------------------------------------------------
+    def _check_frames_call(self, frames, p, raw):
+        """The ValueErrors of iter_denoise_frames_dev, all raised before anything is enqueued."""
+        pipe = self.pipe
+        if pipe.get("sidd_256"):
+            raise ValueError("iter_denoise_frames: pipe['sidd_256'] cuts blocks of a SIDD mosaic into strips; full frames of different sizes "
+                             "are one image each (set sidd_256 False)")
+        if not pipe["full_est"] or "simple" not in pipe["est_type"]:
+            raise ValueError(f"iter_denoise_frames: the blind pipeline needs full_est and a 'simple' est_type, got full_est="
+                             f"{pipe['full_est']!r}, est_type={pipe['est_type']!r}")
+        n_collab = collab_rounds(pipe)
+        if isinstance(frames, torch.Tensor):
+            raise ValueError("iter_denoise_frames: a list of (H, W) frames expected (a stacked tensor goes to iter_denoise_batch)")
+        frames = list(frames)
+        if len(frames) > 65535:
+            raise ValueError(f"iter_denoise_frames: at most 65535 frames per call, got {len(frames)}")
+        exposure = batch_exposure(p, len(frames), raw)
+        frames = nlf.check_frames(frames, None, pipe["k"], raw=raw is not None)
+        return frames, n_collab, exposure
+
+    def iter_denoise_frames_dev(self, frames, p, raw=None):
+        """IterDenoise (YOND_SIDD.py:301-483, `simple` estimator) for a batch of full frames of any even sizes: each image is its frame,
+        as in iter_denoise_dev with nblk = 1, and gets exactly what iter_denoise_dev gives on that frame alone.  No host synchronisation
+        between the first and the last kernel; every round, liveness and selection of stopped images as in iter_denoise_dev.
+        frames: a list of (H_i, W_i) CUDA tensors, float32 Bayer frames, or with raw = (black, white, ratio[, clip]) int16 / uint16 sensor
+        mosaics normalised on load.  p['wp'], p['bl'], p['scale'] and the entries of raw: a scalar or one value per frame (caller order).
+        ValueError before anything is enqueued for a malformed or misaligned frame (nlf.check_frames), a mix of dtypes, 16-bit frames
+        without raw= or float32 frames with it, pipe['sidd_256'], a pipeline without full_est / a 'simple' est_type, the exposure errors
+        of batch_exposure and more than 65535 frames.
+
+        The frames are ordered on the host by padded size (then H, W; ties keep the caller's order), so that every size is a contiguous
+        range of the DEVICE ORDER: res['order'][j] is the caller index of device row j.  The estimator and the parameter chain run once
+        per round for all frames; the VST front end, the network and the inverse run once per size (and chunk).  No frame is copied: the
+        kernels read each one where it lies, so the caller keeps them unchanged until the work is done.
+        Returns dns / regs4 / live = per-round lists like iter_denoise_dev: dns[r][i] is caller frame i's (H_i, W_i) output (the outputs of
+        a round are views into one flat buffer, res['flat'][r], in device order), regs4[r] (nimg, 4) float64 and live[r] (nimg,) int32
+        rows are in DEVICE order."""
+        frames, n_collab, (scale_est, scale, raw_rec) = self._check_frames_call(frames, p, raw)
+        pipe, eng, est = self.pipe, self.engine, nlf._estimator()
+        nimg, dev = len(frames), frames[0].device
+        k, bias_corr, vst_type = pipe["k"], pipe["bias_corr"], pipe.get("vst_type", "exact")
+        full_dn = bool(pipe["full_dn"])
+        pads = [isp.get_p2d((1, 4, f.shape[0] // 2, f.shape[1] // 2), base=32) for f in frames]
+        key = [(f.shape[0] // 2 + pd[2] + pd[3], f.shape[1] // 2 + pd[0] + pd[1], f.shape[0], f.shape[1]) for f, pd in zip(frames, pads)]
+        order = np.asarray(sorted(range(nimg), key=lambda i: key[i]), np.int64)  # stable: equal sizes keep the caller's order
+        groups = []  # (first, end, H, W) ranges of the device order
+        for j, i in enumerate(order):
+            if j and key[order[j - 1]] == key[i]:
+                groups[-1][1] = j + 1
+            else:
+                groups.append([j, j + 1, frames[i].shape[0], frames[i].shape[1]])
+        # (scale_est, scale, bound) per image for round 1 and the collab rounds, as iter_denoise_dev for nblk = 1 (:256, :393, :449)
+        scales1 = np.stack([scale_est, scale, scale if full_dn else scale_est], 1)[order]
+        scales_c = np.stack([scale_est, scale, scale_est], 1)[order]
+        table = nlf.FrameTable([frames[i] for i in order], [scales1, scales_c] + ([raw_rec[order]] if raw is not None else []))
+        s1_dev, sc_dev = (v.view(torch.float64) for v in table.extra[:2])
+        raw_dev = table.extra[2] if raw is not None else None
+        off = table.off.astype(np.int64)
+        # round 1: one self estimate of every frame; its var map is stdfilt(lr, k)**2 of the collab rounds, its first pass gives seg_max
+        lr_var = eng._buf("lr_var", (table.n_el,), torch.float32, dev) if n_collab else None
+        seg_max = torch.empty(nimg, device=dev, dtype=torch.float32) if bias_corr == "pre" else None
+        regs = est.estimate_frames(table, k, var_map=lr_var, seg_max=seg_max, raw=raw_dev)
+        ch = eng.chain_params(regs, seg_max, nimg, 1, *scales1.T, 1, bias_corr, vst_type, scales_dev=s1_dev)
+        psz = C.sizeof(VstParams)
+
+        def denoise(ch, out, fallback=None):
+            for g0, g1, H, W in groups:
+                sl = slice(int(off[g0]), int(off[g1]))
+                part = {key_: ch[key_] for key_ in ("rows", "xnodes", "stride")}
+                part.update(params=ch["params"][g0 * psz:], t=ch["t"][g0:], ok=ch["ok"][g0:])
+                eng.vst_denoise_dev(table.records_from(g0), part, out[sl].view(g1 - g0, H, W), select=fallback is not None,
+                                    fallback=None if fallback is None else fallback[sl], raw=None if raw_dev is None else raw_dev[g0 * RAW_REC.itemsize:],
+                                    shape=(g1 - g0, H, W))
+            return out
+
+        out = denoise(ch, torch.empty(table.n_el, device=dev, dtype=torch.float32))
+        flat, regs4, live = [out], [ch["regs4"]], [ch["ok"]]
+        # rounds 2 .. max_iter + 1: one collab estimate of every frame against the cached var map, the chain with prev=, selection
+        for r in range(2, n_collab + 2):
+            regs = est.estimate_collab_frames(out, table, lr_var, k)
+            ch = eng.chain_params(regs, seg_max, nimg, 1, *scales_c.T, r, bias_corr, vst_type, prev=ch, scales_dev=sc_dev)
+            out = denoise(ch, torch.empty_like(out), fallback=out)
+            flat.append(out)
+            regs4.append(ch["regs4"])
+            live.append(ch["ok"])
+        pos = np.empty(nimg, np.int64)
+        pos[order] = np.arange(nimg)  # device row of caller frame i
+        dns = [[o[int(off[pos[i]]):int(off[pos[i] + 1])].view(frames[i].shape) for i in range(nimg)] for o in flat]
+        return {"dns": dns, "regs4": regs4, "live": live, "flat": flat, "order": order, "table": table}
+
+    def iter_denoise_frames(self, frames, p, raw=None):
+        """IterDenoise for a batch of full frames of any even sizes in one call (iter_denoise_frames_dev), float32 or, with raw=, 16-bit
+        sensor mosaics.  Returns {'raw_dns': [[caller frame i's (H_i, W_i) output] per round, max_iter + 1 of them], 'regs': [(nimg, 2) per
+        round, NaN rows in the rounds an image did not complete], 'rounds': (nimg,)}, everything in the caller's order, after one
+        read-back at the end (read_summary)."""
+        res = self.iter_denoise_frames_dev(frames, p, raw=raw)
+        regs, rounds, _ = self.read_summary(res)
+        pos = np.argsort(res["order"])
+        return {"raw_dns": res["dns"], "regs": [r[pos] for r in regs], "rounds": rounds[pos], "dev": res}
 
     def iter_denoise_host(self, host_in, host_out, p, group=8, lanes=1, wait=True, raw=None):
         """End-to-end batched IterDenoise on HOST buffers: host_in (nimg,nblk,H,W) f32 pinned -> host_out (nimg,H,nblk*W) f32
