@@ -101,6 +101,39 @@ int yond_render_srgb(const float* bayer, uint8_t* bgr, int B, int H, int W, int 
  * Bit-exact against opencv-python 4.13.0. */
 int yond_demosaic_ea(const uint16_t* bayer, uint16_t* rgb, int B, int H, int W, void* stream);
 
+/* ---- the pictures and numbers of a whole SIDD evaluation — YOND_SIDD.py:635-668 (multiprocess_plot) over every image and round at
+ * once, each image rendered with its own metadata (:601-607: bayer_2by2, wb and cst2 of the image) ----
+ * yond_render_cam: one image's camera, the numbers process_sidd_image derives from its metadata (utils/sidd_utils.py:156-180):
+ *   gain = (1/wb_r, 1/wb_g, 1/wb_g, 1/wb_b) per 2x2 site of the flipped frame, row-major (:249-252, :272); cam2rgb = row-normalised
+ *   inv(cst2 x rgb2xyz), row-major (:161-170); flip_lr / flip_ud: the flips of flip_bayer (:182-196).
+ * yond_render_pic: one picture: `src` the (H,W) float32 mosaic (NULL: not rendered), `cam` the index of its camera record, `src_max`
+ *   (optional) a DEVICE float holding max(src, 0) (yond_seg_max): 0 means not rendered — the reference renders and scores nothing for
+ *   an output without a positive value (:644-647).  `reserved` is not read.
+ * yond_render_srgb_cams: yond_render_srgb of B pictures of one size (H, W) in one launch, picture b from pics_dev[b] with camera
+ *   cams_dev[pics_dev[b].cam] (both DEVICE arrays; `cam` is not range-checked), into bgr (B,H,W,3).  Same arithmetic and bytes as
+ *   yond_render_srgb with that camera; a picture that is not rendered leaves its bytes of bgr as they were.
+ * yond_sidd_scores: the per-image table from per-block numbers.  psnr / ssim: (nround, nimg, nblk) float64, yond_block_metrics of
+ *   every round's output against the clean mosaics; psnr_rgb / ssim_rgb (both or neither may be NULL): the same layout,
+ *   yond_block_metrics_rgb8 of the rendered pictures; out_max: (nround, nimg) float32 max(output, 0) per round (yond_seg_max);
+ *   rounds_dev: (nimg) int32, the rounds each image completed.  table: (nround, nimg, 4) float64 = (psnr, ssim, psnr_rgb, ssim_rgb),
+ *   each the sum over the nblk blocks in block order / nblk (:651-665).  Where out_max is 0: psnr = ssim = -1 and the sRGB entries
+ *   NaN; rounds at or beyond rounds_dev[i]: all four NaN; without sRGB inputs the sRGB entries are NaN. */
+typedef struct yond_render_cam {
+  double gain[4];
+  double cam2rgb[9];
+  int32_t flip_lr, flip_ud;
+} yond_render_cam;
+typedef struct yond_render_pic {
+  const float* src;
+  const float* src_max;
+  int32_t cam;
+  int32_t reserved;
+} yond_render_pic;
+int yond_render_srgb_cams(const yond_render_pic* pics_dev, const yond_render_cam* cams_dev, uint8_t* bgr, int B, int H, int W,
+                          void* stream);
+int yond_sidd_scores(const double* psnr, const double* ssim, const double* psnr_rgb, const double* ssim_rgb, const float* out_max,
+                     const int32_t* rounds_dev, int nround, int nimg, int nblk, double* table, void* stream);
+
 /* ---- A3/A4 elementwise, for the function-level surface — utils/isp_algos.py:5-14, :17-33 ---- */
 int yond_vst(const float* x, float* z, size_t n, double sigma, double gain, void* stream);
 int yond_inverse_vst(const float* z, float* x, size_t n, double sigma, double gain, int exact, void* stream);

@@ -44,6 +44,8 @@ SIGNATURES = {
     "yond_block_metrics_rgb8": (_I, [_P, _P, _I, _I, _I, _I, C.POINTER(C.c_double), _P, _P, _P]),
     "yond_render_srgb": (_I, [_P, _P, _I, _I, _I, _I, _I, C.POINTER(C.c_double), C.POINTER(C.c_double), _P]),
     "yond_demosaic_ea": (_I, [_P, _P, _I, _I, _I, _P]),
+    "yond_render_srgb_cams": (_I, [_P, _P, _P, _I, _I, _I, _P]),
+    "yond_sidd_scores": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _P, _P]),
     "yond_vst": (_I, [_P, _P, _SZ, _D, _D, _P]),
     "yond_inverse_vst": (_I, [_P, _P, _SZ, _D, _D, _I, _P]),
     "yond_lut_row": (_I, [_P, _I, _I, _D, _P, _P]),

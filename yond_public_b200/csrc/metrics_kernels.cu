@@ -133,6 +133,40 @@ __global__ void metrics_finish_kernel(double* psnr, double* ssim, int n, double 
   if (ssim) ssim[i] = ssim[i] / nvalid;
 }
 
+// One thread per (round, image) of a SIDD evaluation: the per-image numbers of multiprocess_plot (YOND_SIDD.py:643-665) from the
+// per-block ones — the sum over the blocks in block order / nblk; (-1, -1) and no sRGB numbers where the output has no positive value
+// (:644-647); nothing for rounds the image did not complete.
+__global__ void sidd_scores_kernel(const double* __restrict__ psnr, const double* __restrict__ ssim, const double* __restrict__ psnr_rgb,
+                                   const double* __restrict__ ssim_rgb, const float* __restrict__ out_max,
+                                   const int32_t* __restrict__ rounds, int nround, int nimg, int nblk, double* __restrict__ table) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;  // round * nimg + image
+  if (i >= nround * nimg) return;
+  const int r = i / nimg, img = i - r * nimg;
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  double* o = table + (size_t)i * 4;
+  if (r >= rounds[img]) {
+    o[0] = o[1] = o[2] = o[3] = nan;
+    return;
+  }
+  if (!(out_max[i] > 0.f)) {
+    o[0] = o[1] = -1.0;
+    o[2] = o[3] = nan;
+    return;
+  }
+  const double* src[4] = {psnr, ssim, psnr_rgb, ssim_rgb};
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    if (!src[k]) {
+      o[k] = nan;
+      continue;
+    }
+    const double* v = src[k] + (size_t)i * nblk;
+    double sum = 0.0;
+    for (int b = 0; b < nblk; ++b) sum += v[b];
+    o[k] = sum / nblk;
+  }
+}
+
 template <typename T>
 int block_metrics_impl(const char* who, const T* a, const T* b, int nimg, int H, int Wm, int nblk, int nch, double data_range,
                        float ssim_scale, const double* window11, double* psnr, double* ssim, void* stream) {
@@ -175,4 +209,16 @@ extern "C" int yond_block_metrics(const float* a, const float* b, int nimg, int 
 extern "C" int yond_block_metrics_rgb8(const uint8_t* a, const uint8_t* b, int nimg, int H, int Wm, int nblk, const double* window11,
                                        double* psnr, double* ssim, void* stream) {
   return block_metrics_impl<uint8_t>("yond_block_metrics_rgb8", a, b, nimg, H, Wm, nblk, 3, 255.0, 1.0f, window11, psnr, ssim, stream);
+}
+
+extern "C" int yond_sidd_scores(const double* psnr, const double* ssim, const double* psnr_rgb, const double* ssim_rgb, const float* out_max,
+                                const int32_t* rounds_dev, int nround, int nimg, int nblk, double* table, void* stream) {
+  YOND_REQUIRE(psnr && ssim && out_max && rounds_dev && table, "yond_sidd_scores: null pointer");
+  YOND_REQUIRE(!psnr_rgb == !ssim_rgb, "yond_sidd_scores: give both sRGB inputs or neither");
+  YOND_REQUIRE(nround > 0 && nimg > 0 && nblk > 0 && (long long)nround * nimg <= (1ll << 30), "yond_sidd_scores: bad shape");
+  const int n = nround * nimg;
+  sidd_scores_kernel<<<ceil_div(n, 128), 128, 0, (cudaStream_t)stream>>>(psnr, ssim, psnr_rgb, ssim_rgb, out_max, rounds_dev, nround, nimg,
+                                                                         nblk, table);
+  YOND_LAUNCH_CHECK();
+  return YOND_OK;
 }

@@ -63,12 +63,28 @@ __device__ __forceinline__ void demosaic_px(const uint16_t (*q)[kSW], int ty, in
   }
 }
 
-template <bool kRender>
+// kTable (render only): picture bz is the (H, W) mosaic of record pics[bz] with the camera cams[pics[bz].cam] (yond_render_pic,
+// yond_render_cam), read once per CTA, instead of picture bz of one (B, H, W) tensor under the by-value `p` — every image of a SIDD
+// evaluation with its own metadata, the clean mosaics and each round's output where their owners keep them.  A record without a
+// source, or whose src_max holds no positive value (YOND_SIDD.py:644-647: such an output is neither rendered nor scored), returns
+// before its first load.  p.inv_gamma still comes from the argument.  The arithmetic is the uniform form's.
+template <bool kRender, bool kTable = false>
 __global__ void __launch_bounds__(256) render_kernel(const float* __restrict__ img, const uint16_t* __restrict__ mosaic,
                                                      uint8_t* __restrict__ bgr, uint16_t* __restrict__ rgb16, int H, int W,
-                                                     RenderParams p) {
+                                                     RenderParams p, const yond_render_pic* __restrict__ pics,
+                                                     const yond_render_cam* __restrict__ cams) {
   __shared__ uint16_t q[kSH][kSW];
   __shared__ double steps[256];
+  const yond_render_cam* cam = nullptr;
+  if constexpr (kTable) {
+    const yond_render_pic pic = pics[blockIdx.z];
+    if (pic.src == nullptr || (pic.src_max != nullptr && !(*pic.src_max > 0.f))) return;
+    cam = cams + pic.cam;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) p.gain[i] = cam->gain[i];
+    p.flip_lr = cam->flip_lr, p.flip_ud = cam->flip_ud;
+    img = pic.src;
+  }
   if (kRender) steps[threadIdx.x] = g_gamma_steps[threadIdx.x];
   const int x0 = blockIdx.x * kTW, y0 = blockIdx.y * kTH;
   const size_t plane = (size_t)H * W;
@@ -76,9 +92,13 @@ __global__ void __launch_bounds__(256) render_kernel(const float* __restrict__ i
   for (int i = threadIdx.x; i < kSH * kSW; i += blockDim.x) {
     const int ty = i / kSW, tx = i - ty * kSW;
     const int y = min(max(y0 + ty - 1, 0), H - 1), x = min(max(x0 + tx - 1, 0), W - 1);
-    q[ty][tx] = kRender ? quantise(img + bz * plane, H, W, y, x, p) : __ldg(mosaic + bz * plane + (size_t)y * W + x);
+    q[ty][tx] = kRender ? quantise(kTable ? img : img + bz * plane, H, W, y, x, p) : __ldg(mosaic + bz * plane + (size_t)y * W + x);
   }
   __syncthreads();
+  if constexpr (kTable) {  // read after the tile is built, so that the gains and the matrix are not live at the same time
+#pragma unroll
+    for (int i = 0; i < 9; ++i) p.ccm[i] = cam->cam2rgb[i];
+  }
   const int ly = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int y = y0 + ly;
   if (y >= H) return;
@@ -178,7 +198,22 @@ extern "C" int yond_render_srgb(const float* bayer, uint8_t* bgr, int B, int H, 
   cudaStream_t s = (cudaStream_t)stream;
   YondProfScope prof("render_srgb", s, 7.0 * (double)B * H * W);
   dim3 grid(ceil_div(W, kTW), ceil_div(H, kTH), B);
-  render_kernel<true><<<grid, 256, 0, s>>>(bayer, nullptr, bgr, nullptr, H, W, p);
+  render_kernel<true><<<grid, 256, 0, s>>>(bayer, nullptr, bgr, nullptr, H, W, p, nullptr, nullptr);
+  YOND_LAUNCH_CHECK();
+  return YOND_OK;
+}
+
+extern "C" int yond_render_srgb_cams(const yond_render_pic* pics_dev, const yond_render_cam* cams_dev, uint8_t* bgr, int B, int H,
+                                     int W, void* stream) {
+  YOND_REQUIRE(pics_dev && cams_dev && bgr, "yond_render_srgb_cams: null pointer");
+  if (int e = check_shape("yond_render_srgb_cams", B, H, W)) return e;
+  RenderParams p = {};
+  p.inv_gamma = 1.0 / 2.2;
+  if (int e = upload_gamma_steps(p.inv_gamma)) return e;
+  cudaStream_t s = (cudaStream_t)stream;
+  YondProfScope prof("render_srgb", s, 7.0 * (double)B * H * W);
+  dim3 grid(ceil_div(W, kTW), ceil_div(H, kTH), B);
+  render_kernel<true, true><<<grid, 256, 0, s>>>(nullptr, nullptr, bgr, nullptr, H, W, p, pics_dev, cams_dev);
   YOND_LAUNCH_CHECK();
   return YOND_OK;
 }
@@ -190,7 +225,7 @@ extern "C" int yond_demosaic_ea(const uint16_t* bayer, uint16_t* rgb, int B, int
   cudaStream_t s = (cudaStream_t)stream;
   YondProfScope prof("demosaic_ea", s, 8.0 * (double)B * H * W);
   dim3 grid(ceil_div(W, kTW), ceil_div(H, kTH), B);
-  render_kernel<false><<<grid, 256, 0, s>>>(nullptr, bayer, nullptr, rgb, H, W, p);
+  render_kernel<false><<<grid, 256, 0, s>>>(nullptr, bayer, nullptr, rgb, H, W, p, nullptr, nullptr);
   YOND_LAUNCH_CHECK();
   return YOND_OK;
 }

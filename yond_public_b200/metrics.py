@@ -145,3 +145,106 @@ def sidd_eval_image(outputs, hr_raw, meta=None, nblk=32, rgb=True):
             res["ssim_rgb"].append(float(sr.mean().cpu()))
             res["img_dn"].append(img)
     return res
+
+
+_SSIM_WIN = 11
+_GRID_Z = 65535  # blocks per grid z of the metric and render kernels
+
+
+def _check_mosaics(name, t):
+    if not torch.is_tensor(t) or not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.dim() != 3:
+        raise ValueError(f"{name}: need a contiguous CUDA float32 (nimg, H, nblk*Wb) tensor, got "
+                         f"{tuple(t.shape) if torch.is_tensor(t) else type(t).__name__}"
+                         f"{'' if not torch.is_tensor(t) else f' {t.dtype} on {t.device}'}")
+    if t.data_ptr() % 16:
+        raise ValueError(f"{name}: the data must be 16-byte aligned")
+
+
+def sidd_eval_batch(raw_dns, hr_raw, metas=None, nblk=32, rounds=None, rgb=True):
+    """sidd_eval_image for every image and round of a batch in one pass (YOND_SIDD.py:635-668, the scoring half of the SIDD eval):
+    raw_dns is the list of (nimg, H, nblk*Wb) CUDA float32 mosaics per round that YOND_SIDD.iter_denoise_batch returns, hr_raw the
+    (nimg, H, nblk*Wb) clean mosaics, metas nimg dicts with 'bayer_2by2', 'wb', 'cst2' (None: raw numbers only), rounds the rounds each
+    image completed (iter_denoise_batch's res['rounds']; None: all of them).  Every image is rendered with its own metadata.
+
+    Returns, after one read-back: 'psnr', 'ssim', 'psnr_rgb', 'ssim_rgb': (nround, nimg) float64 NumPy arrays — the mean over the
+    blocks; raw (-1, -1) and sRGB NaN where the output has no positive value (the reference neither renders nor scores it); all four
+    NaN for rounds at or beyond rounds[i] (repeats of the last completed round); sRGB NaN without metas or with rgb=False.
+    'img_hr': (nimg, H, W, 3) and 'img_dn': (nround, nimg, H, W, 3) uint8 CUDA BGR pictures (None without metas or with rgb=False),
+    'rendered': (nround, nimg) bool; the bytes of a picture that was not rendered are unspecified.
+    Raises ValueError, before anything is enqueued, for inputs of the wrong number, shape, device, dtype or layout, metadata without
+    a key or with an unknown Bayer pattern, rounds outside [1, nround], Wm % nblk != 0, blocks smaller than the SSIM window, and
+    more block-channels (or pictures) than one launch of the metric (or render) kernel takes."""
+    from .pipeline import _upload
+    from .render import PIC_REC, camera_records
+    dns = list(raw_dns)
+    _check_mosaics("hr_raw", hr_raw)
+    nimg, H, Wm = hr_raw.shape
+    nround = len(dns)
+    if nround < 1:
+        raise ValueError("raw_dns: need at least one round")
+    for r, t in enumerate(dns):
+        _check_mosaics(f"raw_dns[{r}]", t)
+        if t.shape != hr_raw.shape or t.device != hr_raw.device:
+            raise ValueError(f"raw_dns[{r}]: shape {tuple(t.shape)} on {t.device}, hr_raw is {tuple(hr_raw.shape)} on {hr_raw.device}")
+    do_rgb = bool(rgb and metas is not None)
+    if metas is not None:
+        metas = list(metas)
+        if len(metas) != nimg:
+            raise ValueError(f"metas: {len(metas)} entries for {nimg} images")
+        cams = camera_records(metas)
+    if rounds is None:
+        rnd = np.full(nimg, nround, np.int32)
+    else:
+        rnd = np.asarray(rounds)
+        if rnd.shape != (nimg,):
+            raise ValueError(f"rounds: need one entry per image ({nimg}), got shape {rnd.shape}")
+        if not np.issubdtype(rnd.dtype, np.integer) or (rnd < 1).any() or (rnd > nround).any():
+            raise ValueError(f"rounds: need integers in [1, {nround}], got {rnd.tolist()}")
+        rnd = rnd.astype(np.int32)
+    nblk = int(nblk)
+    if nblk < 1 or Wm % nblk:
+        raise ValueError(f"nblk: {Wm} columns do not split into {nblk} blocks")
+    Wb = Wm // nblk
+    if H < _SSIM_WIN or Wb < _SSIM_WIN:
+        raise ValueError(f"blocks of {H} x {Wb} are smaller than the {_SSIM_WIN} x {_SSIM_WIN} SSIM window")
+    if H % 2 or Wm % 2:
+        raise ValueError(f"H and W must be even (Bayer mosaics), got {H} x {Wm}")
+    if nimg * nblk * (3 if do_rgb else 1) > _GRID_Z or (do_rgb and (nround + 1) * nimg > _GRID_Z):
+        raise ValueError(f"{nimg} images x {nblk} blocks x {nround} rounds: more block-channels or pictures than one launch takes "
+                         f"({_GRID_Z}); split the batch")
+
+    dev = hr_raw.device
+    blk = torch.empty((4 if do_rgb else 2, nround, nimg, nblk), device=dev, dtype=torch.float64)  # per-block psnr, ssim[, _rgb]
+    out_max = torch.empty((nround, nimg), device=dev, dtype=torch.float32)
+    table = torch.empty((nround, nimg, 4), device=dev, dtype=torch.float64)
+    pics = torch.empty((nround + 1, nimg, H, Wm, 3), device=dev, dtype=torch.uint8) if do_rgb else None
+    uploads = [rnd]
+    if do_rgb:  # picture (0, i) the clean mosaic of image i, (r + 1, i) round r's output; none for the rounds it did not complete
+        rec = np.zeros((nround + 1, nimg), PIC_REC)
+        rec["cam"] = np.arange(nimg, dtype=np.int32)
+        rec["src"][0] = hr_raw.data_ptr() + np.arange(nimg, dtype=np.uint64) * (H * Wm * 4)
+        for r, t in enumerate(dns):
+            live = r < rnd
+            rec["src"][r + 1] = np.where(live, t.data_ptr() + np.arange(nimg, dtype=np.uint64) * (H * Wm * 4), 0)
+            rec["src_max"][r + 1] = out_max[r].data_ptr() + np.arange(nimg, dtype=np.uint64) * 4
+        uploads += [rec, cams]
+    up, offs = _upload(uploads, dev)
+    at = [C.c_void_p(up.data_ptr() + o) for o in offs]
+    lib, s = _lib.load(), stream_ptr()
+    win = _WIN.ctypes.data_as(C.POINTER(C.c_double))
+    for r, t in enumerate(dns):
+        check(lib.yond_seg_max(ptr(t), H * Wm, nimg, ptr(out_max[r]), s))
+    if do_rgb:
+        check(lib.yond_render_srgb_cams(at[1], at[2], ptr(pics), (nround + 1) * nimg, H, Wm, s))
+    for r, t in enumerate(dns):
+        check(lib.yond_block_metrics(ptr(t), ptr(hr_raw), nimg, H, Wm, nblk, 1.0, 255.0, win, ptr(blk[0, r]), ptr(blk[1, r]), s))
+        if do_rgb:
+            check(lib.yond_block_metrics_rgb8(ptr(pics[r + 1]), ptr(pics[0]), nimg, H, Wm, nblk, win, ptr(blk[2, r]), ptr(blk[3, r]), s))
+    check(lib.yond_sidd_scores(ptr(blk[0]), ptr(blk[1]), ptr(blk[2]) if do_rgb else None, ptr(blk[3]) if do_rgb else None,
+                               ptr(out_max), at[0], nround, nimg, nblk, ptr(table), s))
+    host = table.cpu().numpy()
+    res = {k: np.ascontiguousarray(host[..., j]) for j, k in enumerate(("psnr", "ssim", "psnr_rgb", "ssim_rgb"))}
+    res["rendered"] = ~np.isnan(res["psnr_rgb"])  # with pictures, a rendered one always has finite sRGB numbers
+    res["img_hr"] = pics[0] if do_rgb else None
+    res["img_dn"] = pics[1:] if do_rgb else None
+    return res

@@ -34,14 +34,37 @@ def cam2rgb_matrix(cst):
     return cam2rgb / np.sum(cam2rgb, axis=-1, keepdims=True)
 
 
+# yond_render_cam / yond_render_pic (include/yond_b200.h)
+CAM_REC = np.dtype([("gain", "<f8", (4,)), ("cam2rgb", "<f8", (9,)), ("flip_lr", "<i4"), ("flip_ud", "<i4")])
+PIC_REC = np.dtype([("src", "<u8"), ("src_max", "<u8"), ("cam", "<i4"), ("reserved", "<i4")])
+META_KEYS = ("bayer_2by2", "wb", "cst2")
+
+
+def camera_records(metas):
+    """One yond_render_cam per SIDD metadata dict (keys 'bayer_2by2', 'wb', 'cst2'): the flips (utils/sidd_utils.py:182-196), gains
+    per 2x2 site (:249-252) and cam2rgb matrix (:161-170) the render of that image uses, in the reference's float64 NumPy arithmetic —
+    the one place process_sidd_image and metrics.sidd_eval_batch take them from.  ValueError for a missing key or an unknown Bayer
+    pattern."""
+    rec = np.zeros(len(metas), CAM_REC)
+    for i, meta in enumerate(metas):
+        missing = [k for k in META_KEYS if k not in meta]
+        if missing:
+            raise ValueError(f"meta {i} lacks {missing}")
+        rec["flip_lr"][i], rec["flip_ud"][i] = _FLIPS[_pattern_key(meta["bayer_2by2"])]
+        wb = np.asarray(meta["wb"], np.float64)
+        rec["gain"][i] = [1 / wb[0][0], 1 / wb[0][1], 1 / wb[0][1], 1 / wb[0][2]]
+        rec["cam2rgb"][i] = cam2rgb_matrix(meta["cst2"]).reshape(-1)
+    return rec
+
+
 def process_sidd_image(image, bayer_pattern, wb, cst, *, save_file_rgb=None):
     """utils/sidd_utils.py:156-180.  image: (H,W) (or (B,H,W) sharing one camera) float32 mosaic, NumPy or CUDA tensor; returns the
     (H,W,3) uint8 BGR picture (NumPy in -> NumPy out, tensor in -> CUDA tensor out), in the flipped orientation the reference
     leaves it in."""
-    flip_lr, flip_ud = _FLIPS[_pattern_key(bayer_pattern)]
-    wb = np.asarray(wb, np.float64)
-    gains = np.array([1 / wb[0][0], 1 / wb[0][1], 1 / wb[0][2]], np.float64)
-    ccm = np.ascontiguousarray(cam2rgb_matrix(cst), np.float64)
+    cam = camera_records([{"bayer_2by2": bayer_pattern, "wb": wb, "cst2": cst}])[0]
+    flip_lr, flip_ud = int(cam["flip_lr"]), int(cam["flip_ud"])
+    gains = np.ascontiguousarray(cam["gain"][[0, 1, 3]])
+    ccm = np.ascontiguousarray(cam["cam2rgb"])
     x, np_in = to_dev(image)
     batched = x.dim() == 3
     xb = x if batched else x[None]
